@@ -4,6 +4,7 @@
   python bench.py [--gpus N] [--steps K] [--warmup W] [--task reach] [--control joints] [--envs 65536]
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
   python bench.py --impl reference ...      # the CPU arm: the oracle port of the reference's PyBullet path on the host cores
+  python bench.py --dump-outputs DIR ...    # also write the last timed step's outputs as DIR/<name>.npy (compare two builds)
 
 A step = one RobotTaskEnv.step of every environment (20 physics sub-steps + controller + observation + reward, auto-reset
 on success / TimeLimit), one kernel launch.  Default workload = BASELINE.json configs[1]: PandaReachJoints-v3, 65,536 envs
@@ -15,13 +16,16 @@ import argparse
 import ctypes
 import json
 import os
+import shutil
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the benchmark writes nothing into the tree, which may be read-only
 
 METRIC = "env-steps/sec"
 # `roofline.traffic` / `launches_per_step` come from profiles/kernel_traffic.json, which scripts/ncu_traffic.py writes from an
@@ -62,8 +66,43 @@ def workload_name(task, control, reward, envs):
 
 # ------------------------------------------------------------------------------------------------ CPU arm (oracle port)
 def oracle_lib():
-    from tests.oracle_util import build_oracle
-    return ctypes.CDLL(build_oracle())
+    """The CPU oracle as build() left it in oracle/; when that library is missing or older than its sources, a private copy is
+    compiled in a temporary directory, so that the tree stays untouched."""
+    src = os.path.join(ROOT, "oracle")
+    so = os.path.join(src, "libpanda_oracle.so")
+    if os.path.exists(so) and all(os.path.getmtime(os.path.join(src, f)) <= os.path.getmtime(so) for f in ("panda_oracle.c", "panda_oracle.h")):
+        return ctypes.CDLL(so)
+    tmp = tempfile.mkdtemp(prefix="panda_oracle_")
+    try:
+        for f in ("Makefile", "panda_oracle.c", "panda_oracle.h"):
+            shutil.copy(os.path.join(src, f), tmp)
+        subprocess.run(["make", "-C", tmp], check=True, stdout=subprocess.DEVNULL)
+        return ctypes.CDLL(os.path.join(tmp, "libpanda_oracle.so"))      # stays mapped after the directory is removed
+    finally:
+        shutil.rmtree(tmp, ignore_errors=True)
+
+
+# what PandaVecEnv.step returns (info["is_success"] is `terminated` again), written by --dump-outputs
+OUTPUT_NAMES = ("observation", "achieved_goal", "desired_goal", "reward", "terminated", "truncated")
+DUMP_BYTES = 63 * 10**6         # under 64 MB in all with the .npy headers
+
+
+def dump_outputs(out_dir, step_out):
+    """Writes one step's outputs as out_dir/<name>.npy in float32 (flags as 0 / 1), one row per env, plus env_index.npy (float64)
+    with the index of each row's env.  Above DUMP_BYTES in all, the rows are a fixed sample of envs (seed 0, sorted)."""
+    import numpy as np
+    import torch
+    obs, rew, term, trunc, _ = step_out
+    arrays = dict(zip(OUTPUT_NAMES, (obs["observation"], obs["achieved_goal"], obs["desired_goal"], rew, term, trunc)))
+    n = rew.shape[0]
+    row_bytes = 8 + 4 * sum(a[0].numel() for a in arrays.values())
+    rows = min(n, DUMP_BYTES // row_bytes)
+    idx = np.arange(n) if rows == n else np.sort(np.random.default_rng(0).choice(n, rows, replace=False))
+    sel = torch.from_numpy(idx).to(rew.device)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a.index_select(0, sel).float().cpu().numpy())
+    np.save(os.path.join(out_dir, "env_index.npy"), idx.astype(np.float64))
 
 
 class CpuPool:
@@ -190,7 +229,7 @@ def run_gpu(args):
 
     def timed_leg(task, control, n, steps, warmup):
         """PREROLL + warmup untimed steps, then `steps` device-timed steps (CUDA events around each step on the launching stream, L2
-        flushed between them).  Returns (env, actions, device seconds on this rank, launches)."""
+        flushed between them).  Returns (env, actions, device seconds on this rank, launches, what the last timed step returned)."""
         A = action_dim(task, control)
         env = p.PandaVecEnv(task, n, reward_type=args.reward, control_type=control, device=local, seed=args.seed, env_id_offset=rank * n, auto_reset=True)
         actions = torch.rand((ncyc, n, A), device=dev, generator=gen) * 2 - 1      # synthetic actions, resident in HBM
@@ -206,16 +245,18 @@ def run_gpu(args):
         l0 = p.kernel_launches()
         for k, (a, b) in enumerate(ev):
             flush.zero_()                              # L2 flush between timed iterations (outside the event pair)
-            a.record(); env.step(actions[(k + warmup) % ncyc]); b.record()
+            a.record(); last = env.step(actions[(k + warmup) % ncyc]); b.record()
         barrier()
-        return env, actions, sum(a.elapsed_time(b) for a, b in ev) / 1e3, p.kernel_launches() - l0
+        return env, actions, sum(a.elapsed_time(b) for a, b in ev) / 1e3, p.kernel_launches() - l0, last
 
     n, A = args.envs, action_dim(args.task, args.control)
     sampler = ClockSampler(local) if rank == 0 else None
     t_wall0 = time.perf_counter()
-    env, actions, dev_s_local, launches = timed_leg(args.task, args.control, n, args.steps, args.warmup)
+    env, actions, dev_s_local, launches, last = timed_leg(args.task, args.control, n, args.steps, args.warmup)
     t_wall = time.perf_counter() - t_wall0
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last)                                   # rank 0's envs
     dev_s = allmax(dev_s_local)                                                     # max over ranks
     stats = torch.tensor(env.stats(), dtype=torch.float64, device=dev)
     if world > 1:
@@ -251,7 +292,7 @@ def run_gpu(args):
         for task2, ctrl2, n2, k2 in (("reach", "ee", 65536, 30), ("pick_and_place", "ee", 32768, 30), ("push", "ee", 65536, 20), ("slide", "ee", 65536, 20), ("stack", "ee", 65536, 15)):
             sec2, err2 = -1.0, None
             try:                          # rank-local work only inside the try: a failure on one rank must not leave the others in a collective
-                env2, act2, sec2, _ = timed_leg(task2, ctrl2, n2, k2, 3)
+                env2, act2, sec2, _, _ = timed_leg(task2, ctrl2, n2, k2, 3)
                 env2.close(); del act2
             except Exception as exc:
                 err2 = repr(exc)
@@ -431,7 +472,12 @@ def main():
     ap.add_argument("--seed", type=int, default=0)
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--no-her", action="store_true", help="skip the HER compute_reward measurement")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs (rank 0's envs) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200")
     args.warmup = max(args.warmup, 3)
     if args.impl == "reference":
         run_reference(args)
