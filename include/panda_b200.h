@@ -89,6 +89,18 @@ int pg_step(pg_env* env, const float* actions, float* obs, float* achieved_goal,
  * per-env EE target quaternion [N,4] (x,y,z,w; float32, normalised inside) fed to the IK instead of (1,0,0,0).  ee control only. */
 int pg_step_oriented(pg_env* env, const float* actions, const float* target_quat, float* obs, float* achieved_goal, float* desired_goal,
                      float* reward, unsigned char* terminated, unsigned char* truncated, int auto_reset, void* stream);
+/* pybullet getContactPoints after RobotTaskEnv.step, for every env: as pg_step_oriented, plus the contacts of the step's last sub-step
+ * (rows below; normalForce = applied impulse / timeStep) and their number per env.  contacts / contact_count may be NULL (DEVICE).
+ * contacts [N, C, 16] float32 with C = pg_max_contacts; rows at and beyond contact_count[i] are unspecified.  Row words:
+ *   0-2 contact point (world), as the contact model generates it;  3-5 normal on B, pointing from B to A (world);  6 normal force (N);
+ *   7 lateral friction force 1 (N), 8-10 its direction;  11 lateral friction force 2 (N), 12-14 its direction;  15 id_a + 32 * id_b
+ *   (an exact float).  Ids are pg_render's segmentation ids: 1 plane, 2 table, 3 / 4 objects, 14 hand (link 8), 15 / 16 fingers
+ *   (links 9 / 10).  There is no contactDistance.  With auto_reset the report describes the finished step, like reward. */
+int pg_step_contacts(pg_env* env, const float* actions, const float* target_quat, float* obs, float* achieved_goal, float* desired_goal,
+                     float* reward, unsigned char* terminated, unsigned char* truncated, int auto_reset,
+                     float* contacts, unsigned char* contact_count, void* stream);
+/* C of the rows above: contacts per env and sub-step of the handle's scene (10, or 22 for Stack; later candidates are dropped). */
+int pg_max_contacts(const pg_env* env, int* per_env);
 /* Action scaling of Panda.set_action: defaults 0.05 (ee / joint displacement, panda.py:81,103) and 0.2 (fingers, panda.py:65);
  * the fork's panda_cartesian.py:67,157 uses 1.0 / 1.0. */
 int pg_set_action_scale(pg_env* env, double ee_scale, double finger_scale);

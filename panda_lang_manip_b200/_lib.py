@@ -18,7 +18,7 @@ REWARD = {"sparse": 0, "dense": 1}
 PRECISION = {"f32": 0, "f64": 1}
 
 SYMBOLS = [
-    "pg_create", "pg_destroy", "pg_dims", "pg_reset", "pg_step", "pg_step_oriented", "pg_set_action_scale", "pg_step_host", "pg_host_pin", "pg_host_unpin", "pg_compute_reward", "pg_is_success",
+    "pg_create", "pg_destroy", "pg_dims", "pg_reset", "pg_step", "pg_step_oriented", "pg_step_contacts", "pg_max_contacts", "pg_set_action_scale", "pg_step_host", "pg_host_pin", "pg_host_unpin", "pg_compute_reward", "pg_is_success",
     "pg_compute_reward_host", "pg_is_success_host", "pg_her_relabel", "pg_save_state", "pg_restore_state", "pg_remove_state", "pg_get_state", "pg_set_state",
     "pg_inverse_kinematics", "pg_get_ee_pose", "pg_create_bare", "pg_set_motors", "pg_get_motors", "pg_sim_step", "pg_inverse_kinematics_link", "pg_get_link_state",
     "pg_save_state_async", "pg_restore_state_async", "pg_host_stage_allocations", "pg_reset_seeded", "pg_set_task_params", "pg_set_substeps",
@@ -53,6 +53,8 @@ def load() -> ctypes.CDLL:
     lib.pg_reset.argtypes = [vp, vp, vp, vp, vp, vp, vp, vp]
     lib.pg_step.argtypes = [vp, vp, vp, vp, vp, vp, vp, vp, c_int, vp]
     lib.pg_step_oriented.argtypes = [vp, vp, vp, vp, vp, vp, vp, vp, vp, c_int, vp]
+    lib.pg_step_contacts.argtypes = [vp, vp, vp, vp, vp, vp, vp, vp, vp, c_int, vp, vp, vp]
+    lib.pg_max_contacts.argtypes = [vp, pi]
     lib.pg_set_action_scale.argtypes = [vp, ctypes.c_double, ctypes.c_double]
     lib.pg_step_host.argtypes = [vp, vp, vp, vp, vp, vp, vp, vp, c_int]
     lib.pg_host_pin.argtypes = [vp, ctypes.c_size_t]

@@ -341,7 +341,7 @@ static int ensure_group_streams(pg_env* e, int k) {
     return PG_OK;
 }
 static int step_impl(pg_env* e, const float* actions, const float* target_quat, float* obs, float* ag, float* dg, float* reward, unsigned char* terminated,
-                     unsigned char* truncated, int auto_reset, cudaStream_t stream, const HostIO* hio) {
+                     unsigned char* truncated, int auto_reset, float* contacts, unsigned char* contact_count, cudaStream_t stream, const HostIO* hio) {
     PG_CUDA(cudaSetDevice(e->device));
     // Contact-aware scheduling (see perm_*_kernel): large batches are re-sorted by their contact state before every launch, and a
     // step is cut into `segments` launches of consecutive sub-steps so that envs which make contact mid-step are regrouped; small
@@ -373,7 +373,8 @@ static int step_impl(pg_env* e, const float* actions, const float* target_quat, 
         int* ghist = hist + (size_t)(t0 / PERM_CHUNK + g) * PERM_BUCKETS;
         const int nsub = e->Ef.P.nsub;
         for (int sg = 0; sg < segs; sg++) {
-            StepIO io{target_quat, actions, obs, ag, dg, reward, terminated, truncated, auto_reset, sg * nsub / segs, (sg + 1) * nsub / segs};
+            StepIO io{target_quat, actions, obs, ag, dg, reward, terminated, truncated, auto_reset, sg * nsub / segs, (sg + 1) * nsub / segs,
+                      contacts, contact_count};
             if (io.s0 == io.s1) continue;       // fewer sub-steps than segments
             if (use_perm) {
                 perm_hist_kernel<<<nchunks, PERM_THREADS, 0, st>>>(key + t0, ghist, cnt);
@@ -395,12 +396,22 @@ static int step_impl(pg_env* e, const float* actions, const float* target_quat, 
     PG_CUDA(cudaGetLastError());
     return PG_OK;
 }
-int pg_step_oriented(pg_env* e, const float* actions, const float* target_quat, float* obs, float* ag, float* dg, float* reward, unsigned char* terminated,
-                     unsigned char* truncated, int auto_reset, void* stream) {
+int pg_step_contacts(pg_env* e, const float* actions, const float* target_quat, float* obs, float* ag, float* dg, float* reward, unsigned char* terminated,
+                     unsigned char* truncated, int auto_reset, float* contacts, unsigned char* contact_count, void* stream) {
     if (!e || !actions) return fail(PG_ERR_ARG, "pg_step: NULL handle or actions");
     if (e->task == PG_TASK_BARE) return fail(PG_ERR_ARG, "pg_step: a bare world is advanced with pg_sim_step");
     if (target_quat && e->ctrl != CTRL_EE) return fail(PG_ERR_ARG, "pg_step_oriented: a target orientation needs ee control");
-    return step_impl(e, actions, target_quat, obs, ag, dg, reward, terminated, truncated, auto_reset, (cudaStream_t)stream, nullptr);
+    return step_impl(e, actions, target_quat, obs, ag, dg, reward, terminated, truncated, auto_reset, contacts, contact_count, (cudaStream_t)stream, nullptr);
+}
+int pg_step_oriented(pg_env* e, const float* actions, const float* target_quat, float* obs, float* ag, float* dg, float* reward, unsigned char* terminated,
+                     unsigned char* truncated, int auto_reset, void* stream) {
+    return pg_step_contacts(e, actions, target_quat, obs, ag, dg, reward, terminated, truncated, auto_reset, nullptr, nullptr, stream);
+}
+int pg_max_contacts(const pg_env* e, int* per_env) {
+    if (!e || !per_env) return fail(PG_ERR_ARG, "pg_max_contacts: NULL argument");
+    if (e->task == PG_TASK_BARE) return fail(PG_ERR_ARG, "pg_max_contacts: bare worlds have no contact report");
+    *per_env = max_contacts(e->nobj);
+    return PG_OK;
 }
 
 static int ensure_host_path(pg_env* e) {
@@ -454,7 +465,7 @@ int pg_step_host(pg_env* e, const float* actions, float* obs, float* ag, float* 
         o.host = o.direct ? o.user : (void*)((char*)e->h_out + ((const char*)o.dev - (const char*)e->d_out));
     }
     HostIO hio{src, (float*)outs[0].host, (float*)outs[1].host, (float*)outs[2].host, (float*)outs[3].host, (unsigned char*)outs[4].host, (unsigned char*)outs[5].host};
-    rc = step_impl(e, e->d_act, nullptr, d_obs, d_ag, d_dg, d_rew, d_term, d_trunc, auto_reset, e->hstream, &hio); if (rc != PG_OK) return rc;
+    rc = step_impl(e, e->d_act, nullptr, d_obs, d_ag, d_dg, d_rew, d_term, d_trunc, auto_reset, nullptr, nullptr, e->hstream, &hio); if (rc != PG_OK) return rc;
     PG_CUDA(cudaStreamSynchronize(e->hstream));
     for (const Out& o : outs) if (o.user && !o.direct) memcpy(o.user, o.host, o.bytes);
     return PG_OK;

@@ -407,6 +407,29 @@ template <typename T, int NOBJ> PG_HD ContactCtx<T, NOBJ> contact_ctx(Contacts<T
     for (int o = 0; o < NOBJ; o++) X.sgo[o] = (A == 3 + o) ? T(1) : ((B == 3 + o) ? T(-1) : T(0));
     return X;
 }
+
+// ---------------------------------------------------------------------------------------------- contact report
+// pybullet getContactPoints of the last sub-step, one row of REPORT_WORDS per contact (pg_step_contacts, include/panda_b200.h):
+// point (3), normal on B pointing from B to A (3), normal force, lateral friction force 1 and its direction (1 + 3), force 2 and its
+// direction (1 + 3), id_a + 32 id_b.  Forces are the solver's accumulated impulses / dt.  Body ids are the segmentation ids of
+// pg_render: 1 plane, 2 table, 3 / 4 objects, 14 hand, 15 / 16 fingers.  The record's distance word holds the normal row's rhs by now,
+// so the row has no contactDistance.
+constexpr int REPORT_WORDS = 16;
+PG_HD constexpr int report_body_id(int body) { return body < 3 ? 14 + body : body; }      // body codes 0..2 robot boxes, 3 + o objects
+template <typename T, typename R> PG_HD void contact_report_row(const Scene<T>& S, Contacts<T>& C, int c, R* row) {
+    const V3<T> P = mk<T>(C.f(c, C_P), C.f(c, C_P + 1), C.f(c, C_P + 2)), n = mk<T>(C.f(c, C_N), C.f(c, C_N + 1), C.f(c, C_N + 2));
+    const int code = (int)C.f(c, C_CODE), A = (code & 7) - 1, B = ((code >> 3) & 7) - 1;
+    V3<T> t1, t2;
+    if (code & 128) { t1 = mk<T>(T(0), T(-1), T(0)); t2 = mk<T>(T(1), T(0), T(0)); }     // table kinds: the rows' axis-aligned tangents
+    else plane_space(n, t1, t2);
+    // static body B: robot boxes only touch the table top; an object vertex is on the table or the ground plane by collect_contacts' rule
+    const int idb = B >= 0 ? report_body_id(B) : ((A < 3 || (over_table(S, P) && P.z > T(-0.05))) ? 2 : 1);
+    const T k = Consts<T>::inv_dt;
+    const T v[REPORT_WORDS] = {P.x, P.y, P.z, n.x, n.y, n.z, C.f(c, C_APP) * k, C.f(c, C_APP + 1) * k, t1.x, t1.y, t1.z, C.f(c, C_APP + 2) * k, t2.x, t2.y, t2.z,
+                               T(report_body_id(A) + 32 * idb)};
+#pragma unroll
+    for (int w = 0; w < REPORT_WORDS; w++) row[w] = (R)v[w];
+}
 template <typename T, int NOBJ> PG_HD void robot_wrench(const OpSpace<T>& Op, const ContactCtx<T, NOBJ>& X, V3<T> d, T* w) {
     V3<T> m = cross(X.P - Op.O6, d);
     T fd = dot(Op.hy, d);

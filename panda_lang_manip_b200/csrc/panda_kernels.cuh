@@ -45,6 +45,8 @@ struct StepIO {
     const float* actions; float* obs; float* ag; float* dg; float* reward; unsigned char* terminated; unsigned char* truncated;
     int auto_reset;
     int s0, s1;                  // sub-step range of this launch: [0, nsub) = a whole step
+    float* contacts;             // [n, max_contacts(nobj), REPORT_WORDS] contact report of the step's last sub-step, or NULL
+    unsigned char* contact_count;   // [n] its rows per env, or NULL
 };
 struct ResetIO {
     const unsigned char* mask; const double* goal_override; const double* object_override; float* obs; float* ag; float* dg;
@@ -320,6 +322,13 @@ __global__ void __launch_bounds__((step_block<T, TASK>())) step_kernel(const __g
         env_step_sim<T, TASK, CTRL, BS>(E.M, E.S, q, qd, ob, act, (first && io.target_quat) ? tquat : nullptr, C, sched_key, target, qc, io.s0, io.s1, E.P.nsub);
         if (E.dbg) { E.dbg[2 * (size_t)(E.t0 + t)] = clock64() - clk0; unsigned smid; asm volatile("mov.u32 %0, %%smid;" : "=r"(smid)); E.dbg[2 * (size_t)(E.t0 + t) + 1] = (long long)sched_key | ((long long)smid << 16); }
         if (C.dropped > 0) atomicAdd(&s_stats[5], (double)C.dropped);
+        if (last) {     // the report of the step that just ended: the records are still in this thread's column of the slab, before any reset
+            if (io.contacts) {
+                float* rows = io.contacts + (size_t)i * (max_contacts(NOBJ) * REPORT_WORDS);
+                for (int c = 0; c < C.n; c++) contact_report_row(E.S, C, c, rows + c * REPORT_WORDS);
+            }
+            if (io.contact_count) io.contact_count[i] = (unsigned char)C.n;
+        }
         double goal[6];
         if (last) {     // the goal is only needed now: loaded after the simulation so that it does not occupy registers across the solver
             load_goal(E, i, goal);

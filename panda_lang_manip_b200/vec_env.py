@@ -26,11 +26,13 @@ class PandaVecEnv:
     ``control_type`` "ee"|"joints".  ``env_id_offset`` is the global index of env 0 (sharded runs), ``precision`` "f32"
     (product path) or "f64" (parity debugging).  ``n_substeps`` is PyBullet(n_substeps) (pybullet.py:26); ``distance_threshold`` and the
     ``*_range_low/high`` noise boxes are the task constructors' keyword arguments (tasks/*.py __init__), see ``set_task_params``.
+    ``contact_report``: every ``step`` also reports the contacts of its last sub-step (pybullet getContactPoints), see ``contacts``.
     """
 
     def __init__(self, task: str, num_envs: int, reward_type: str = "sparse", control_type: str = "ee", device: int = 0,
                  seed: int = 0, env_id_offset: int = 0, precision: str = "f32", auto_reset: bool = True, n_substeps: int = 20,
-                 distance_threshold: Optional[float] = None, goal_range_low=None, goal_range_high=None, obj_range_low=None, obj_range_high=None) -> None:
+                 distance_threshold: Optional[float] = None, goal_range_low=None, goal_range_high=None, obj_range_low=None, obj_range_high=None,
+                 contact_report: bool = False) -> None:
         import ctypes
         if not torch.cuda.is_available():
             raise _lib.PandaB200Error("PandaVecEnv needs a CUDA device: the B200 kernels are the only implementation")
@@ -59,6 +61,13 @@ class PandaVecEnv:
         self.reward = torch.empty((n,), dtype=f32, device=self.device)
         self.terminated = torch.empty((n,), dtype=torch.uint8, device=self.device)
         self.truncated = torch.empty((n,), dtype=torch.uint8, device=self.device)
+        self._contacts = self._contact_count = None
+        if contact_report:
+            c = ctypes.c_int()
+            _lib.check(self.lib.pg_max_contacts(h, ctypes.byref(c)))
+            self.max_contacts = c.value
+            self._contacts = torch.zeros((n, self.max_contacts, 16), dtype=f32, device=self.device)
+            self._contact_count = torch.zeros((n,), dtype=torch.uint8, device=self.device)
         self.reset()
 
     # -- lifecycle ---------------------------------------------------------------------------------------------------
@@ -137,9 +146,25 @@ class PandaVecEnv:
         if a.shape != (self.num_envs, self.action_dim):
             raise ValueError(f"actions must be [{self.num_envs}, {self.action_dim}], got {tuple(a.shape)}")
         tq = None if target_orientation is None else target_orientation.to(device=self.device, dtype=torch.float32).reshape(self.num_envs, 4).contiguous()
-        _lib.check(self.lib.pg_step_oriented(self._h, _ptr(a), _ptr(tq), _ptr(self.obs), _ptr(self.achieved_goal), _ptr(self.desired_goal), _ptr(self.reward),
-                                    _ptr(self.terminated), _ptr(self.truncated), int(self.auto_reset), self._stream()))
+        _lib.check(self.lib.pg_step_contacts(self._h, _ptr(a), _ptr(tq), _ptr(self.obs), _ptr(self.achieved_goal), _ptr(self.desired_goal), _ptr(self.reward),
+                                             _ptr(self.terminated), _ptr(self.truncated), int(self.auto_reset), _ptr(self._contacts), _ptr(self._contact_count),
+                                             self._stream()))
         return self._obs_dict(), self.reward, self.terminated, self.truncated, {"is_success": self.terminated}
+
+    def contacts(self) -> Dict[str, torch.Tensor]:
+        """pybullet getContactPoints after the last ``step``, for every env (env built with ``contact_report=True``): the contacts of the
+        step's last sub-step, padded to ``max_contacts`` per env (10, or 22 for Stack); entries at and beyond ``count[i]`` are unspecified.
+        The float entries are views of the env's report buffer, overwritten by the next step: ``position`` [N,C,3] (world), ``normal`` [N,C,3] (on B, from B to
+        A), ``normal_force`` [N,C] (N), ``lateral_friction1`` / ``lateral_friction2`` [N,C] (N) with ``lateral_friction_dir1`` /
+        ``lateral_friction_dir2`` [N,C,3], ``body_a`` / ``body_b`` [N,C] int32 segmentation ids (1 plane, 2 table, 3 / 4 objects, 14 hand,
+        15 / 16 fingers) and ``count`` [N] int32 are decoded copies.  With auto-reset the report describes the finished step, like ``reward``."""
+        if self._contacts is None:
+            raise _lib.PandaB200Error("contacts(): this env was built without contact_report=True")
+        r = self._contacts
+        ids = r[..., 15].to(torch.int32)
+        return {"position": r[..., 0:3], "normal": r[..., 3:6], "normal_force": r[..., 6], "lateral_friction1": r[..., 7], "lateral_friction_dir1": r[..., 8:11],
+                "lateral_friction2": r[..., 11], "lateral_friction_dir2": r[..., 12:15], "body_a": ids % 32, "body_b": ids // 32,
+                "count": self._contact_count.to(torch.int32)}
 
     def step_host(self, actions: np.ndarray):
         """End-to-end step with host buffers (numpy in, numpy out): H2D copy, kernel, D2H copy inside the call."""
