@@ -81,8 +81,7 @@ int pg_set_substeps(pg_env* env, int n_substeps);
  * Ordering: everything the call enqueues is ordered after the work already on `stream` and completes before work enqueued on
  * `stream` afterwards.  Batches of >= 4096 envs are advanced by several launches (a step cut into sub-step segments, each after a
  * re-sort of the thread -> env map) and, from 16384 envs, in env groups on streams the handle owns, forked from and joined back
- * to `stream` with events (legal under stream capture).  None of this changes a result.  Environment knobs for A/B runs:
- * PG_SORT_ENVS=0, PG_SEGMENTS=<divisor of 20>, PG_GROUPS=<1..8>. */
+ * to `stream` with events (legal under stream capture).  None of this changes a result. */
 int pg_step(pg_env* env, const float* actions, float* obs, float* achieved_goal, float* desired_goal, float* reward,
             unsigned char* terminated, unsigned char* truncated, int auto_reset, void* stream);
 /* The fork's orientation-target control (panda_gym/envs/robots/panda_ori.py:52-99: set_action(action, euler_xyz)): as pg_step, with a

@@ -67,12 +67,11 @@ struct pg_env {
     std::map<int, void*> snaps; int next_snap = 0;
     RenderPrim* prims = nullptr; RenderScene rscene;  // analytic renderer: per-env primitive lists (allocated at the first pg_render)
     std::vector<void*> snap_pool;                    // buffers of removed snapshots, reused by the next save (no allocation in a save / remove loop)
-    bool sort_envs = true;                            // PG_SORT_ENVS=0 disables the contact-aware thread->env map (A/B measurements)
     // env groups: sorted batches are cut into groups of consecutive envs, each advanced on its own stream, so that the tail of
     // one group's launch (a few contact-heavy blocks) overlaps with the other groups' launches instead of idling the GPU
     long long* dbg = nullptr;
     int groups = 1; cudaStream_t gstream[8] = {}; cudaEvent_t ev_fork = nullptr, ev_join[8] = {};
-    int segments = 4;                                 // launches per step for sorted batches (see pg_create); PG_SEGMENTS overrides (a divisor of 20)
+    int segments = 4;                                 // launches per step for sorted batches (see pg_create)
     // host-buffer path: pinned staging + device I/O buffers + private stream
     cudaStream_t hstream = nullptr;
     float *h_act = nullptr, *h_out = nullptr; float* d_act = nullptr; float* d_out = nullptr; size_t out_floats = 0; size_t out_bytes = 0;
@@ -117,25 +116,15 @@ template <typename E> static int her_vector_bytes(int G, const void* a, const vo
     }
     return (int)sizeof(E);
 }
-template <typename E, int TASK, int HT> static void launch_her_ht(const E* next_ag, const E* dg, const long long* src, const long long* goal_src, E* dg_out, E* ag_out, float* reward,
-                                                                  long long m, long long pitch, int reward_type, double thr, cudaStream_t st) {
-    const long long per_block = 256LL * HT;
-    const int grid = (int)std::min<long long>((m + per_block - 1) / per_block, 148LL * 32);
-    const int vb = her_vector_bytes<E>(task_goal_dim(TASK), next_ag, dg, pitch);
-    if (vb == 16) her_relabel_kernel<E, TASK, 16, HT><<<grid, 256, 0, st>>>(next_ag, dg, src, goal_src, dg_out, ag_out, reward, m, pitch, reward_type, thr);
-    else if (vb == 8) her_relabel_kernel<E, TASK, 8, HT><<<grid, 256, 0, st>>>(next_ag, dg, src, goal_src, dg_out, ag_out, reward, m, pitch, reward_type, thr);
-    else her_relabel_kernel<E, TASK, (int)sizeof(E), HT><<<grid, 256, 0, st>>>(next_ag, dg, src, goal_src, dg_out, ag_out, reward, m, pitch, reward_type, thr);
-    g_launches++;
-}
 template <typename E, int TASK> static void launch_her_task(const E* next_ag, const E* dg, const long long* src, const long long* goal_src, E* dg_out, E* ag_out, float* reward,
                                                             long long m, long long pitch, int reward_type, double thr, cudaStream_t st) {
-    static const int ht = [] { const char* v = getenv("PG_HER_INFLIGHT"); const int k = v ? atoi(v) : HER_INFLIGHT; return (k == 1 || k == 2 || k == 4 || k == 8) ? k : HER_INFLIGHT; }();
-    switch (ht) {
-    case 1: launch_her_ht<E, TASK, 1>(next_ag, dg, src, goal_src, dg_out, ag_out, reward, m, pitch, reward_type, thr, st); break;
-    case 2: launch_her_ht<E, TASK, 2>(next_ag, dg, src, goal_src, dg_out, ag_out, reward, m, pitch, reward_type, thr, st); break;
-    case 8: launch_her_ht<E, TASK, 8>(next_ag, dg, src, goal_src, dg_out, ag_out, reward, m, pitch, reward_type, thr, st); break;
-    default: launch_her_ht<E, TASK, 4>(next_ag, dg, src, goal_src, dg_out, ag_out, reward, m, pitch, reward_type, thr, st); break;
-    }
+    const long long per_block = 256LL * HER_INFLIGHT;
+    const int grid = (int)std::min<long long>((m + per_block - 1) / per_block, 148LL * 32);
+    const int vb = her_vector_bytes<E>(task_goal_dim(TASK), next_ag, dg, pitch);
+    if (vb == 16) her_relabel_kernel<E, TASK, 16><<<grid, 256, 0, st>>>(next_ag, dg, src, goal_src, dg_out, ag_out, reward, m, pitch, reward_type, thr);
+    else if (vb == 8) her_relabel_kernel<E, TASK, 8><<<grid, 256, 0, st>>>(next_ag, dg, src, goal_src, dg_out, ag_out, reward, m, pitch, reward_type, thr);
+    else her_relabel_kernel<E, TASK, (int)sizeof(E)><<<grid, 256, 0, st>>>(next_ag, dg, src, goal_src, dg_out, ag_out, reward, m, pitch, reward_type, thr);
+    g_launches++;
 }
 template <typename E> static void launch_her(int task, const E* next_ag, const E* dg, const long long* src, const long long* goal_src, E* dg_out, E* ag_out, float* reward,
                                              long long m, long long pitch, int reward_type, double thr, cudaStream_t st) {
@@ -188,7 +177,6 @@ int pg_create(int task, int control_type, int reward_type, int num_envs, int dev
     if (rc != PG_OK) { pg_destroy(e); return rc; }
     e->Ef.S = make_scene<float>(task); e->Ed.S = make_scene<double>(task);
     e->Ef.P = e->Ed.P = make_task_params(task);
-    { const char* v = getenv("PG_SORT_ENVS"); if (v && v[0] == '0') e->sort_envs = false; }
     const bool light = e->nobj == 0 && control_type == CTRL_JOINTS;
     e->segments = light ? 4 : 20;
     { const char* v = getenv("PG_DEBUG_TIMING"); if (v && v[0] == '1') { PG_CUDA(cudaMalloc(&e->dbg, (size_t)e->n * 2 * sizeof(long long))); PG_CUDA(cudaMemset(e->dbg, 0, (size_t)e->n * 2 * sizeof(long long))); } }
@@ -196,12 +184,10 @@ int pg_create(int task, int control_type, int reward_type, int num_envs, int dev
     // measured defaults (profiles/r1_notes.md): contact scenes and ee control re-sort before every sub-step and run 4 env groups (2 for ee-controlled Reach);
     // joint-controlled Reach (few contacts) keeps 4 launches per step on one stream
     e->groups = (num_envs >= 16384 && !light) ? (e->nobj == 0 ? 2 : 4) : 1;
-    { const char* v = getenv("PG_GROUPS"); if (v) { int k = atoi(v); if (k >= 1 && k <= 8) e->groups = k; } }
     if (e->groups > 1) {
         PG_CUDA(cudaEventCreateWithFlags(&e->ev_fork, cudaEventDisableTiming));
         for (int g = 0; g < e->groups; g++) { PG_CUDA(cudaStreamCreateWithFlags(&e->gstream[g], cudaStreamNonBlocking)); PG_CUDA(cudaEventCreateWithFlags(&e->ev_join[g], cudaEventDisableTiming)); }
     }
-    { const char* v = getenv("PG_SEGMENTS"); if (v) { int k = atoi(v); if (k >= 1 && k <= 20 && 20 % k == 0) e->segments = k; } }
     *out = e;
     rc = pg_reset(e, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr);
     if (rc != PG_OK) { pg_destroy(e); *out = nullptr; return rc; }
@@ -223,7 +209,6 @@ int pg_create_bare(int num_envs, int device, int precision, const double* robot_
     pg_env* e = new pg_env();
     e->task = PG_TASK_BARE; e->ctrl = CTRL_JOINTS; e->reward = 0; e->n = num_envs; e->device = device; e->precision = precision;
     e->nobj = n_bodies; e->obs_dim = 0; e->goal_dim = 0; e->act_dim = 0; e->max_steps = 0; e->state_dim = 18 + 13 * n_bodies + 1;
-    e->sort_envs = false;
     // a world without a robot still carries one (the kernels are built around it): it is parked 1 km up, out of reach of everything
     const double parked[3] = {0.0, 0.0, 1000.0};
     rc = alloc_state(e, 0, 0, robot_base ? robot_base : parked);
@@ -332,32 +317,22 @@ int pg_set_substeps(pg_env* e, int n_substeps) {
 // Host-buffer mode of a step (pg_step_host): every env group copies its own action rows in before its first launch and its own
 // output rows out after its last one, on its own stream -- group g's device-to-host copies overlap group g+1's kernels.
 struct HostIO { const float* act; float* obs; float* ag; float* dg; float* rew; unsigned char* term; unsigned char* trunc; };
-static int ensure_group_streams(pg_env* e, int k) {
-    if (!e->ev_fork) PG_CUDA(cudaEventCreateWithFlags(&e->ev_fork, cudaEventDisableTiming));
-    for (int g = 0; g < k; g++) {
-        if (!e->gstream[g]) PG_CUDA(cudaStreamCreateWithFlags(&e->gstream[g], cudaStreamNonBlocking));
-        if (!e->ev_join[g]) PG_CUDA(cudaEventCreateWithFlags(&e->ev_join[g], cudaEventDisableTiming));
-    }
-    return PG_OK;
-}
 static int step_impl(pg_env* e, const float* actions, const float* target_quat, float* obs, float* ag, float* dg, float* reward, unsigned char* terminated,
                      unsigned char* truncated, int auto_reset, float* contacts, unsigned char* contact_count, cudaStream_t stream, const HostIO* hio) {
     PG_CUDA(cudaSetDevice(e->device));
     // Contact-aware scheduling (see perm_*_kernel): large batches are re-sorted by their contact state before every launch, and a
     // step is cut into `segments` launches of consecutive sub-steps so that envs which make contact mid-step are regrouped; small
     // batches keep the identity map, one launch per step and the tiled I/O path.  Results do not depend on either choice.
-    const bool use_perm = e->sort_envs && e->n >= 4096;
+    const bool use_perm = e->n >= 4096;
     const int segs = use_perm ? e->segments : 1;
     const unsigned short* key = e->precision == PG_F32 ? e->Ef.ccount : e->Ed.ccount;
     int* hist = e->precision == PG_F32 ? e->Ef.hist : e->Ed.hist;
     int* perm = e->precision == PG_F32 ? e->Ef.perm : e->Ed.perm;
     EnvDev<float> Ef = e->Ef; EnvDev<double> Ed = e->Ed;
     if (!use_perm) { Ef.perm = nullptr; Ed.perm = nullptr; }
-    int groups = use_perm ? e->groups : 1;
-    // host mode pipelines the copies against the env groups the configuration already has; PG_HOST_GROUPS forces more (measured: on one
-    // GPU the single-stream Reach-joints configuration loses 5 % when cut into 4 groups only to overlap 0.2 ms of copies)
-    if (hio && use_perm && e->n >= 16384) { static const int hg = getenv("PG_HOST_GROUPS") ? atoi(getenv("PG_HOST_GROUPS")) : 0; if (hg > groups && hg <= 8) groups = hg; }
-    if (groups > 1) { int rc = ensure_group_streams(e, groups); if (rc != PG_OK) return rc; }
+    // host mode pipelines the copies against the env groups the configuration already has (measured: on one GPU the single-stream
+    // Reach-joints configuration loses 5 % when cut into 4 groups only to overlap 0.2 ms of copies)
+    const int groups = use_perm ? e->groups : 1;
     // group g owns the envs (and thread slots) [g * gsize, min(n, (g + 1) * gsize)), gsize a multiple of the sort chunk
     const int gsize = ((e->n + groups - 1) / groups + PERM_CHUNK - 1) / PERM_CHUNK * PERM_CHUNK;
     const size_t A = e->act_dim, O = e->obs_dim, G = e->goal_dim;

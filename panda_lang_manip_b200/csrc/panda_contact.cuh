@@ -139,20 +139,6 @@ constexpr int JX_SLOTS = 42;            // Jx: per arm joint j, angular (z_j) an
 PG_HD constexpr int max_contacts(int nobj) { return nobj <= 1 ? 10 : 22; }
 PG_HD constexpr int solver_slots(int nobj) { return JX_SLOTS + max_contacts(nobj) * REC; }
 enum { C_P = 0, C_N = 3, C_INVD = 6, C_RHS = 9, C_APP = 12, C_MU = 15, C_CODE = 16 };
-// Response cache of robot-only scenes (Reach): while an env has at most YC_MAX contacts -- two fingertips on the table are four -- the
-// records of the contacts YC_MAX .. 9 are unused, and the three rows' operational-space impulse responses y = Lambda w (8 words each) of
-// the first YC_MAX contacts live there: a row application is then 8 shared-memory loads + 8 FMAs instead of the 40-FMA Lambda product.
-constexpr int YC_MAX = 4;
-// Measured build variants (profiles/r2_solver_structure_ab): PG_YC = the response cache, PG_OOL = the full sweep as a non-inlined function,
-// PG_WATCH_EE (panda_env.cuh) = the watched sweep for ee control.  None of them beats round 1's structure on B200, so all default to 0.
-#ifndef PG_YC
-#define PG_YC 0
-#endif
-#ifndef PG_OOL
-#define PG_OOL 0
-#endif
-PG_HD constexpr bool yc_supported(int nobj) { return PG_YC && nobj == 0 && (max_contacts(nobj) - YC_MAX) * REC >= YC_MAX * 24; }
-PG_HD constexpr int yc_slot(int c, int k) { return JX_SLOTS + YC_MAX * REC + (c * 3 + k) * 8; }
 
 template <typename T> struct CStore {   // per-thread view of the shared-memory slab (host test build: a plain array, stride 1)
     T* base; int stride;
@@ -165,7 +151,6 @@ template <typename T> struct Contacts {
     int nB, nA;                 // contacts are collected in type order: [0, nB) object vertex on a plane, [nB, nB + nA) robot box on the table, then generic
     bool near;                  // the gripper is within 3 cm of the table or inside an object's broad-phase sphere (scheduling hint)
     bool capped;                // the last solve ran (nearly) all 50 sweeps (scheduling hint)
-    bool ycache;                // the rows' impulse responses are cached in the store (robot-only scenes with at most YC_MAX contacts, see YC_SLOT)
     PG_HD T& f(int c, int k) { return st.at(JX_SLOTS + c * REC + k); }
     PG_HD T& jx(int j, int a) { return st.at(6 * j + a); }
 };
@@ -231,7 +216,6 @@ PG_HD void collect_contacts(const Scene<T>& S, const World<T, NOBJ>& W, const Ob
         }
     }
     C.nA = C.n - C.nB;
-    C.ycache = yc_supported(NOBJ) && C.n <= YC_MAX;
     // 3. robot box <-> object, both directions
     if (NOBJ > 0) {
 #pragma unroll
@@ -469,12 +453,6 @@ template <int AX, int SG, typename T, int NOBJ> struct AxisRow {
         for (int k = 0; k < 8; k++) d8[k] += y[k] * di;
         F8[I1] += m1 * di; F8[I2] += m2 * di; F8[3 + AX] += T(SG) * di; F8[6] += f6 * di; F8[7] += f7 * di;
     }
-    PG_HD T den(const OpSpace<T>& Op) const { T y[8]; lam(Op, y); return jdv(y); }
-    PG_HD void apply_cached(const T* y, T di, T* d8, T* F8) const {      // y = lam(Op) from the response cache
-#pragma unroll
-        for (int k = 0; k < 8; k++) d8[k] += y[k] * di;
-        F8[I1] += m1 * di; F8[I2] += m2 * di; F8[3 + AX] += T(SG) * di; F8[6] += f6 * di; F8[7] += f7 * di;
-    }
 };
 // Object-vs-plane row along SG * e_AX (the object is body A): J = [e; r x e], W = [e/m; Iinv (r x e)] with r x e_AX two-sparse.
 template <int AX, int SG, typename T> struct ObjAxisRow {
@@ -487,7 +465,6 @@ template <int AX, int SG, typename T> struct ObjAxisRow {
         const int c2[3] = {I2 == 0 ? 0 : (I2 == 1 ? 1 : 2), I2 == 0 ? 1 : (I2 == 1 ? 3 : 4), I2 == 0 ? 2 : (I2 == 1 ? 4 : 5)};
         return mk<T>(I[c1[0]] * m1 + I[c2[0]] * m2, I[c1[1]] * m1 + I[c2[1]] * m2, I[c1[2]] * m1 + I[c2[2]] * m2);
     }
-    PG_HD T den(const T* I, T inv_mass) const { V3<T> w = wang(I); const T a[3] = {w.x, w.y, w.z}; return inv_mass + m1 * a[I1] + m2 * a[I2]; }
     PG_HD void apply(const T* I, T inv_mass, T di, V3<T>& vl, V3<T>& va) const {
         const T dl = T(SG) * di * inv_mass;
         if (AX == 0) vl.x += dl; else if (AX == 1) vl.y += dl; else vl.z += dl;
@@ -502,7 +479,7 @@ template <typename T> PG_HD T dot8(const T* a, const T* b) {
 }
 
 // 1/D and rhs of the three rows of every contact (setupMultiBodyContactConstraint: speculative when separated, ERP when penetrating)
-template <typename T, int NOBJ, bool ROBOT = true>
+template <typename T, int NOBJ>
 PG_HD void rows_setup(const Scene<T>& S, const World<T, NOBJ>& W, const OpSpace<T>& Op, const Obj<T>* ob, Contacts<T>& C) {
     for (int c = 0; c < C.n; c++) {
         ContactCtx<T, NOBJ> X = contact_ctx<T, NOBJ>(C, c);
@@ -513,18 +490,12 @@ PG_HD void rows_setup(const Scene<T>& S, const World<T, NOBJ>& W, const OpSpace<
         for (int k = 0; k < 3; k++) {
             V3<T> d = k == 0 ? X.n : (k == 1 ? t1 : t2);
             T den = T(0), rel = T(0);
-            if (ROBOT) {
-                if (NOBJ == 0 || (X.table && X.rb >= 0)) {
-                    T y[8];
-                    if (k == 0) { AxisRow<2, 1, T, NOBJ> r(Op, X); r.lam(Op, y); den += r.jdv(y); rel += r.jdv(Op.v); }
-                    else if (k == 1) { AxisRow<1, -1, T, NOBJ> r(Op, X); r.lam(Op, y); den += r.jdv(y); rel += r.jdv(Op.v); }
-                    else { AxisRow<0, 1, T, NOBJ> r(Op, X); r.lam(Op, y); den += r.jdv(y); rel += r.jdv(Op.v); }
-                    if (yc_supported(NOBJ) && C.ycache) {
-#pragma unroll
-                        for (int a = 0; a < 8; a++) C.st.at(yc_slot(c, k) + a) = y[a];
-                    }
-                } else if (X.rb >= 0) { T w[8], y[8]; robot_wrench<T, NOBJ>(Op, X, d, w); lambda_mul(Op, w, y); den += dot8(w, y); rel += dot8(w, Op.v); }
-            }
+            if (NOBJ == 0 || (X.table && X.rb >= 0)) {
+                T y[8];
+                if (k == 0) { AxisRow<2, 1, T, NOBJ> r(Op, X); r.lam(Op, y); den += r.jdv(y); rel += r.jdv(Op.v); }
+                else if (k == 1) { AxisRow<1, -1, T, NOBJ> r(Op, X); r.lam(Op, y); den += r.jdv(y); rel += r.jdv(Op.v); }
+                else { AxisRow<0, 1, T, NOBJ> r(Op, X); r.lam(Op, y); den += r.jdv(y); rel += r.jdv(Op.v); }
+            } else if (X.rb >= 0) { T w[8], y[8]; robot_wrench<T, NOBJ>(Op, X, d, w); lambda_mul(Op, w, y); den += dot8(w, y); rel += dot8(w, Op.v); }
 #pragma unroll
             for (int o = 0; o < NOBJ; o++) {
                 if (X.sgo[o] != T(0)) {
@@ -591,9 +562,7 @@ PG_HD void contact_apply(const Scene<T>& S, const World<T, NOBJ>& W, const OpSpa
 // velocity change of a sweep is <= 1e-7; semi-implicit Euler.
 // The sequential-impulse loop.  FAST: the 14 arm limit rows are only watched; returns true if one of them would have engaged
 // (the caller then restarts with FAST = false).  Two instantiations, so the hot loop carries only the rows it executes.
-// ROBOT = false (the light path of the split scheme below): no robot box is in contact, so the operational-space code, the robot-on-table
-// rows and (with one object) the generic rows do not exist in the instantiation -- the contacts are object vertices on a plane only.
-template <typename T, int NOBJ, bool FAST, bool ROBOT = true>
+template <typename T, int NOBJ, bool FAST>
 PG_HD bool pgs_solve(const T* max_imp, const Scene<T>& S, const World<T, NOBJ>& W, const OpSpace<T>& Op, const T (*Minv)[ND], JointRows<T>& R,
                      Contacts<T>& C, const Obj<T>* ob, const bool robot_contacts, T* dvq, V3<T>* dvl, V3<T>* dva) {
     const int nc = C.n;
@@ -603,11 +572,11 @@ PG_HD bool pgs_solve(const T* max_imp, const Scene<T>& S, const World<T, NOBJ>& 
         T res = T(0), watch = T(0);
         joint_rows_sweep<FAST>(max_imp, Minv, R, dvq, it, res, watch);
         if (FAST && watch > T(0)) { live = true; break; }
-        if ((ROBOT || NOBJ > 0) && nc > 0) {
+        if (nc > 0) {
             T d8[8], F8[8];
 #pragma unroll
             for (int a = 0; a < 8; a++) { d8[a] = T(0); F8[a] = T(0); }
-            if (ROBOT && robot_contacts) {       // operational-space velocity change so far: Jx dvq
+            if (robot_contacts) {       // operational-space velocity change so far: Jx dvq
 #pragma unroll
                 for (int j = 0; j < 7; j++) {
 #pragma unroll
@@ -618,22 +587,17 @@ PG_HD bool pgs_solve(const T* max_imp, const Scene<T>& S, const World<T, NOBJ>& 
             // Typed passes: the three kinds of contact run different row code, and a warp pays for every kind present in any of its
             // lanes at a given contact index; looping kind by kind (collection order = kind order, so the row order is unchanged)
             // makes lanes meet in the same code even when their counts differ.
-            const int eB = !ROBOT ? nc : (NOBJ > 0 ? C.nB : 0), eA = !ROBOT ? nc : (NOBJ > 0 ? C.nB + C.nA : nc);
+            const int eB = NOBJ > 0 ? C.nB : 0, eA = NOBJ > 0 ? C.nB + C.nA : nc;
             auto normal_row = [&](int c, auto kind) {
                 constexpr int K = decltype(kind)::value;
                 ContactCtx<T, NOBJ> X = contact_ctx<T, NOBJ>(C, c);
                 T app = C.f(c, C_APP), inv = C.f(c, C_INVD), di = T(0);
-                if constexpr (K == KIND_ROBOT_TABLE && ROBOT) {
+                if constexpr (K == KIND_ROBOT_TABLE) {
                     AxisRow<2, 1, T, NOBJ> row(Op, X);
                     di = C.f(c, C_RHS) - app * (X.soft ? S.soft_cfm * inv : T(0)) - row.jdv(d8) * inv;
                     di = fmax(di, -app);              // accumulated normal impulse >= 0, on the change (short dependency chain)
                     C.f(c, C_APP) = app + di;
-                    if (yc_supported(NOBJ) && C.ycache) {
-                        T y[8];
-#pragma unroll
-                        for (int a = 0; a < 8; a++) y[a] = C.st.at(yc_slot(c, 0) + a);
-                        row.apply_cached(y, di, d8, F8);
-                    } else row.apply(Op, di, d8, F8);
+                    row.apply(Op, di, d8, F8);
                 } else if constexpr (K == KIND_OBJ_PLANE) {       // object vertex on the table / ground plane
                     const int o = (NOBJ == 2 && X.sgo[NOBJ - 1] != T(0)) ? 1 : 0;
                     ObjAxisRow<2, 1, T> row(X.P - ob[o].pos);
@@ -641,7 +605,7 @@ PG_HD bool pgs_solve(const T* max_imp, const Scene<T>& S, const World<T, NOBJ>& 
                     di = fmax(di, -app);              // accumulated normal impulse >= 0, on the change (short dependency chain)
                     C.f(c, C_APP) = app + di;
                     row.apply(W.Iinv[o], T(1) / S.mass[o], di, dvl[o], dva[o]);
-                } else if constexpr (ROBOT) {
+                } else {
                     T jd = dot(X.n, contact_dv<T, NOBJ>(Op, X, d8, dvl, dva, ob));
                     di = C.f(c, C_RHS) - app * (X.soft ? S.soft_cfm * inv : T(0)) - jd * inv;
                     di = fmax(di, -app);              // accumulated normal impulse >= 0, on the change (short dependency chain)
@@ -668,7 +632,7 @@ PG_HD bool pgs_solve(const T* max_imp, const Scene<T>& S, const World<T, NOBJ>& 
                     C.f(c, C_APP + 1) = s1; C.f(c, C_APP + 2) = s2;
                     const T im = T(1) / S.mass[o];
                     r1.apply(W.Iinv[o], im, d1, dvl[o], dva[o]); r2.apply(W.Iinv[o], im, d2, dvl[o], dva[o]);
-                } else if constexpr (K == KIND_ROBOT_TABLE && ROBOT) {
+                } else if constexpr (K == KIND_ROBOT_TABLE) {
                     AxisRow<1, -1, T, NOBJ> r1(Op, X); AxisRow<0, 1, T, NOBJ> r2(Op, X);
                     T s1 = a1 + C.f(c, C_RHS + 1) - r1.jdv(d8) * i1, s2 = a2 + C.f(c, C_RHS + 2) - r2.jdv(d8) * i2;
                     T len = sqrt(s1 * s1 + s2 * s2);
@@ -682,19 +646,14 @@ PG_HD bool pgs_solve(const T* max_imp, const Scene<T>& S, const World<T, NOBJ>& 
                         V3<T> m = cross(r, fdir);
                         T fd = dot(Op.hy, fdir);
                         T w[8] = {m.x, m.y, m.z, fdir.x, fdir.y, T(0), X.rb == 1 ? fd : T(0), X.rb == 2 ? -fd : T(0)};
-                        if (yc_supported(NOBJ) && C.ycache) {      // the two tangent rows' cached responses
 #pragma unroll
-                            for (int k = 0; k < 8; k++) { d8[k] += C.st.at(yc_slot(c, 1) + k) * d1 + C.st.at(yc_slot(c, 2) + k) * d2; F8[k] += w[k]; }
-                        } else {
-#pragma unroll
-                            for (int k = 0; k < 8; k++) {
-                                d8[k] += Op.L[sidx(k, 0)] * w[0] + Op.L[sidx(k, 1)] * w[1] + Op.L[sidx(k, 2)] * w[2] + Op.L[sidx(k, 3)] * w[3] + Op.L[sidx(k, 4)] * w[4]
-                                       + Op.L[sidx(k, 6)] * w[6] + Op.L[sidx(k, 7)] * w[7];
-                                F8[k] += w[k];
-                            }
+                        for (int k = 0; k < 8; k++) {
+                            d8[k] += Op.L[sidx(k, 0)] * w[0] + Op.L[sidx(k, 1)] * w[1] + Op.L[sidx(k, 2)] * w[2] + Op.L[sidx(k, 3)] * w[3] + Op.L[sidx(k, 4)] * w[4]
+                                   + Op.L[sidx(k, 6)] * w[6] + Op.L[sidx(k, 7)] * w[7];
+                            F8[k] += w[k];
                         }
                     }
-                } else if constexpr (ROBOT) {
+                } else {
                     V3<T> t1, t2; plane_space(X.n, t1, t2);
                     const V3<T> u = contact_dv<T, NOBJ>(Op, X, d8, dvl, dva, ob);
                     T j1 = dot(t1, u), j2 = dot(t2, u);
@@ -710,14 +669,14 @@ PG_HD bool pgs_solve(const T* max_imp, const Scene<T>& S, const World<T, NOBJ>& 
             {
                 int c = 0;
                 if (NOBJ > 0) for (; c < eB; c++) normal_row(c, KindTag<KIND_OBJ_PLANE>{});
-                if (ROBOT) for (; c < eA; c++) normal_row(c, KindTag<KIND_ROBOT_TABLE>{});
-                if (ROBOT && NOBJ > 0) for (; c < nc; c++) normal_row(c, KindTag<KIND_GENERIC>{});
+                for (; c < eA; c++) normal_row(c, KindTag<KIND_ROBOT_TABLE>{});
+                if (NOBJ > 0) for (; c < nc; c++) normal_row(c, KindTag<KIND_GENERIC>{});
                 c = 0;
                 if (NOBJ > 0) for (; c < eB; c++) friction_rows(c, KindTag<KIND_OBJ_PLANE>{});
-                if (ROBOT) for (; c < eA; c++) friction_rows(c, KindTag<KIND_ROBOT_TABLE>{});
-                if (ROBOT && NOBJ > 0) for (; c < nc; c++) friction_rows(c, KindTag<KIND_GENERIC>{});
+                for (; c < eA; c++) friction_rows(c, KindTag<KIND_ROBOT_TABLE>{});
+                if (NOBJ > 0) for (; c < nc; c++) friction_rows(c, KindTag<KIND_GENERIC>{});
             }
-            if (ROBOT && robot_contacts) {       // fold this sweep's contact wrench back into the joint velocities: dvq += M^-1 Jx^T F8
+            if (robot_contacts) {       // fold this sweep's contact wrench back into the joint velocities: dvq += M^-1 Jx^T F8
                 T tau[ND];
 #pragma unroll
                 for (int j = 0; j < 7; j++) {
@@ -777,70 +736,9 @@ PG_HD void world_inertia(const Scene<T>& S, int o, World<T, NOBJ>& W) {
     W.Iinv[o][5] = ix * R.X.z * R.X.z + iy * R.Y.z * R.Y.z + iz * R.Z.z * R.Z.z;
 }
 
-// The full sweep (every arm-limit row real) of the env path lives in a separate, NON-INLINED function with its own register allocation:
-// it runs only for envs whose arm limits engage (never in random-action rollouts, sometimes under scripted policies), and inlined next
-// to the watched sweep it cost every env 13-25 % (code size and register allocation of the hot loop: round 1 therefore gave ee control the
-// full sweep for everybody).  What it needs is handed over in a local-memory record; the contact records already sit in shared memory.
-#ifdef __CUDACC__
-#define PG_NOINLINE __noinline__
-#else
-#define PG_NOINLINE __attribute__((noinline))
-#endif
-template <typename T, int NOBJ> struct FullSolveIO {
-    T Minv[ND][ND];
-    JointRows<T> R;
-    T max_imp[ND];
-    OpSpace<T> Op;
-    Obj<T> ob[NOBJ > 0 ? NOBJ : 1];
-    T Iinv[NOBJ > 0 ? NOBJ : 1][6];
-    T dvq[ND]; V3<T> dvl[NOBJ > 0 ? NOBJ : 1], dva[NOBJ > 0 ? NOBJ : 1];     // out
-    int n, nr, nB, nA, ycache;                  // in: the collection's counters
-    int capped, any_limit;                      // out
-};
-template <typename T, int NOBJ, int STRIDE>
-PG_NOINLINE
-#ifdef __CUDACC__
-__host__ __device__
-#endif
-void full_solve(const Scene<T>& S, FullSolveIO<T, NOBJ>& H, T* sbase) {
-    Contacts<T> C; C.st.base = sbase; C.st.stride = STRIDE;
-    C.n = H.n; C.nr = H.nr; C.nB = H.nB; C.nA = H.nA; C.cap = max_contacts(NOBJ); C.dropped = 0; C.near = false; C.capped = false; C.ycache = H.ycache != 0;
-    T Minv[ND][ND], mx[ND];
-#pragma unroll
-    for (int i = 0; i < ND; i++) {
-#pragma unroll
-        for (int j = 0; j < ND; j++) Minv[i][j] = H.Minv[i][j];
-        mx[i] = H.max_imp[i];
-    }
-    World<T, NOBJ> W;
-    Obj<T> ob[NOBJ > 0 ? NOBJ : 1];
-#pragma unroll
-    for (int o = 0; o < NOBJ; o++) {
-        ob[o] = H.ob[o];
-#pragma unroll
-        for (int k = 0; k < 6; k++) W.Iinv[o][k] = H.Iinv[o][k];
-    }
-    JointRows<T> R = H.R;
-    T dvq[ND];
-    V3<T> dvl[NOBJ > 0 ? NOBJ : 1], dva[NOBJ > 0 ? NOBJ : 1];
-#pragma unroll
-    for (int d = 0; d < ND; d++) { dvq[d] = T(0); R.mot_app[d] = T(0); R.lim_app[2 * d] = T(0); R.lim_app[2 * d + 1] = T(0); }
-#pragma unroll
-    for (int o = 0; o < NOBJ; o++) { dvl[o] = mk<T>(0, 0, 0); dva[o] = mk<T>(0, 0, 0); }
-    for (int c = 0; c < C.n; c++) { C.f(c, C_APP) = T(0); C.f(c, C_APP + 1) = T(0); C.f(c, C_APP + 2) = T(0); }
-    pgs_solve<T, NOBJ, false, true>(mx, S, W, H.Op, Minv, R, C, ob, H.nr > 0, dvq, dvl, dva);
-    bool any = false;       // did an arm limit row actually carry impulse?
-#pragma unroll
-    for (int r = 0; r < 14; r++) any = any || R.lim_app[r] > T(0);
-#pragma unroll
-    for (int d = 0; d < ND; d++) H.dvq[d] = dvq[d];
-#pragma unroll
-    for (int o = 0; o < NOBJ; o++) { H.dvl[o] = dvl[o]; H.dva[o] = dva[o]; }
-    H.capped = C.capped; H.any_limit = any;
-}
-
-// WATCH_LIMITS (the env path): watched arm-limit rows inline, the full sweep out of line; !WATCH_LIMITS (bare worlds): the full sweep inline.
-template <typename T, int NOBJ, bool WATCH_LIMITS, bool GENERIC_MOTORS = false, int STRIDE = 1>
+// WATCH_LIMITS (joint control): the arm-limit rows are only watched, and the solve restarts inline with every row real when one would
+// engage; !WATCH_LIMITS (ee control, bare worlds): every row real from the start.
+template <typename T, int NOBJ, bool WATCH_LIMITS, bool GENERIC_MOTORS = false>
 PG_HD void env_substep(const Model<T>& M, const Scene<T>& S, T* q, T* qd, const T* target, Obj<T>* ob, Contacts<T>& C, bool& full_sweep, bool& limits_active,
                        const T* mot = nullptr) {
     T sn[7], cs[7], Minv[ND][ND], qdd[ND];
@@ -884,43 +782,18 @@ PG_HD void env_substep(const Model<T>& M, const Scene<T>& S, T* q, T* qd, const 
 #ifdef PG_HOST_DEBUG
         if (live) g_dbg_fallbacks++;
 #endif
-        if (WATCH_LIMITS && PG_OOL) {     // every row real, from zero impulses, out of line
-            FullSolveIO<T, NOBJ> H;
+        if (live) {
 #pragma unroll
-            for (int i = 0; i < ND; i++) {
+            for (int d = 0; d < ND; d++) { dvq[d] = T(0); R.mot_app[d] = T(0); R.lim_app[2 * d] = T(0); R.lim_app[2 * d + 1] = T(0); }
 #pragma unroll
-                for (int j = 0; j < ND; j++) H.Minv[i][j] = Minv[i][j];
-                H.max_imp[i] = M.max_imp[i];
-            }
-            H.R = R; H.Op = Op;
-#pragma unroll
-            for (int o = 0; o < NOBJ; o++) {
-                H.ob[o] = ob[o];
-#pragma unroll
-                for (int k = 0; k < 6; k++) H.Iinv[o][k] = W.Iinv[o][k];
-            }
-            H.n = C.n; H.nr = C.nr; H.nB = C.nB; H.nA = C.nA; H.ycache = C.ycache;
-            full_solve<T, NOBJ, STRIDE>(S, H, C.st.base);
-#pragma unroll
-            for (int d = 0; d < ND; d++) dvq[d] = H.dvq[d];
-#pragma unroll
-            for (int o = 0; o < NOBJ; o++) { dvl[o] = H.dvl[o]; dva[o] = H.dva[o]; }
-            C.capped = H.capped != 0;
-            limits_active = limits_active || H.any_limit != 0 || live;
-        } else {
-            if (live) {
-#pragma unroll
-                for (int d = 0; d < ND; d++) { dvq[d] = T(0); R.mot_app[d] = T(0); R.lim_app[2 * d] = T(0); R.lim_app[2 * d + 1] = T(0); }
-#pragma unroll
-                for (int o = 0; o < NOBJ; o++) { dvl[o] = mk<T>(0, 0, 0); dva[o] = mk<T>(0, 0, 0); }
-                for (int c = 0; c < C.n; c++) { C.f(c, C_APP) = T(0); C.f(c, C_APP + 1) = T(0); C.f(c, C_APP + 2) = T(0); }
-            }
-            pgs_solve<T, NOBJ, false>(M.max_imp, S, W, Op, Minv, R, C, ob, robot_contacts, dvq, dvl, dva);
-            bool any = false;
-#pragma unroll
-            for (int r = 0; r < 14; r++) any = any || R.lim_app[r] > T(0);
-            limits_active = limits_active || any || live;
+            for (int o = 0; o < NOBJ; o++) { dvl[o] = mk<T>(0, 0, 0); dva[o] = mk<T>(0, 0, 0); }
+            for (int c = 0; c < C.n; c++) { C.f(c, C_APP) = T(0); C.f(c, C_APP + 1) = T(0); C.f(c, C_APP + 2) = T(0); }
         }
+        pgs_solve<T, NOBJ, false>(M.max_imp, S, W, Op, Minv, R, C, ob, robot_contacts, dvq, dvl, dva);
+        bool any = false;
+#pragma unroll
+        for (int r = 0; r < 14; r++) any = any || R.lim_app[r] > T(0);
+        limits_active = limits_active || any || live;
     }
 #pragma unroll
     for (int d = 0; d < ND; d++) { qd[d] += dvq[d]; q[d] += qd[d] * Consts<T>::dt; }

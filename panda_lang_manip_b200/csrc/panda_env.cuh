@@ -194,8 +194,8 @@ PG_HD void step_reward(int reward_type, const float* ag, const double* goal, dou
 
 // The simulation part of RobotTaskEnv.step for one environment, or the sub-step range [s0, s1) of it (a step may be cut into segments so
 // that the envs can be re-sorted in between; the motor targets travel through `target`).  q/qd/ob are updated in place; qc receives the
-// link-transform cache of the last sub-step (valid when s1 == nsub).  STRIDE: word stride of the env's column in the contact store.
-template <typename T, int TASK, int CTRL, int STRIDE>
+// link-transform cache of the last sub-step (valid when s1 == nsub).
+template <typename T, int TASK, int CTRL>
 PG_HD void env_step_sim(const Model<T>& M, const Scene<T>& S, T* q, T* qd, Obj<T>* ob, const float* action, const float* target_quat, Contacts<T>& C, int& sched_key,
                         T* target, T* qc, int s0 = 0, int s1 = 20, int nsub = 20) {
     constexpr int NOBJ = task_nobj(TASK);
@@ -213,10 +213,7 @@ PG_HD void env_step_sim(const Model<T>& M, const Scene<T>& S, T* q, T* qd, Obj<T
             // watched arm-limit rows: a measured policy -- +25 % with joint control, -37..55 % with ee control (contact rows dominate there), so
             // it is enabled for joint control only.  Round 2 re-measured the alternatives (full sweep out of line, watched sweep for ee
             // control, a rolled local-memory fallback inside the one loop: 3-10x slower): profiles/r2_solver_structure_ab.
-#ifndef PG_WATCH_EE
-#define PG_WATCH_EE 0
-#endif
-            env_substep<T, NOBJ, (PG_WATCH_EE || CTRL == CTRL_JOINTS), false, STRIDE>(M, S, q, qd, target, ob, C, full_sweep, limits_active);
+            env_substep<T, NOBJ, CTRL == CTRL_JOINTS>(M, S, q, qd, target, ob, C, full_sweep, limits_active);
             if (C.n > 0) nsub_contact++;
             near = near || C.near;
         }
@@ -233,11 +230,11 @@ PG_HD void env_step_finish(const Model<T>& M, int reward_type, const T* q, const
     step_reward<TASK>(reward_type, ag, goal, thr, reward, success);
 }
 // the whole step (host test build and small callers)
-template <typename T, int TASK, int CTRL, int STRIDE = 1>
+template <typename T, int TASK, int CTRL>
 PG_HD void env_step(const Model<T>& M, const Scene<T>& S, int reward_type, T* q, T* qd, Obj<T>* ob, const double* goal, const float* action, const float* target_quat,
                     float* obs, float* ag, float* dg, float& reward, unsigned char& success, Contacts<T>& C, int& sched_key, T* target, int nsub = 20, double thr = -1.0) {
     T qc[ND];
-    env_step_sim<T, TASK, CTRL, STRIDE>(M, S, q, qd, ob, action, target_quat, C, sched_key, target, qc, 0, nsub, nsub);
+    env_step_sim<T, TASK, CTRL>(M, S, q, qd, ob, action, target_quat, C, sched_key, target, qc, 0, nsub, nsub);
     env_step_finish<T, TASK>(M, reward_type, q, qd, qc, ob, goal, thr < 0.0 ? threshold_f64(TASK) : thr, obs, ag, dg, reward, success);
 }
 

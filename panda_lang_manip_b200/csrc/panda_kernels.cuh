@@ -11,10 +11,8 @@ namespace pg {
 
 constexpr int BLOCK = 128;
 // envs per block of the step kernel (a block is what the SM schedules and frees: smaller blocks release their shared memory and warp
-// slots as soon as their own envs are done); A/B: make EXTRA=-DPG_STEP_BLOCK=32
-#ifndef PG_STEP_BLOCK
-#define PG_STEP_BLOCK 128
-#endif
+// slots as soon as their own envs are done)
+constexpr int STEP_BLOCK = 128;
 
 template <typename T> struct EnvDev {
     int n;                       // environments on this device
@@ -280,7 +278,7 @@ template <int W, typename E> __device__ __forceinline__ void row_store(E* g, int
 // Threads per block: 128, except where the solver slab of 128 envs would exceed the 227 kB a block may own (fp64 parity mode on the
 // two-object scene: 416 slots x 8 B x 128 = 426 kB) -- those run 32-env blocks.
 constexpr size_t SMEM_LIMIT = 227 * 1024;
-template <typename T, int TASK> constexpr int step_block() { return (size_t)solver_slots(task_nobj(TASK)) * PG_STEP_BLOCK * sizeof(T) <= SMEM_LIMIT ? PG_STEP_BLOCK : 32; }
+template <typename T, int TASK> constexpr int step_block() { return (size_t)solver_slots(task_nobj(TASK)) * STEP_BLOCK * sizeof(T) <= SMEM_LIMIT ? STEP_BLOCK : 32; }
 template <typename T, int TASK, int CTRL> constexpr size_t step_smem_bytes() {
     constexpr int O = task_obs_dim(TASK), G = task_goal_dim(TASK), NA = task_act_dim(TASK, CTRL), BS = step_block<T, TASK>();
     constexpr int W = O > NA ? (O > G ? O : G) : (NA > G ? NA : G);
@@ -319,7 +317,7 @@ __global__ void __launch_bounds__((step_block<T, TASK>())) step_kernel(const __g
         float tquat[4];
         if (first && io.target_quat) row_load<4>(io.target_quat, i, tquat);
         const long long clk0 = E.dbg ? clock64() : 0;
-        env_step_sim<T, TASK, CTRL, BS>(E.M, E.S, q, qd, ob, act, (first && io.target_quat) ? tquat : nullptr, C, sched_key, target, qc, io.s0, io.s1, E.P.nsub);
+        env_step_sim<T, TASK, CTRL>(E.M, E.S, q, qd, ob, act, (first && io.target_quat) ? tquat : nullptr, C, sched_key, target, qc, io.s0, io.s1, E.P.nsub);
         if (E.dbg) { E.dbg[2 * (size_t)(E.t0 + t)] = clock64() - clk0; unsigned smid; asm volatile("mov.u32 %0, %%smid;" : "=r"(smid)); E.dbg[2 * (size_t)(E.t0 + t) + 1] = (long long)sched_key | ((long long)smid << 16); }
         if (C.dropped > 0) atomicAdd(&s_stats[5], (double)C.dropped);
         if (last) {     // the report of the step that just ended: the records are still in this thread's column of the slab, before any reset
@@ -583,12 +581,12 @@ template <typename E, int G, int VB> struct RowLoad {
         }
     }
 };
-constexpr int HER_INFLIGHT = 4;      // default; PG_HER_INFLIGHT=1|2|4|8 selects another instantiation (A/B)
-template <typename E, int TASK, int VB, int HT = HER_INFLIGHT>
+constexpr int HER_INFLIGHT = 4;      // transitions in flight per thread (two row gathers each)
+template <typename E, int TASK, int VB>
 __global__ void __launch_bounds__(256) her_relabel_kernel(const E* __restrict__ next_ag, const E* __restrict__ dg, const long long* __restrict__ src,
                                                           const long long* __restrict__ goal_src, E* __restrict__ dg_out, E* __restrict__ ag_out,
                                                           float* __restrict__ reward, long long m, long long pitch, int reward_type, double threshold) {
-    constexpr int G = task_goal_dim(TASK);
+    constexpr int G = task_goal_dim(TASK), HT = HER_INFLIGHT;
     using RL = RowLoad<E, G, VB>;
     const E thr = (E)threshold;
     const long long stride = (long long)gridDim.x * blockDim.x;
