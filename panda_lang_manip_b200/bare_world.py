@@ -8,15 +8,12 @@ import numpy as np
 import torch
 
 from . import _lib
+from .vec_env import _Handle, _ptr
 
 JOINT_TO_DOF = {0: 0, 1: 1, 2: 2, 3: 3, 4: 4, 5: 5, 6: 6, 9: 7, 10: 8}
 
 
-def _ptr(t):
-    return None if t is None else t.data_ptr()
-
-
-class PandaBareWorld:
+class PandaBareWorld(_Handle):
     """num_envs worlds: Panda at ``robot_base`` (None: no robot), up to two free bodies, optional table top (z = 0) and ground plane.
 
     ``bodies``: sequence of dicts ``{"shape": "box"|"cylinder", "half_extents": (hx,hy,hz) | "radius"/"height", "mass", "position",
@@ -50,20 +47,6 @@ class PandaBareWorld:
         self._h = h
         self.state_dim = 18 + 13 * self.n_bodies + 1
 
-    def close(self) -> None:
-        if getattr(self, "_h", None) is not None:
-            self.lib.pg_destroy(self._h)
-            self._h = None
-
-    def __del__(self):
-        try:
-            self.close()
-        except Exception:
-            pass
-
-    def _stream(self):
-        return torch.cuda.current_stream(self.device).cuda_stream
-
     # ---- PyBullet.step / control_joints ---------------------------------------------------------------------------------------------
     def step(self, n_substeps: int = 20) -> None:
         """pybullet.py:52-55: n_substeps x stepSimulation (1/500 s each)."""
@@ -89,24 +72,6 @@ class PandaBareWorld:
             m[:, d, 0], m[:, d, 1], m[:, d, 2], m[:, d, 3], m[:, d, 4] = 0.1, 1.0, float(a), 0.0, float(f)
         self.set_motors(m)
 
-    # ---- state ----------------------------------------------------------------------------------------------------------------------
-    def get_state(self) -> torch.Tensor:
-        """[N, 18 + 13 n_bodies + 1] float64: q(9) qd(9) | per body pos3 quat4 lin3 ang3 | step counter."""
-        s = torch.empty((self.num_envs, self.state_dim), dtype=torch.float64, device=self.device)
-        _lib.check(self.lib.pg_get_state(self._h, _ptr(s), self._stream()))
-        return s
-
-    def set_state(self, state: torch.Tensor, mask: Optional[torch.Tensor] = None) -> None:
-        s = state.to(device=self.device, dtype=torch.float64).contiguous()
-        m = None if mask is None else mask.to(device=self.device, dtype=torch.uint8).contiguous()
-        _lib.check(self.lib.pg_set_state(self._h, _ptr(s), _ptr(m), self._stream()))
-        torch.cuda.current_stream(self.device).synchronize()
-
-    def link_state(self, link: int) -> torch.Tensor:
-        out = torch.empty((self.num_envs, 13), dtype=torch.float64, device=self.device)
-        _lib.check(self.lib.pg_get_link_state(self._h, int(link), _ptr(out), self._stream()))
-        return out
-
     def inverse_kinematics(self, link: int, position, orientation) -> torch.Tensor:
         p = torch.as_tensor(np.asarray(position, dtype=np.float64), device=self.device).expand(self.num_envs, 3).contiguous()
         o = torch.as_tensor(np.asarray(orientation, dtype=np.float64), device=self.device).expand(self.num_envs, 4).contiguous()
@@ -114,20 +79,3 @@ class PandaBareWorld:
         _lib.check(self.lib.pg_inverse_kinematics_link(self._h, int(link), _ptr(p), _ptr(o), _ptr(out), self._stream()))
         torch.cuda.current_stream(self.device).synchronize()
         return out
-
-    def render(self, *args, **kwargs):
-        """As PandaVecEnv.render: depth / colour / point cloud of every world (pg_render)."""
-        from .vec_env import PandaVecEnv
-        return PandaVecEnv.render(self, *args, **kwargs)
-
-    def save_state(self) -> int:
-        import ctypes
-        sid = ctypes.c_int()
-        _lib.check(self.lib.pg_save_state_async(self._h, ctypes.byref(sid), self._stream()))
-        return sid.value
-
-    def restore_state(self, state_id: int) -> None:
-        _lib.check(self.lib.pg_restore_state_async(self._h, int(state_id), self._stream()))
-
-    def remove_state(self, state_id: int) -> None:
-        _lib.check(self.lib.pg_remove_state(self._h, int(state_id)))

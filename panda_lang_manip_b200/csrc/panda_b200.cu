@@ -7,6 +7,7 @@
 #include <algorithm>
 #include <map>
 #include <string>
+#include <type_traits>
 #include <vector>
 #include "panda_b200.h"
 #include "panda_kernels.cuh"
@@ -32,29 +33,19 @@ void launch_render(const RenderPrim* prims, const RenderCamera& C, int n_envs, f
 PG_DECL(float, 0) PG_DECL(float, 1) PG_DECL(float, 2) PG_DECL(float, 3) PG_DECL(float, 4) PG_DECL(float, 5)
 PG_DECL(double, 0) PG_DECL(double, 1) PG_DECL(double, 2) PG_DECL(double, 3) PG_DECL(double, 4) PG_DECL(double, 5)
 
-template <typename T> struct Dispatch {
-    static void step(int task, const EnvDev<T>& E, int ctrl, const StepIO& io, cudaStream_t st) {
-        switch (task) {
-        case 0: launch_step<T, 0>(E, ctrl, io, st); break; case 1: launch_step<T, 1>(E, ctrl, io, st); break;
-        case 2: launch_step<T, 2>(E, ctrl, io, st); break; case 3: launch_step<T, 3>(E, ctrl, io, st); break;
-        case 4: launch_step<T, 4>(E, ctrl, io, st); break; default: launch_step<T, 5>(E, ctrl, io, st); break;
-        }
-    }
-    static void reset(int task, const EnvDev<T>& E, const ResetIO& io, cudaStream_t st) {
-        switch (task) {
-        case 0: launch_reset<T, 0>(E, io, st); break; case 1: launch_reset<T, 1>(E, io, st); break;
-        case 2: launch_reset<T, 2>(E, io, st); break; case 3: launch_reset<T, 3>(E, io, st); break;
-        case 4: launch_reset<T, 4>(E, io, st); break; default: launch_reset<T, 5>(E, io, st); break;
-        }
-    }
-    static cudaError_t configure(int task) {
-        switch (task) {
-        case 0: return configure_step<T, 0>(); case 1: return configure_step<T, 1>(); case 2: return configure_step<T, 2>();
-        case 3: return configure_step<T, 3>(); case 4: return configure_step<T, 4>(); case 5: return configure_step<T, 5>();
-        default: return configure_bare<T>();
-        }
-    }
-};
+// The kernels are templates over the task: calls f(std::integral_constant<int, K>()) for the K of Ks equal to the runtime id
+// (nothing if none is).  Only the listed Ks are instantiated.
+template <int... Ks, typename F> static void dispatch(int id, F&& f) {
+    (void)((id == Ks && (f(std::integral_constant<int, Ks>()), true)) || ...);
+}
+// goal layouts: 3-D position (tasks 0-3, thr 0.05), Stack 6-D (thr 0.1), Flip quaternion (thr 0.2); the goal kernels exist per layout
+static int goal_layout(int task) { return task == TASK_STACK || task == TASK_FLIP ? task : 0; }
+// f(float()) for PG_F32 goal arrays, f(double()) otherwise
+template <typename F> static auto with_dtype(int dtype, F&& f) { return dtype == PG_F32 ? f(float()) : f(double()); }
+static bool valid_task(int task) { return task >= 0 && task <= 5; }
+static bool valid_reward_type(int reward_type) { return reward_type >= 0 && reward_type <= 1; }
+// the reference's distance_threshold of a task; 0.0 for a bad task, which the _t form then rejects
+static double default_threshold(int task) { return valid_task(task) ? threshold_f64(task) : 0.0; }
 }  // namespace pg
 
 using namespace pg;
@@ -77,6 +68,26 @@ struct pg_env {
     float *h_act = nullptr, *h_out = nullptr; float* d_act = nullptr; float* d_out = nullptr; size_t out_floats = 0; size_t out_bytes = 0;
 };
 
+// f(E) with the handle's bound state: Ef for PG_F32 handles, Ed for PG_F64 ones.  Only that copy points at device memory (the
+// other one's pointers are NULL), so every read of a handle's device state goes through here.
+template <typename F> static auto with_env(pg_env* e, F&& f) { return e->precision == PG_F32 ? f(e->Ef) : f(e->Ed); }
+// One thread per env on `stream`: f(E, grid, st) launches a BLOCK-wide kernel over the bound state E.
+template <typename F> static int launch_per_env(pg_env* e, void* stream, F&& f) {
+    PG_CUDA(cudaSetDevice(e->device));
+    const int grid = (e->n + BLOCK - 1) / BLOCK;
+    with_env(e, [&](auto& E) { f(E, grid, (cudaStream_t)stream); });
+    g_launches++;
+    PG_CUDA(cudaGetLastError());
+    return PG_OK;
+}
+// stats[first, first + count) to the host (see EnvDev::stats)
+static int read_stats(pg_env* e, int first, int count, double* out) {
+    PG_CUDA(cudaSetDevice(e->device));
+    const double* stats = with_env(e, [](auto& E) { return E.stats; });
+    PG_CUDA(cudaMemcpy(out, stats + first, count * sizeof(double), cudaMemcpyDeviceToHost));
+    return PG_OK;
+}
+
 template <typename T> static void bind(EnvDev<T>& E, pg_env* e, char* base, unsigned long long seed, long long id0) {
     const size_t n = (size_t)e->n;
     E.n = e->n; E.reward_type = e->reward; E.id0 = id0; E.seed = seed;
@@ -98,11 +109,9 @@ template <typename E, bool WANT_REWARD> static void launch_reward(int task, cons
     const int vec_ok = (((uintptr_t)ag | (uintptr_t)dg) & 15) == 0;
     long long blocks = (m / 2 + 255) / 256 + 1;
     int grid = (int)(blocks < 148LL * 32 ? blocks : 148LL * 32);   // grid-stride; capped at a multiple of the SM count
-    switch (task) {
-    case 4: reward_kernel<E, 4, WANT_REWARD><<<grid, 256, 0, st>>>(ag, dg, reward, success, m, reward_type, vec_ok, thr); break;
-    case 5: reward_kernel<E, 5, WANT_REWARD><<<grid, 256, 0, st>>>(ag, dg, reward, success, m, reward_type, vec_ok, thr); break;
-    default: reward_kernel<E, 0, WANT_REWARD><<<grid, 256, 0, st>>>(ag, dg, reward, success, m, reward_type, vec_ok, thr); break;   // all 3-D position goals share thr 0.05
-    }
+    dispatch<0, 4, 5>(goal_layout(task), [&](auto L) {
+        reward_kernel<E, L, WANT_REWARD><<<grid, 256, 0, st>>>(ag, dg, reward, success, m, reward_type, vec_ok, thr);
+    });
     g_launches++;
 }
 
@@ -128,11 +137,68 @@ template <typename E, int TASK> static void launch_her_task(const E* next_ag, co
 }
 template <typename E> static void launch_her(int task, const E* next_ag, const E* dg, const long long* src, const long long* goal_src, E* dg_out, E* ag_out, float* reward,
                                              long long m, long long pitch, int reward_type, double thr, cudaStream_t st) {
-    switch (task) {     // goal layouts: 3-D position (thr 0.05), Stack 6-D (thr 0.1), Flip quaternion (thr 0.2)
-    case 4: launch_her_task<E, 4>(next_ag, dg, src, goal_src, dg_out, ag_out, reward, m, pitch, reward_type, thr, st); break;
-    case 5: launch_her_task<E, 5>(next_ag, dg, src, goal_src, dg_out, ag_out, reward, m, pitch, reward_type, thr, st); break;
-    default: launch_her_task<E, 0>(next_ag, dg, src, goal_src, dg_out, ag_out, reward, m, pitch, reward_type, thr, st); break;
+    dispatch<0, 4, 5>(goal_layout(task), [&](auto L) {
+        launch_her_task<E, L>(next_ag, dg, src, goal_src, dg_out, ag_out, reward, m, pitch, reward_type, thr, st);
+    });
+}
+
+// Host-buffer mode of a step (pg_step_host): every env group copies its own action rows in before its first launch and its own
+// output rows out after its last one, on its own stream -- group g's device-to-host copies overlap group g+1's kernels.
+struct HostIO { const float* act; float* obs; float* ag; float* dg; float* rew; unsigned char* term; unsigned char* trunc; };
+// E: a copy of the handle's bound state, adjusted per launch
+template <typename T> static int step_impl(pg_env* e, EnvDev<T> E, const float* actions, const float* target_quat, float* obs, float* ag, float* dg, float* reward,
+                                           unsigned char* terminated, unsigned char* truncated, int auto_reset, float* contacts, unsigned char* contact_count,
+                                           cudaStream_t stream, const HostIO* hio) {
+    PG_CUDA(cudaSetDevice(e->device));
+    // Contact-aware scheduling (see perm_*_kernel): large batches are re-sorted by their contact state before every launch, and a
+    // step is cut into `segments` launches of consecutive sub-steps so that envs which make contact mid-step are regrouped; small
+    // batches keep the identity map, one launch per step and the tiled I/O path.  Results do not depend on either choice.
+    const bool use_perm = e->n >= 4096;
+    const int segs = use_perm ? e->segments : 1;
+    const unsigned short* key = E.ccount;
+    int* hist = E.hist;
+    int* perm = E.perm;
+    if (!use_perm) E.perm = nullptr;
+    // host mode pipelines the copies against the env groups the configuration already has (measured: on one GPU the single-stream
+    // Reach-joints configuration loses 5 % when cut into 4 groups only to overlap 0.2 ms of copies)
+    const int groups = use_perm ? e->groups : 1;
+    // group g owns the envs (and thread slots) [g * gsize, min(n, (g + 1) * gsize)), gsize a multiple of the sort chunk
+    const int gsize = ((e->n + groups - 1) / groups + PERM_CHUNK - 1) / PERM_CHUNK * PERM_CHUNK;
+    const size_t A = e->act_dim, O = e->obs_dim, G = e->goal_dim;
+    if (groups > 1) PG_CUDA(cudaEventRecord(e->ev_fork, stream));
+    for (int g = 0; g < groups; g++) {
+        const int t0 = g * gsize, cnt = std::min(e->n, t0 + gsize) - t0;
+        if (cnt <= 0) break;
+        cudaStream_t st = groups > 1 ? e->gstream[g] : stream;
+        if (groups > 1) PG_CUDA(cudaStreamWaitEvent(st, e->ev_fork, 0));
+        if (hio) PG_CUDA(cudaMemcpyAsync(const_cast<float*>(actions) + t0 * A, hio->act + t0 * A, (size_t)cnt * A * sizeof(float), cudaMemcpyHostToDevice, st));
+        E.t0 = t0; E.tcount = cnt;
+        const int nchunks = (cnt + PERM_CHUNK - 1) / PERM_CHUNK;
+        int* ghist = hist + (size_t)(t0 / PERM_CHUNK + g) * PERM_BUCKETS;
+        const int nsub = E.P.nsub;
+        for (int sg = 0; sg < segs; sg++) {
+            StepIO io{target_quat, actions, obs, ag, dg, reward, terminated, truncated, auto_reset, sg * nsub / segs, (sg + 1) * nsub / segs,
+                      contacts, contact_count};
+            if (io.s0 == io.s1) continue;       // fewer sub-steps than segments
+            if (use_perm) {
+                perm_hist_kernel<<<nchunks, PERM_THREADS, 0, st>>>(key + t0, ghist, cnt);
+                perm_scatter_kernel<<<nchunks, PERM_THREADS, 0, st>>>(key + t0, ghist, perm + t0, cnt, nchunks, t0);
+                g_launches += 2;
+            }
+            dispatch<0, 1, 2, 3, 4, 5>(e->task, [&](auto K) { launch_step<T, K>(E, e->ctrl, io, st); });
+        }
+        if (hio) {
+            if (hio->obs) PG_CUDA(cudaMemcpyAsync(hio->obs + t0 * O, obs + t0 * O, (size_t)cnt * O * sizeof(float), cudaMemcpyDeviceToHost, st));
+            if (hio->ag) PG_CUDA(cudaMemcpyAsync(hio->ag + t0 * G, ag + t0 * G, (size_t)cnt * G * sizeof(float), cudaMemcpyDeviceToHost, st));
+            if (hio->dg) PG_CUDA(cudaMemcpyAsync(hio->dg + t0 * G, dg + t0 * G, (size_t)cnt * G * sizeof(float), cudaMemcpyDeviceToHost, st));
+            if (hio->rew) PG_CUDA(cudaMemcpyAsync(hio->rew + t0, reward + t0, (size_t)cnt * sizeof(float), cudaMemcpyDeviceToHost, st));
+            if (hio->term) PG_CUDA(cudaMemcpyAsync(hio->term + t0, terminated + t0, (size_t)cnt, cudaMemcpyDeviceToHost, st));
+            if (hio->trunc) PG_CUDA(cudaMemcpyAsync(hio->trunc + t0, truncated + t0, (size_t)cnt, cudaMemcpyDeviceToHost, st));
+        }
+        if (groups > 1) { PG_CUDA(cudaEventRecord(e->ev_join[g], st)); PG_CUDA(cudaStreamWaitEvent(stream, e->ev_join[g], 0)); }
     }
+    PG_CUDA(cudaGetLastError());
+    return PG_OK;
 }
 
 extern "C" {
@@ -150,22 +216,26 @@ static int check_device(int device, const char* who) {
 }
 // state allocation + model; the caller fills the scene
 static int alloc_state(pg_env* e, unsigned long long seed, long long env_id_offset, const double base[3]) {
-    if (e->precision == PG_F32) { bind(e->Ef, e, nullptr, seed, env_id_offset); } else { bind(e->Ed, e, nullptr, seed, env_id_offset); }
-    cudaError_t err = cudaMalloc(&e->blob, e->blob_bytes);
-    if (err != cudaSuccess) return cuda_fail(err, "cudaMalloc(state)");
-    PG_CUDA(cudaMemset(e->blob, 0, e->blob_bytes));
-    if (e->precision == PG_F32) { bind(e->Ef, e, (char*)e->blob, seed, env_id_offset); e->Ef.M = make_model<float>(base); }
-    else { bind(e->Ed, e, (char*)e->blob, seed, env_id_offset); e->Ed.M = make_model<double>(base); }
-    // the > 48 kB dynamic shared memory opt-in is per function and per device: done for this handle's device, errors reported
-    cudaError_t ce = e->precision == PG_F32 ? Dispatch<float>::configure(e->task) : Dispatch<double>::configure(e->task);
-    if (ce != cudaSuccess) return cuda_fail(ce, "cudaFuncSetAttribute(step kernel shared memory)");
-    return PG_OK;
+    return with_env(e, [&](auto& E) -> int {
+        using T = std::remove_pointer_t<decltype(E.q)>;
+        bind(E, e, nullptr, seed, env_id_offset);
+        cudaError_t err = cudaMalloc(&e->blob, e->blob_bytes);
+        if (err != cudaSuccess) return cuda_fail(err, "cudaMalloc(state)");
+        PG_CUDA(cudaMemset(e->blob, 0, e->blob_bytes));
+        bind(E, e, (char*)e->blob, seed, env_id_offset); E.M = make_model<T>(base);
+        // the > 48 kB dynamic shared memory opt-in is per function and per device: done for this handle's device, errors reported
+        cudaError_t ce = cudaSuccess;
+        if (e->task == PG_TASK_BARE) ce = configure_bare<T>();
+        else dispatch<0, 1, 2, 3, 4, 5>(e->task, [&](auto K) { ce = configure_step<T, K>(); });
+        if (ce != cudaSuccess) return cuda_fail(ce, "cudaFuncSetAttribute(step kernel shared memory)");
+        return PG_OK;
+    });
 }
 
 int pg_create(int task, int control_type, int reward_type, int num_envs, int device, unsigned long long seed, long long env_id_offset,
               int precision, pg_env** out) {
     if (!out) return fail(PG_ERR_ARG, "pg_create: out is NULL");
-    if (task < 0 || task > 5 || control_type < 0 || control_type > 1 || reward_type < 0 || reward_type > 1 || num_envs <= 0 || precision < 0 || precision > 1)
+    if (!valid_task(task) || control_type < 0 || control_type > 1 || !valid_reward_type(reward_type) || num_envs <= 0 || precision < 0 || precision > 1)
         return fail(PG_ERR_ARG, "pg_create: bad task / control_type / reward_type / num_envs / precision");
     int rc = check_device(device, "pg_create"); if (rc != PG_OK) return rc;
     pg_env* e = new pg_env();
@@ -282,7 +352,10 @@ int pg_reset_seeded(pg_env* e, const unsigned char* mask, const unsigned long lo
     if (e->task == PG_TASK_BARE) return fail(PG_ERR_ARG, "pg_reset: a bare world has no task to reset; use pg_set_state");
     PG_CUDA(cudaSetDevice(e->device));
     ResetIO io{mask, goal_override, object_override, obs, ag, dg, seeds};
-    if (e->precision == PG_F32) Dispatch<float>::reset(e->task, e->Ef, io, (cudaStream_t)stream); else Dispatch<double>::reset(e->task, e->Ed, io, (cudaStream_t)stream);
+    with_env(e, [&](auto& E) {
+        using T = std::remove_pointer_t<decltype(E.q)>;
+        dispatch<0, 1, 2, 3, 4, 5>(e->task, [&](auto K) { launch_reset<T, K>(E, io, (cudaStream_t)stream); });
+    });
     PG_CUDA(cudaGetLastError());
     return PG_OK;
 }
@@ -299,7 +372,7 @@ int pg_set_action_scale(pg_env* e, double ee_scale, double finger_scale) {
 int pg_set_task_params(pg_env* e, double distance_threshold, const double* goal_range_low, const double* goal_range_high, const double* obj_range_low, const double* obj_range_high) {
     if (!e || e->task == PG_TASK_BARE) return fail(PG_ERR_ARG, "pg_set_task_params: needs a task handle");
     if (!(distance_threshold >= 0)) return fail(PG_ERR_ARG, "pg_set_task_params: distance_threshold must be >= 0");
-    TaskParams P = e->Ef.P;
+    TaskParams P = with_env(e, [](auto& E) { return E.P; });
     P.thr64 = distance_threshold; P.thr32 = (float)distance_threshold;
     for (int k = 0; k < 3; k++) { if (goal_range_low) P.goal_lo[k] = goal_range_low[k]; if (goal_range_high) P.goal_hi[k] = goal_range_high[k]; }
     for (int k = 0; k < 2; k++) { if (obj_range_low) P.obj_lo[k] = obj_range_low[k]; if (obj_range_high) P.obj_hi[k] = obj_range_high[k]; }
@@ -314,69 +387,14 @@ int pg_set_substeps(pg_env* e, int n_substeps) {
     e->Ef.P.nsub = e->Ed.P.nsub = n_substeps;
     return PG_OK;
 }
-// Host-buffer mode of a step (pg_step_host): every env group copies its own action rows in before its first launch and its own
-// output rows out after its last one, on its own stream -- group g's device-to-host copies overlap group g+1's kernels.
-struct HostIO { const float* act; float* obs; float* ag; float* dg; float* rew; unsigned char* term; unsigned char* trunc; };
-static int step_impl(pg_env* e, const float* actions, const float* target_quat, float* obs, float* ag, float* dg, float* reward, unsigned char* terminated,
-                     unsigned char* truncated, int auto_reset, float* contacts, unsigned char* contact_count, cudaStream_t stream, const HostIO* hio) {
-    PG_CUDA(cudaSetDevice(e->device));
-    // Contact-aware scheduling (see perm_*_kernel): large batches are re-sorted by their contact state before every launch, and a
-    // step is cut into `segments` launches of consecutive sub-steps so that envs which make contact mid-step are regrouped; small
-    // batches keep the identity map, one launch per step and the tiled I/O path.  Results do not depend on either choice.
-    const bool use_perm = e->n >= 4096;
-    const int segs = use_perm ? e->segments : 1;
-    const unsigned short* key = e->precision == PG_F32 ? e->Ef.ccount : e->Ed.ccount;
-    int* hist = e->precision == PG_F32 ? e->Ef.hist : e->Ed.hist;
-    int* perm = e->precision == PG_F32 ? e->Ef.perm : e->Ed.perm;
-    EnvDev<float> Ef = e->Ef; EnvDev<double> Ed = e->Ed;
-    if (!use_perm) { Ef.perm = nullptr; Ed.perm = nullptr; }
-    // host mode pipelines the copies against the env groups the configuration already has (measured: on one GPU the single-stream
-    // Reach-joints configuration loses 5 % when cut into 4 groups only to overlap 0.2 ms of copies)
-    const int groups = use_perm ? e->groups : 1;
-    // group g owns the envs (and thread slots) [g * gsize, min(n, (g + 1) * gsize)), gsize a multiple of the sort chunk
-    const int gsize = ((e->n + groups - 1) / groups + PERM_CHUNK - 1) / PERM_CHUNK * PERM_CHUNK;
-    const size_t A = e->act_dim, O = e->obs_dim, G = e->goal_dim;
-    if (groups > 1) PG_CUDA(cudaEventRecord(e->ev_fork, stream));
-    for (int g = 0; g < groups; g++) {
-        const int t0 = g * gsize, cnt = std::min(e->n, t0 + gsize) - t0;
-        if (cnt <= 0) break;
-        cudaStream_t st = groups > 1 ? e->gstream[g] : stream;
-        if (groups > 1) PG_CUDA(cudaStreamWaitEvent(st, e->ev_fork, 0));
-        if (hio) PG_CUDA(cudaMemcpyAsync(const_cast<float*>(actions) + t0 * A, hio->act + t0 * A, (size_t)cnt * A * sizeof(float), cudaMemcpyHostToDevice, st));
-        Ef.t0 = Ed.t0 = t0; Ef.tcount = Ed.tcount = cnt;
-        const int nchunks = (cnt + PERM_CHUNK - 1) / PERM_CHUNK;
-        int* ghist = hist + (size_t)(t0 / PERM_CHUNK + g) * PERM_BUCKETS;
-        const int nsub = e->Ef.P.nsub;
-        for (int sg = 0; sg < segs; sg++) {
-            StepIO io{target_quat, actions, obs, ag, dg, reward, terminated, truncated, auto_reset, sg * nsub / segs, (sg + 1) * nsub / segs,
-                      contacts, contact_count};
-            if (io.s0 == io.s1) continue;       // fewer sub-steps than segments
-            if (use_perm) {
-                perm_hist_kernel<<<nchunks, PERM_THREADS, 0, st>>>(key + t0, ghist, cnt);
-                perm_scatter_kernel<<<nchunks, PERM_THREADS, 0, st>>>(key + t0, ghist, perm + t0, cnt, nchunks, t0);
-                g_launches += 2;
-            }
-            if (e->precision == PG_F32) Dispatch<float>::step(e->task, Ef, e->ctrl, io, st); else Dispatch<double>::step(e->task, Ed, e->ctrl, io, st);
-        }
-        if (hio) {
-            if (hio->obs) PG_CUDA(cudaMemcpyAsync(hio->obs + t0 * O, obs + t0 * O, (size_t)cnt * O * sizeof(float), cudaMemcpyDeviceToHost, st));
-            if (hio->ag) PG_CUDA(cudaMemcpyAsync(hio->ag + t0 * G, ag + t0 * G, (size_t)cnt * G * sizeof(float), cudaMemcpyDeviceToHost, st));
-            if (hio->dg) PG_CUDA(cudaMemcpyAsync(hio->dg + t0 * G, dg + t0 * G, (size_t)cnt * G * sizeof(float), cudaMemcpyDeviceToHost, st));
-            if (hio->rew) PG_CUDA(cudaMemcpyAsync(hio->rew + t0, reward + t0, (size_t)cnt * sizeof(float), cudaMemcpyDeviceToHost, st));
-            if (hio->term) PG_CUDA(cudaMemcpyAsync(hio->term + t0, terminated + t0, (size_t)cnt, cudaMemcpyDeviceToHost, st));
-            if (hio->trunc) PG_CUDA(cudaMemcpyAsync(hio->trunc + t0, truncated + t0, (size_t)cnt, cudaMemcpyDeviceToHost, st));
-        }
-        if (groups > 1) { PG_CUDA(cudaEventRecord(e->ev_join[g], st)); PG_CUDA(cudaStreamWaitEvent(stream, e->ev_join[g], 0)); }
-    }
-    PG_CUDA(cudaGetLastError());
-    return PG_OK;
-}
 int pg_step_contacts(pg_env* e, const float* actions, const float* target_quat, float* obs, float* ag, float* dg, float* reward, unsigned char* terminated,
                      unsigned char* truncated, int auto_reset, float* contacts, unsigned char* contact_count, void* stream) {
     if (!e || !actions) return fail(PG_ERR_ARG, "pg_step: NULL handle or actions");
     if (e->task == PG_TASK_BARE) return fail(PG_ERR_ARG, "pg_step: a bare world is advanced with pg_sim_step");
     if (target_quat && e->ctrl != CTRL_EE) return fail(PG_ERR_ARG, "pg_step_oriented: a target orientation needs ee control");
-    return step_impl(e, actions, target_quat, obs, ag, dg, reward, terminated, truncated, auto_reset, contacts, contact_count, (cudaStream_t)stream, nullptr);
+    return with_env(e, [&](auto& E) {
+        return step_impl(e, E, actions, target_quat, obs, ag, dg, reward, terminated, truncated, auto_reset, contacts, contact_count, (cudaStream_t)stream, nullptr);
+    });
 }
 int pg_step_oriented(pg_env* e, const float* actions, const float* target_quat, float* obs, float* ag, float* dg, float* reward, unsigned char* terminated,
                      unsigned char* truncated, int auto_reset, void* stream) {
@@ -440,7 +458,8 @@ int pg_step_host(pg_env* e, const float* actions, float* obs, float* ag, float* 
         o.host = o.direct ? o.user : (void*)((char*)e->h_out + ((const char*)o.dev - (const char*)e->d_out));
     }
     HostIO hio{src, (float*)outs[0].host, (float*)outs[1].host, (float*)outs[2].host, (float*)outs[3].host, (unsigned char*)outs[4].host, (unsigned char*)outs[5].host};
-    rc = step_impl(e, e->d_act, nullptr, d_obs, d_ag, d_dg, d_rew, d_term, d_trunc, auto_reset, nullptr, nullptr, e->hstream, &hio); if (rc != PG_OK) return rc;
+    rc = with_env(e, [&](auto& E) { return step_impl(e, E, e->d_act, nullptr, d_obs, d_ag, d_dg, d_rew, d_term, d_trunc, auto_reset, nullptr, nullptr, e->hstream, &hio); });
+    if (rc != PG_OK) return rc;
     PG_CUDA(cudaStreamSynchronize(e->hstream));
     for (const Out& o : outs) if (o.user && !o.direct) memcpy(o.user, o.host, o.bytes);
     return PG_OK;
@@ -448,44 +467,50 @@ int pg_step_host(pg_env* e, const float* actions, float* obs, float* ag, float* 
 
 int pg_compute_reward_t(int task, int reward_type, double threshold, const void* ag, const void* dg, float* reward, long long m, int dtype, void* stream) {
     if (m == 0) return PG_OK;       // an empty batch is valid (its pointers may be NULL)
-    if (task < 0 || task > 5 || reward_type < 0 || reward_type > 1 || !ag || !dg || !reward || m < 0 || !(threshold >= 0)) return fail(PG_ERR_ARG, "pg_compute_reward: bad argument");
-    if (dtype == PG_F32) launch_reward<float, true>(task, (const float*)ag, (const float*)dg, reward, nullptr, m, reward_type, threshold, (cudaStream_t)stream);
-    else launch_reward<double, true>(task, (const double*)ag, (const double*)dg, reward, nullptr, m, reward_type, threshold, (cudaStream_t)stream);
+    if (!valid_task(task) || !valid_reward_type(reward_type) || !ag || !dg || !reward || m < 0 || !(threshold >= 0)) return fail(PG_ERR_ARG, "pg_compute_reward: bad argument");
+    with_dtype(dtype, [&](auto x) {
+        using E = decltype(x);
+        launch_reward<E, true>(task, (const E*)ag, (const E*)dg, reward, nullptr, m, reward_type, threshold, (cudaStream_t)stream);
+    });
     PG_CUDA(cudaGetLastError());
     return PG_OK;
 }
 int pg_is_success_t(int task, double threshold, const void* ag, const void* dg, unsigned char* success, long long m, int dtype, void* stream) {
     if (m == 0) return PG_OK;
-    if (task < 0 || task > 5 || !ag || !dg || !success || m < 0 || !(threshold >= 0)) return fail(PG_ERR_ARG, "pg_is_success: bad argument");
-    if (dtype == PG_F32) launch_reward<float, false>(task, (const float*)ag, (const float*)dg, nullptr, success, m, 0, threshold, (cudaStream_t)stream);
-    else launch_reward<double, false>(task, (const double*)ag, (const double*)dg, nullptr, success, m, 0, threshold, (cudaStream_t)stream);
+    if (!valid_task(task) || !ag || !dg || !success || m < 0 || !(threshold >= 0)) return fail(PG_ERR_ARG, "pg_is_success: bad argument");
+    with_dtype(dtype, [&](auto x) {
+        using E = decltype(x);
+        launch_reward<E, false>(task, (const E*)ag, (const E*)dg, nullptr, success, m, 0, threshold, (cudaStream_t)stream);
+    });
     PG_CUDA(cudaGetLastError());
     return PG_OK;
 }
 int pg_compute_reward(int task, int reward_type, const void* ag, const void* dg, float* reward, long long m, int dtype, void* stream) {
-    return pg_compute_reward_t(task, reward_type, task >= 0 && task <= 5 ? threshold_f64(task) : 0.0, ag, dg, reward, m, dtype, stream);
+    return pg_compute_reward_t(task, reward_type, default_threshold(task), ag, dg, reward, m, dtype, stream);
 }
 int pg_is_success(int task, const void* ag, const void* dg, unsigned char* success, long long m, int dtype, void* stream) {
-    return pg_is_success_t(task, task >= 0 && task <= 5 ? threshold_f64(task) : 0.0, ag, dg, success, m, dtype, stream);
+    return pg_is_success_t(task, default_threshold(task), ag, dg, success, m, dtype, stream);
 }
 int pg_her_relabel_pitched(int task, int reward_type, double threshold, const void* next_ag, const void* dg, long long pitch, const long long* src, const long long* goal_src,
                            void* dg_out, void* ag_out, float* reward, long long m, int dtype, void* stream) {
     if (m == 0) return PG_OK;
-    if (task < 0 || task > 5 || reward_type < 0 || reward_type > 1 || !next_ag || !dg || !src || !goal_src || !dg_out || !reward || m < 0 || !(threshold >= 0))
+    if (!valid_task(task) || !valid_reward_type(reward_type) || !next_ag || !dg || !src || !goal_src || !dg_out || !reward || m < 0 || !(threshold >= 0))
         return fail(PG_ERR_ARG, "pg_her_relabel: bad argument");
     if (pitch < task_goal_dim(task)) return fail(PG_ERR_ARG, "pg_her_relabel_pitched: the row pitch is smaller than the goal dimension");
-    if (dtype == PG_F32) launch_her<float>(task, (const float*)next_ag, (const float*)dg, src, goal_src, (float*)dg_out, (float*)ag_out, reward, m, pitch, reward_type, threshold, (cudaStream_t)stream);
-    else launch_her<double>(task, (const double*)next_ag, (const double*)dg, src, goal_src, (double*)dg_out, (double*)ag_out, reward, m, pitch, reward_type, threshold, (cudaStream_t)stream);
+    with_dtype(dtype, [&](auto x) {
+        using E = decltype(x);
+        launch_her<E>(task, (const E*)next_ag, (const E*)dg, src, goal_src, (E*)dg_out, (E*)ag_out, reward, m, pitch, reward_type, threshold, (cudaStream_t)stream);
+    });
     PG_CUDA(cudaGetLastError());
     return PG_OK;
 }
 int pg_her_relabel_t(int task, int reward_type, double threshold, const void* next_ag, const void* dg, const long long* src, const long long* goal_src, void* dg_out, void* ag_out,
                      float* reward, long long m, int dtype, void* stream) {
-    return pg_her_relabel_pitched(task, reward_type, threshold, next_ag, dg, task >= 0 && task <= 5 ? task_goal_dim(task) : 0, src, goal_src, dg_out, ag_out, reward, m, dtype, stream);
+    return pg_her_relabel_pitched(task, reward_type, threshold, next_ag, dg, valid_task(task) ? task_goal_dim(task) : 0, src, goal_src, dg_out, ag_out, reward, m, dtype, stream);
 }
 int pg_her_relabel(int task, int reward_type, const void* next_ag, const void* dg, const long long* src, const long long* goal_src, void* dg_out, void* ag_out,
                    float* reward, long long m, int dtype, void* stream) {
-    return pg_her_relabel_t(task, reward_type, task >= 0 && task <= 5 ? threshold_f64(task) : 0.0, next_ag, dg, src, goal_src, dg_out, ag_out, reward, m, dtype, stream);
+    return pg_her_relabel_t(task, reward_type, default_threshold(task), next_ag, dg, src, goal_src, dg_out, ag_out, reward, m, dtype, stream);
 }
 // Host-array entry points (the path stable-baselines3's HerReplayBuffer takes through env_method("compute_reward"), reference
 // panda_gym/envs/core.py:226, examples/train_push.py:1-12).  Staging is cached per device and only ever grows: after the first call
@@ -515,7 +540,7 @@ static int stage_for(int device, size_t in_bytes, size_t out_bytes, HostStage** 
 }
 long long pg_host_stage_allocations(void) { return g_stage_allocs; }
 static int reward_host(bool want_reward, int task, int reward_type, double thr, const void* ag, const void* dg, void* result, long long m, int dtype, int device) {
-    const size_t es = dtype == PG_F32 ? 4 : 8, bytes = (size_t)m * task_goal_dim(task) * es, out_bytes = (size_t)m * (want_reward ? 4 : 1);
+    const size_t es = with_dtype(dtype, [](auto x) { return sizeof(x); }), bytes = (size_t)m * task_goal_dim(task) * es, out_bytes = (size_t)m * (want_reward ? 4 : 1);
     HostStage* h = nullptr;
     int rc = stage_for(device, bytes, out_bytes, &h); if (rc != PG_OK) return rc;
     PG_CUDA(cudaMemcpyAsync(h->da, ag, bytes, cudaMemcpyHostToDevice, h->st));
@@ -530,19 +555,19 @@ static int reward_host(bool want_reward, int task, int reward_type, double thr, 
 }
 int pg_compute_reward_host_t(int task, int reward_type, double threshold, const void* ag, const void* dg, float* reward, long long m, int dtype, int device) {
     if (m == 0) return PG_OK;
-    if (task < 0 || task > 5 || reward_type < 0 || reward_type > 1 || !ag || !dg || !reward || m < 0 || !(threshold >= 0)) return fail(PG_ERR_ARG, "pg_compute_reward_host: bad argument");
+    if (!valid_task(task) || !valid_reward_type(reward_type) || !ag || !dg || !reward || m < 0 || !(threshold >= 0)) return fail(PG_ERR_ARG, "pg_compute_reward_host: bad argument");
     return reward_host(true, task, reward_type, threshold, ag, dg, reward, m, dtype, device);
 }
 int pg_is_success_host_t(int task, double threshold, const void* ag, const void* dg, unsigned char* success, long long m, int dtype, int device) {
     if (m == 0) return PG_OK;
-    if (task < 0 || task > 5 || !ag || !dg || !success || m < 0 || !(threshold >= 0)) return fail(PG_ERR_ARG, "pg_is_success_host: bad argument");
+    if (!valid_task(task) || !ag || !dg || !success || m < 0 || !(threshold >= 0)) return fail(PG_ERR_ARG, "pg_is_success_host: bad argument");
     return reward_host(false, task, 0, threshold, ag, dg, success, m, dtype, device);
 }
 int pg_compute_reward_host(int task, int reward_type, const void* ag, const void* dg, float* reward, long long m, int dtype, int device) {
-    return pg_compute_reward_host_t(task, reward_type, task >= 0 && task <= 5 ? threshold_f64(task) : 0.0, ag, dg, reward, m, dtype, device);
+    return pg_compute_reward_host_t(task, reward_type, default_threshold(task), ag, dg, reward, m, dtype, device);
 }
 int pg_is_success_host(int task, const void* ag, const void* dg, unsigned char* success, long long m, int dtype, int device) {
-    return pg_is_success_host_t(task, task >= 0 && task <= 5 ? threshold_f64(task) : 0.0, ag, dg, success, m, dtype, device);
+    return pg_is_success_host_t(task, default_threshold(task), ag, dg, success, m, dtype, device);
 }
 
 // Snapshots are stream-ordered: one device-to-device copy of the handle's single SoA allocation, enqueued on the caller's stream
@@ -591,32 +616,14 @@ int pg_remove_state(pg_env* e, int state_id) {
 
 int pg_get_state(pg_env* e, double* state, void* stream) {
     if (!e || !state) return fail(PG_ERR_ARG, "pg_get_state: NULL argument");
-    PG_CUDA(cudaSetDevice(e->device));
-    const int grid = (e->n + BLOCK - 1) / BLOCK;
-    if (e->precision == PG_F32) get_state_kernel<float><<<grid, BLOCK, 0, (cudaStream_t)stream>>>(e->Ef, e->nobj, e->goal_dim, state);
-    else get_state_kernel<double><<<grid, BLOCK, 0, (cudaStream_t)stream>>>(e->Ed, e->nobj, e->goal_dim, state);
-    g_launches++;
-    PG_CUDA(cudaGetLastError());
-    return PG_OK;
+    return launch_per_env(e, stream, [&](auto& E, int grid, cudaStream_t st) { get_state_kernel<<<grid, BLOCK, 0, st>>>(E, e->nobj, e->goal_dim, state); });
 }
 int pg_set_state(pg_env* e, const double* state, const unsigned char* mask, void* stream) {
     if (!e || !state) return fail(PG_ERR_ARG, "pg_set_state: NULL argument");
-    PG_CUDA(cudaSetDevice(e->device));
-    const int grid = (e->n + BLOCK - 1) / BLOCK;
-    if (e->precision == PG_F32) set_state_kernel<float><<<grid, BLOCK, 0, (cudaStream_t)stream>>>(e->Ef, e->nobj, e->goal_dim, state, mask);
-    else set_state_kernel<double><<<grid, BLOCK, 0, (cudaStream_t)stream>>>(e->Ed, e->nobj, e->goal_dim, state, mask);
-    g_launches++;
-    PG_CUDA(cudaGetLastError());
-    return PG_OK;
+    return launch_per_env(e, stream, [&](auto& E, int grid, cudaStream_t st) { set_state_kernel<<<grid, BLOCK, 0, st>>>(E, e->nobj, e->goal_dim, state, mask); });
 }
 static int launch_ik(pg_env* e, int link, const double* position, const double* orientation, double* joint_angles, int out7, void* stream) {
-    PG_CUDA(cudaSetDevice(e->device));
-    const int grid = (e->n + BLOCK - 1) / BLOCK;
-    if (e->precision == PG_F32) ik_kernel<float><<<grid, BLOCK, 0, (cudaStream_t)stream>>>(e->Ef, link, position, orientation, joint_angles, out7);
-    else ik_kernel<double><<<grid, BLOCK, 0, (cudaStream_t)stream>>>(e->Ed, link, position, orientation, joint_angles, out7);
-    g_launches++;
-    PG_CUDA(cudaGetLastError());
-    return PG_OK;
+    return launch_per_env(e, stream, [&](auto& E, int grid, cudaStream_t st) { ik_kernel<<<grid, BLOCK, 0, st>>>(E, link, position, orientation, joint_angles, out7); });
 }
 int pg_inverse_kinematics(pg_env* e, const double* position, const double* orientation, double* joint_angles, void* stream) {
     if (!e || !position || !orientation || !joint_angles) return fail(PG_ERR_ARG, "pg_inverse_kinematics: NULL argument");
@@ -630,54 +637,35 @@ int pg_inverse_kinematics_link(pg_env* e, int link, const double* position, cons
 int pg_get_link_state(pg_env* e, int link, double* out, void* stream) {
     if (!e || !out) return fail(PG_ERR_ARG, "pg_get_link_state: NULL argument");
     if (link < 0 || link > 11) return fail(PG_ERR_ARG, "pg_get_link_state: link must be 0..11");
-    PG_CUDA(cudaSetDevice(e->device));
-    const int grid = (e->n + BLOCK - 1) / BLOCK;
-    if (e->precision == PG_F32) link_state_kernel<float><<<grid, BLOCK, 0, (cudaStream_t)stream>>>(e->Ef, link, out);
-    else link_state_kernel<double><<<grid, BLOCK, 0, (cudaStream_t)stream>>>(e->Ed, link, out);
-    g_launches++;
-    PG_CUDA(cudaGetLastError());
-    return PG_OK;
+    return launch_per_env(e, stream, [&](auto& E, int grid, cudaStream_t st) { link_state_kernel<<<grid, BLOCK, 0, st>>>(E, link, out); });
 }
 int pg_set_motors(pg_env* e, const double* motors, const unsigned char* mask, void* stream) {
     if (!e || !motors) return fail(PG_ERR_ARG, "pg_set_motors: NULL argument");
     if (e->task != PG_TASK_BARE) return fail(PG_ERR_ARG, "pg_set_motors: task handles derive their motor targets from the action inside pg_step (Panda.set_action); raw motors exist on bare worlds");
-    PG_CUDA(cudaSetDevice(e->device));
-    const int grid = (e->n + BLOCK - 1) / BLOCK;
-    if (e->precision == PG_F32) set_motors_kernel<float><<<grid, BLOCK, 0, (cudaStream_t)stream>>>(e->Ef, motors, mask);
-    else set_motors_kernel<double><<<grid, BLOCK, 0, (cudaStream_t)stream>>>(e->Ed, motors, mask);
-    g_launches++;
-    PG_CUDA(cudaGetLastError());
-    return PG_OK;
+    return launch_per_env(e, stream, [&](auto& E, int grid, cudaStream_t st) { set_motors_kernel<<<grid, BLOCK, 0, st>>>(E, motors, mask); });
 }
 int pg_get_motors(pg_env* e, double* motors, void* stream) {
     if (!e || !motors) return fail(PG_ERR_ARG, "pg_get_motors: NULL argument");
     if (e->task != PG_TASK_BARE) return fail(PG_ERR_ARG, "pg_get_motors: bare worlds only");
-    PG_CUDA(cudaSetDevice(e->device));
-    const int grid = (e->n + BLOCK - 1) / BLOCK;
-    if (e->precision == PG_F32) get_motors_kernel<float><<<grid, BLOCK, 0, (cudaStream_t)stream>>>(e->Ef, motors);
-    else get_motors_kernel<double><<<grid, BLOCK, 0, (cudaStream_t)stream>>>(e->Ed, motors);
-    g_launches++;
-    PG_CUDA(cudaGetLastError());
-    return PG_OK;
+    return launch_per_env(e, stream, [&](auto& E, int grid, cudaStream_t st) { get_motors_kernel<<<grid, BLOCK, 0, st>>>(E, motors); });
 }
 int pg_sim_step(pg_env* e, int n_substeps, void* stream) {
     if (!e || n_substeps < 0) return fail(PG_ERR_ARG, "pg_sim_step: bad argument");
     if (e->task != PG_TASK_BARE) return fail(PG_ERR_ARG, "pg_sim_step: task handles step through pg_step (controller + sub-steps + observation in one call)");
     if (n_substeps == 0) return PG_OK;
     PG_CUDA(cudaSetDevice(e->device));
-    if (e->precision == PG_F32) launch_bare_step<float>(e->Ef, e->nobj, n_substeps, (cudaStream_t)stream);
-    else launch_bare_step<double>(e->Ed, e->nobj, n_substeps, (cudaStream_t)stream);
+    with_env(e, [&](auto& E) { launch_bare_step(E, e->nobj, n_substeps, (cudaStream_t)stream); });
     PG_CUDA(cudaGetLastError());
     return PG_OK;
 }
 static void fill_render_scene(pg_env* e) {
     RenderScene& R = e->rscene;
     memset(&R, 0, sizeof R);
-    const Scene<double>& S = e->precision == PG_F32 ? scene_cast<double>(e->Ef.S) : e->Ed.S;
+    Scene<double> S; double bz;
+    with_env(e, [&](auto& E) { S = scene_cast<double>(E.S); bz = E.M.base[2]; });
     R.nobj = e->nobj;
     R.has_table = S.table_x0 < S.table_x1; R.table[0] = (float)S.table_x0; R.table[1] = (float)S.table_x1; R.table[2] = (float)S.table_y0; R.table[3] = (float)S.table_y1; R.table_height = 0.4f;
     R.has_plane = S.ground_z > -1e29; R.plane_z = (float)S.ground_z;
-    const double bz = e->precision == PG_F32 ? (double)e->Ef.M.base[2] : e->Ed.M.base[2];
     R.has_robot = bz < 500.0;                                  // a bare world without a robot parks it 1 km up
     const float bc[3] = {-0.04f, 0.0f, 0.07f}, bh[3] = {0.11f, 0.1f, 0.07f};     // panda_link0: approximate extents (its mesh is not available)
     for (int k = 0; k < 3; k++) { R.base_c[k] = bc[k]; R.base_h[k] = bh[k]; }
@@ -717,26 +705,22 @@ int pg_render(pg_env* e, int width, int height, const double* camera, int crop, 
                                                       {26, 230, 26, 255}, {235, 235, 235, 255}};     // plane 0.15, table 0.95, objects (tasks/ *.py rgba_color), robot
     memcpy(C.color, col, sizeof col);
     C.background[0] = 223; C.background[1] = 54; C.background[2] = 45; C.background[3] = 255;          // pybullet.py:28 default background_color
-    if (e->precision == PG_F32) launch_render_setup<float>(e->Ef, e->rscene, e->prims, (cudaStream_t)stream); else launch_render_setup<double>(e->Ed, e->rscene, e->prims, (cudaStream_t)stream);
+    with_env(e, [&](auto& E) { launch_render_setup(E, e->rscene, e->prims, (cudaStream_t)stream); });
     launch_render(e->prims, C, e->n, depth, rgba, segmentation, points, valid, (cudaStream_t)stream);
     PG_CUDA(cudaGetLastError());
     return PG_OK;
 }
 int pg_get_ee_pose(pg_env* e, double* pose, void* stream) {
     if (!e || !pose) return fail(PG_ERR_ARG, "pg_get_ee_pose: NULL argument");
-    PG_CUDA(cudaSetDevice(e->device));
-    const int grid = (e->n + BLOCK - 1) / BLOCK;
-    if (e->precision == PG_F32) ee_pose_kernel<float><<<grid, BLOCK, 0, (cudaStream_t)stream>>>(e->Ef, pose);
-    else ee_pose_kernel<double><<<grid, BLOCK, 0, (cudaStream_t)stream>>>(e->Ed, pose);
-    g_launches++;
-    PG_CUDA(cudaGetLastError());
-    return PG_OK;
+    return launch_per_env(e, stream, [&](auto& E, int grid, cudaStream_t st) { ee_pose_kernel<<<grid, BLOCK, 0, st>>>(E, pose); });
 }
 int pg_debug_schedule(pg_env* e, unsigned short* key_host, int* perm_host) {
     if (!e || !key_host || !perm_host) return fail(PG_ERR_ARG, "pg_debug_schedule: NULL argument");
     PG_CUDA(cudaSetDevice(e->device));
-    PG_CUDA(cudaMemcpy(key_host, e->precision == PG_F32 ? e->Ef.ccount : e->Ed.ccount, (size_t)e->n * sizeof(unsigned short), cudaMemcpyDeviceToHost));
-    PG_CUDA(cudaMemcpy(perm_host, e->precision == PG_F32 ? e->Ef.perm : e->Ed.perm, (size_t)e->n * sizeof(int), cudaMemcpyDeviceToHost));
+    const unsigned short* key = nullptr; const int* perm = nullptr;
+    with_env(e, [&](auto& E) { key = E.ccount; perm = E.perm; });
+    PG_CUDA(cudaMemcpy(key_host, key, (size_t)e->n * sizeof(unsigned short), cudaMemcpyDeviceToHost));
+    PG_CUDA(cudaMemcpy(perm_host, perm, (size_t)e->n * sizeof(int), cudaMemcpyDeviceToHost));
     return PG_OK;
 }
 int pg_debug_timing(pg_env* e, long long* out) {
@@ -749,25 +733,21 @@ int pg_debug_timing(pg_env* e, long long* out) {
 }
 int pg_contact_overflows(pg_env* e, long long* count) {
     if (!e || !count) return fail(PG_ERR_ARG, "pg_contact_overflows: NULL argument");
-    PG_CUDA(cudaSetDevice(e->device));
     double d = 0;
-    PG_CUDA(cudaMemcpy(&d, (e->precision == PG_F32 ? e->Ef.stats : e->Ed.stats) + 5, sizeof(double), cudaMemcpyDeviceToHost));
-    *count = (long long)d;
-    return PG_OK;
+    const int rc = read_stats(e, 5, 1, &d);
+    if (rc == PG_OK) *count = (long long)d;
+    return rc;
 }
 int pg_diverged(pg_env* e, long long* count) {
     if (!e || !count) return fail(PG_ERR_ARG, "pg_diverged: NULL argument");
-    PG_CUDA(cudaSetDevice(e->device));
     double d = 0;
-    PG_CUDA(cudaMemcpy(&d, (e->precision == PG_F32 ? e->Ef.stats : e->Ed.stats) + 4, sizeof(double), cudaMemcpyDeviceToHost));
-    *count = (long long)d;
-    return PG_OK;
+    const int rc = read_stats(e, 4, 1, &d);
+    if (rc == PG_OK) *count = (long long)d;
+    return rc;
 }
 int pg_stats(pg_env* e, double out[4]) {
     if (!e || !out) return fail(PG_ERR_ARG, "pg_stats: NULL argument");
-    PG_CUDA(cudaSetDevice(e->device));
-    PG_CUDA(cudaMemcpy(out, e->precision == PG_F32 ? e->Ef.stats : e->Ed.stats, 4 * sizeof(double), cudaMemcpyDeviceToHost));
-    return PG_OK;
+    return read_stats(e, 0, 4, out);
 }
 
 }  // extern "C"

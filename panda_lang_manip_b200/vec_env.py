@@ -19,7 +19,81 @@ def _ptr(t: Optional[torch.Tensor]):
     return None if t is None else t.data_ptr()
 
 
-class PandaVecEnv:
+class _Handle:
+    """What task envs and bare worlds do alike with their pg_env handle: raw state, link state, snapshots, rendering and closing.
+    Subclasses set ``lib`` (the loaded library), ``_h`` (the handle), ``num_envs``, ``device`` and ``state_dim``."""
+
+    def close(self) -> None:
+        if getattr(self, "_h", None) is not None:
+            self.lib.pg_destroy(self._h)
+            self._h = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    def _stream(self):
+        return torch.cuda.current_stream(self.device).cuda_stream
+
+    # -- snapshots / raw state ---------------------------------------------------------------------------------------
+    def save_state(self) -> int:
+        """Stream-ordered snapshot (one device-to-device copy on the current stream, no synchronisation)."""
+        import ctypes
+        sid = ctypes.c_int()
+        _lib.check(self.lib.pg_save_state_async(self._h, ctypes.byref(sid), self._stream()))
+        return sid.value
+
+    def restore_state(self, state_id: int) -> None:
+        _lib.check(self.lib.pg_restore_state_async(self._h, int(state_id), self._stream()))
+
+    def remove_state(self, state_id: int) -> None:
+        _lib.check(self.lib.pg_remove_state(self._h, int(state_id)))
+
+    def get_state(self) -> torch.Tensor:
+        """[N, state_dim] float64: q(9) qd(9) | per object pos3 quat4 lin3 ang3 | goal (task envs only) | episode step."""
+        s = torch.empty((self.num_envs, self.state_dim), dtype=torch.float64, device=self.device)
+        _lib.check(self.lib.pg_get_state(self._h, _ptr(s), self._stream()))
+        return s
+
+    def set_state(self, state: torch.Tensor, mask: Optional[torch.Tensor] = None) -> None:
+        s = state.to(device=self.device, dtype=torch.float64).contiguous()
+        m = None if mask is None else mask.to(device=self.device, dtype=torch.uint8).contiguous()
+        _lib.check(self.lib.pg_set_state(self._h, _ptr(s), _ptr(m), self._stream()))
+        torch.cuda.current_stream(self.device).synchronize()
+
+    def link_state(self, link: int) -> torch.Tensor:
+        """[N,13] float64 = getLinkState(link, computeLinkVelocity=1): CoM-frame position, quaternion (x,y,z,w), linear and angular
+        velocity of link 0..11, with pybullet's one-sub-step-stale link-transform cache (SURVEY App. B.5)."""
+        out = torch.empty((self.num_envs, 13), dtype=torch.float64, device=self.device)
+        _lib.check(self.lib.pg_get_link_state(self._h, int(link), _ptr(out), self._stream()))
+        return out
+
+    def render(self, width: int = 480, height: int = 480, target_position=(0.0, 0.0, 0.0), distance: float = 1.4, yaw: float = 45, pitch: float = -30, roll: float = 0,
+               crop: bool = True, rgb: bool = True, points: bool = True, segmentation: bool = False) -> Dict[str, torch.Tensor]:
+        """PyBullet.render (the fork's camera path, pybullet.py:149-264) for every env: analytic ray casting of the primitive scene.
+        Returns a dict of device tensors: ``depth`` [N,H,W] (OpenGL depth-buffer values), ``rgb`` [N,H,W,3] uint8, ``points`` [N,H,W,3]
+        (the reference's deprojection; NaN where filtered) with ``valid`` [N,H,W] bool (depth < 0.99 and, with ``crop``, the
+        reference's workspace box), ``segmentation`` [N,H,W] uint8."""
+        n, dev = self.num_envs, self.device
+        cam = np.ascontiguousarray([*[float(x) for x in target_position], float(distance), float(yaw), float(pitch), float(roll)], dtype=np.float64)
+        out = {"depth": torch.empty((n, height, width), dtype=torch.float32, device=dev)}
+        rgba = torch.empty((n, height, width, 4), dtype=torch.uint8, device=dev) if rgb else None
+        pts = torch.empty((n, height, width, 3), dtype=torch.float32, device=dev) if points else None
+        val = torch.empty((n, height, width), dtype=torch.uint8, device=dev) if points else None
+        seg = torch.empty((n, height, width), dtype=torch.uint8, device=dev) if segmentation else None
+        _lib.check(self.lib.pg_render(self._h, int(width), int(height), cam.ctypes.data, int(bool(crop)), _ptr(out["depth"]), _ptr(rgba), _ptr(seg), _ptr(pts), _ptr(val), self._stream()))
+        if rgb:
+            out["rgb"] = rgba[..., :3]
+        if points:
+            out["points"], out["valid"] = pts, val.bool()
+        if segmentation:
+            out["segmentation"] = seg
+        return out
+
+
+class PandaVecEnv(_Handle):
     """num_envs lock-stepped panda_gym environments resident in HBM.
 
     Args mirror the reference constructors (panda_gym/envs/panda_tasks.py): ``reward_type`` "sparse"|"dense",
@@ -88,18 +162,7 @@ class PandaVecEnv:
         for ptr in list(getattr(self, "_pinned", {})):
             self.lib.pg_host_unpin(ptr)
             self._pinned.pop(ptr, None)
-        if getattr(self, "_h", None) is not None:
-            self.lib.pg_destroy(self._h)
-            self._h = None
-
-    def __del__(self):
-        try:
-            self.close()
-        except Exception:
-            pass
-
-    def _stream(self):
-        return torch.cuda.current_stream(self.device).cuda_stream
+        super().close()
 
     def _obs_dict(self) -> Dict[str, torch.Tensor]:
         return {"observation": self.obs, "achieved_goal": self.achieved_goal, "desired_goal": self.desired_goal}
@@ -187,19 +250,6 @@ class PandaVecEnv:
         return is_success(self.task, achieved_goal, desired_goal, threshold=self.distance_threshold)
 
     # -- snapshots / raw state ---------------------------------------------------------------------------------------
-    def save_state(self) -> int:
-        """Stream-ordered snapshot (one device-to-device copy on the current stream, no synchronisation)."""
-        import ctypes
-        sid = ctypes.c_int()
-        _lib.check(self.lib.pg_save_state_async(self._h, ctypes.byref(sid), self._stream()))
-        return sid.value
-
-    def restore_state(self, state_id: int) -> None:
-        _lib.check(self.lib.pg_restore_state_async(self._h, int(state_id), self._stream()))
-
-    def remove_state(self, state_id: int) -> None:
-        _lib.check(self.lib.pg_remove_state(self._h, int(state_id)))
-
     def lookahead(self, candidate_actions: torch.Tensor, commit: bool = True):
         """Batched greedy look-ahead search (reference docs/usage/save_restore_state.rst:8-41: save_state, try K sampled actions
         from the same state, keep the one with the best reward): ``candidate_actions`` is [K, N, A]; every env evaluates its K
@@ -229,18 +279,6 @@ class PandaVecEnv:
         out = self.step(best_a) if commit else None
         return best_a, best_r, out
 
-    def get_state(self) -> torch.Tensor:
-        """[N, state_dim] float64: q(9) qd(9) | per object pos3 quat4 lin3 ang3 | goal | episode step."""
-        s = torch.empty((self.num_envs, self.state_dim), dtype=torch.float64, device=self.device)
-        _lib.check(self.lib.pg_get_state(self._h, _ptr(s), self._stream()))
-        return s
-
-    def set_state(self, state: torch.Tensor, mask: Optional[torch.Tensor] = None) -> None:
-        s = state.to(device=self.device, dtype=torch.float64).contiguous()
-        m = None if mask is None else mask.to(device=self.device, dtype=torch.uint8).contiguous()
-        _lib.check(self.lib.pg_set_state(self._h, _ptr(s), _ptr(m), self._stream()))
-        torch.cuda.current_stream(self.device).synchronize()
-
     def inverse_kinematics(self, position, orientation, link: Optional[int] = None) -> torch.Tensor:
         """calculateInverseKinematics from the current joint state.  ``link=None``: the env path's link-11 solve, [N,7] arm angles;
         ``link=k``: PyBullet.inverse_kinematics(body, k, ...) for any link 0..11, all nine joint values [N,9]."""
@@ -254,39 +292,10 @@ class PandaVecEnv:
             _lib.check(self.lib.pg_inverse_kinematics_link(self._h, int(link), _ptr(p), _ptr(o), _ptr(out), self._stream()))
         return out
 
-    def link_state(self, link: int) -> torch.Tensor:
-        """[N,13] float64 = getLinkState(link, computeLinkVelocity=1): CoM-frame position, quaternion (x,y,z,w), linear and angular
-        velocity of link 0..11, with pybullet's one-sub-step-stale link-transform cache (SURVEY App. B.5)."""
-        out = torch.empty((self.num_envs, 13), dtype=torch.float64, device=self.device)
-        _lib.check(self.lib.pg_get_link_state(self._h, int(link), _ptr(out), self._stream()))
-        return out
-
     def ee_pose(self) -> torch.Tensor:
         """[N,7] float64: end-effector position and quaternion (x,y,z,w) from the current joint state."""
         out = torch.empty((self.num_envs, 7), dtype=torch.float64, device=self.device)
         _lib.check(self.lib.pg_get_ee_pose(self._h, _ptr(out), self._stream()))
-        return out
-
-    def render(self, width: int = 480, height: int = 480, target_position=(0.0, 0.0, 0.0), distance: float = 1.4, yaw: float = 45, pitch: float = -30, roll: float = 0,
-               crop: bool = True, rgb: bool = True, points: bool = True, segmentation: bool = False) -> Dict[str, torch.Tensor]:
-        """PyBullet.render (the fork's camera path, pybullet.py:149-264) for every env: analytic ray casting of the primitive scene.
-        Returns a dict of device tensors: ``depth`` [N,H,W] (OpenGL depth-buffer values), ``rgb`` [N,H,W,3] uint8, ``points`` [N,H,W,3]
-        (the reference's deprojection; NaN where filtered) with ``valid`` [N,H,W] bool (depth < 0.99 and, with ``crop``, the
-        reference's workspace box), ``segmentation`` [N,H,W] uint8."""
-        n, dev = self.num_envs, self.device
-        cam = np.ascontiguousarray([*[float(x) for x in target_position], float(distance), float(yaw), float(pitch), float(roll)], dtype=np.float64)
-        out = {"depth": torch.empty((n, height, width), dtype=torch.float32, device=dev)}
-        rgba = torch.empty((n, height, width, 4), dtype=torch.uint8, device=dev) if rgb else None
-        pts = torch.empty((n, height, width, 3), dtype=torch.float32, device=dev) if points else None
-        val = torch.empty((n, height, width), dtype=torch.uint8, device=dev) if points else None
-        seg = torch.empty((n, height, width), dtype=torch.uint8, device=dev) if segmentation else None
-        _lib.check(self.lib.pg_render(self._h, int(width), int(height), cam.ctypes.data, int(bool(crop)), _ptr(out["depth"]), _ptr(rgba), _ptr(seg), _ptr(pts), _ptr(val), self._stream()))
-        if rgb:
-            out["rgb"] = rgba[..., :3]
-        if points:
-            out["points"], out["valid"] = pts, val.bool()
-        if segmentation:
-            out["segmentation"] = seg
         return out
 
     def diverged(self) -> int:

@@ -207,23 +207,24 @@ def test_seed_determinism_and_snapshot():
 def test_auto_reset_truncation_and_stats():
     import panda_lang_manip_b200 as p
     n = 512
-    env = p.PandaVecEnv("reach", n, control_type="joints", seed=3)
-    zero = torch.zeros((n, 7), device="cuda")
-    term_seen = torch.zeros(n, dtype=torch.uint8, device="cuda")
-    for t in range(50):
+    for precision in ("f32", "f64"):
+        env = p.PandaVecEnv("reach", n, control_type="joints", seed=3, precision=precision)
+        zero = torch.zeros((n, 7), device="cuda")
+        term_seen = torch.zeros(n, dtype=torch.uint8, device="cuda")
+        for t in range(50):
+            _, _, term, trunc, _ = env.step(zero)
+            term_seen |= term
+            if t < 49:
+                assert int(trunc.sum()) == 0
+        assert bool(((trunc == 1) | (term_seen == 1)).all())      # at step 50 every env has either succeeded earlier (and restarted) or is truncated now
+        st = env.stats()
+        assert st[0] >= int(trunc.sum()) and st[3] > 0
+        assert env.diverged() == 0
+        bad = env.get_state(); bad[:7, 0] = float("nan")          # poison 7 envs: they are counted, truncated and restarted
+        env.set_state(bad)
         _, _, term, trunc, _ = env.step(zero)
-        term_seen |= term
-        if t < 49:
-            assert int(trunc.sum()) == 0
-    assert bool(((trunc == 1) | (term_seen == 1)).all())      # at step 50 every env has either succeeded earlier (and restarted) or is truncated now
-    st = env.stats()
-    assert st[0] >= int(trunc.sum()) and st[3] > 0
-    assert env.diverged() == 0
-    bad = env.get_state(); bad[:7, 0] = float("nan")          # poison 7 envs: they are counted, truncated and restarted
-    env.set_state(bad)
-    _, _, term, trunc, _ = env.step(zero)
-    assert env.diverged() == 7 and int(trunc[:7].sum()) == 7 and bool(torch.isfinite(env.get_state()).all())
-    env.close()
+        assert env.diverged() == 7 and int(trunc[:7].sum()) == 7 and bool(torch.isfinite(env.get_state()).all())
+        env.close()
 
 
 def test_large_batch_properties():
@@ -338,25 +339,26 @@ def test_host_path_pinned_and_pageable_buffers_agree():
     """pg_step_host copies directly from / to page-locked buffers (pg_host_pin) and through its staging slabs otherwise: same results."""
     import panda_lang_manip_b200 as p
     n = 300
-    a_env = p.PandaVecEnv("push", n, seed=4, auto_reset=False)
-    b_env = p.PandaVecEnv("push", n, seed=4, auto_reset=False)
-    rng = np.random.default_rng(0)
-    pinned = a_env.pin_host(np.zeros((n, 3), np.float32))
-    for t in range(3):
-        act = rng.uniform(-1, 1, (n, 3)).astype(np.float32)
-        pinned[:] = act
-        oa, ra, ta, ua, _ = a_env.step_host(pinned)
-        ob, rb, tb, ub, _ = b_env.step(torch.from_numpy(act).cuda())
-        assert np.array_equal(oa["observation"], ob["observation"].cpu().numpy()) and np.array_equal(oa["desired_goal"], ob["desired_goal"].cpu().numpy())
-        assert np.array_equal(ra, rb.cpu().numpy()) and np.array_equal(ta, tb.cpu().numpy())
-    # the raw entry point with pageable outputs (staging slabs) on a third twin
-    c_env = p.PandaVecEnv("push", n, seed=4, auto_reset=False)
-    rng = np.random.default_rng(0)
-    o2, g2, d2, r2, t2, u2 = np.empty((n, 18), np.float32), np.empty((n, 3), np.float32), np.empty((n, 3), np.float32), np.empty(n, np.float32), np.empty(n, np.uint8), np.empty(n, np.uint8)
-    for t in range(3):
-        act = rng.uniform(-1, 1, (n, 3)).astype(np.float32)
-        rc = c_env.lib.pg_step_host(c_env._h, act.ctypes.data, o2.ctypes.data, g2.ctypes.data, d2.ctypes.data, r2.ctypes.data, t2.ctypes.data, u2.ctypes.data, 0)
-        assert rc == 0
-    assert np.array_equal(o2, oa["observation"]) and np.array_equal(r2, ra) and np.array_equal(t2, ta)
-    a_env.unpin_host(pinned)
-    a_env.close(); b_env.close(); c_env.close()
+    for precision in ("f32", "f64"):
+        a_env = p.PandaVecEnv("push", n, seed=4, auto_reset=False, precision=precision)
+        b_env = p.PandaVecEnv("push", n, seed=4, auto_reset=False, precision=precision)
+        rng = np.random.default_rng(0)
+        pinned = a_env.pin_host(np.zeros((n, 3), np.float32))
+        for t in range(3):
+            act = rng.uniform(-1, 1, (n, 3)).astype(np.float32)
+            pinned[:] = act
+            oa, ra, ta, ua, _ = a_env.step_host(pinned)
+            ob, rb, tb, ub, _ = b_env.step(torch.from_numpy(act).cuda())
+            assert np.array_equal(oa["observation"], ob["observation"].cpu().numpy()) and np.array_equal(oa["desired_goal"], ob["desired_goal"].cpu().numpy())
+            assert np.array_equal(ra, rb.cpu().numpy()) and np.array_equal(ta, tb.cpu().numpy())
+        # the raw entry point with pageable outputs (staging slabs) on a third twin
+        c_env = p.PandaVecEnv("push", n, seed=4, auto_reset=False, precision=precision)
+        rng = np.random.default_rng(0)
+        o2, g2, d2, r2, t2, u2 = np.empty((n, 18), np.float32), np.empty((n, 3), np.float32), np.empty((n, 3), np.float32), np.empty(n, np.float32), np.empty(n, np.uint8), np.empty(n, np.uint8)
+        for t in range(3):
+            act = rng.uniform(-1, 1, (n, 3)).astype(np.float32)
+            rc = c_env.lib.pg_step_host(c_env._h, act.ctypes.data, o2.ctypes.data, g2.ctypes.data, d2.ctypes.data, r2.ctypes.data, t2.ctypes.data, u2.ctypes.data, 0)
+            assert rc == 0
+        assert np.array_equal(o2, oa["observation"]) and np.array_equal(r2, ra) and np.array_equal(t2, ta)
+        a_env.unpin_host(pinned)
+        a_env.close(); b_env.close(); c_env.close()

@@ -20,7 +20,7 @@ def _quat_R(q):
 
 def _scene_prims(env, i, task):
     """The primitive list the kernel builds, rebuilt independently from the state (free bodies) and from getLinkState-style link poses
-    with computeForwardKinematics (pg_get_ee_pose-equivalent: the oracle's FK on the fresh joint state)."""
+    with computeForwardKinematics (pg_get_ee_pose-equivalent: the oracle's FK on the fresh joint state), and that FK's EE (link 11) pose."""
     from tests.oracle_util import OracleSim
     st = env.get_state()[i].cpu().numpy()
     slide = task == "slide"
@@ -42,23 +42,31 @@ def _scene_prims(env, i, task):
         com = np.array(LINK_BOX[l][0]) if l < 7 else np.array({8: [0, 0, 0.04], 9: [0, 0.01, 0.02], 10: [0, -0.01, 0.02]}[l])
         origin = p - R @ com                                         # link frame origin
         prims.append(("box", 6 + l, origin + R @ np.array(c), R, box))
+    ee_p, ee_q, _, _ = s.link_state(11)
     s.close()
-    return prims
+    return prims, np.concatenate([ee_p, ee_q])
 
 
-@pytest.mark.parametrize("task", ["reach", "push", "slide", "stack"])
-def test_render_matches_the_oracle(task):
+RENDER_TASKS = ["reach", "push", "slide", "stack"]
+
+
+@pytest.mark.parametrize("task,precision", [pytest.param(t, "f32", id=t) for t in RENDER_TASKS] + [pytest.param(t, "f64", id=f"{t}-f64") for t in RENDER_TASKS])
+def test_render_matches_the_oracle(task, precision):
     import panda_lang_manip_b200 as p
     n, W, H = 3, 160, 120
-    env = p.PandaVecEnv(task, n, control_type="joints", seed=4, auto_reset=False)
+    env = p.PandaVecEnv(task, n, control_type="joints", seed=4, auto_reset=False, precision=precision)
     g = torch.Generator(device="cuda").manual_seed(0)
     for _ in range(6):
         env.step(torch.rand((n, env.action_dim), device="cuda", generator=g) * 2 - 1)
     cam = dict(target_position=(-0.1, 0.0, 0.05), distance=1.1, yaw=35.0, pitch=-32.0, roll=0.0)
     out = env.render(W, H, crop=True, segmentation=True, **cam)
     assert out["depth"].shape == (n, H, W) and out["rgb"].shape == (n, H, W, 3) and out["points"].shape == (n, H, W, 3)
+    ee = env.ee_pose().cpu().numpy()
     for i in range(n):
-        d, seg, pts, valid = ro.render(_scene_prims(env, i, task), W, H, target=cam["target_position"], distance=cam["distance"], yaw=cam["yaw"], pitch=cam["pitch"], roll=cam["roll"], crop=True)
+        prims, ee_ref = _scene_prims(env, i, task)
+        assert np.abs(ee[i, :3] - ee_ref[:3]).max() < 1e-5, (ee[i], ee_ref)
+        assert min(np.abs(ee[i, 3:] - ee_ref[3:]).max(), np.abs(ee[i, 3:] + ee_ref[3:]).max()) < 1e-5, (ee[i], ee_ref)    # q and -q: one rotation
+        d, seg, pts, valid = ro.render(prims, W, H, target=cam["target_position"], distance=cam["distance"], yaw=cam["yaw"], pitch=cam["pitch"], roll=cam["roll"], crop=True)
         gd, gs, gp, gv = out["depth"][i].cpu().numpy(), out["segmentation"][i].cpu().numpy(), out["points"][i].cpu().numpy(), out["valid"][i].cpu().numpy()
         same = gs == seg
         assert same.mean() > 0.995, (task, i, same.mean())            # silhouette pixels may fall on either side in float32
