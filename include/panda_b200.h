@@ -183,6 +183,28 @@ int pg_get_link_state(pg_env* env, int link, double* out, void* stream);
  * get_ee_orientation, panda_gym/envs/robots/panda_cartesian.py:218-225). */
 int pg_get_ee_pose(pg_env* env, double* pose, void* stream);
 
+/* The fork's scripted motion primitives (panda_gym/envs/robots/panda_cartesian.py:47-68: move, grasp, release) for every env of an
+ * ee-controlled task handle.  A pg_motion plan is bound to a batch size and a device and serves any handle of that size on that
+ * device.  Each env runs its own primitive with its own step count; a primitive begun on an env replaces the one it was running.
+ *   move: way-points 1.5 cm apart (20 for a distance under 3 cm) from the EE position when the move begins to goal_pos [N,3], and a
+ *     Slerp from the EE orientation then to goal_quat [N,4] (x,y,z,w; float64, normalised inside).  Each step's action is the next
+ *     way-point minus the current EE position, finger action 0.
+ *   gripper: `steps` steps of zero displacement with the finger action finger_action (grasp: -1, 30 steps; release: width, 30 steps),
+ *     holding the current EE orientation.  Not for the blocked-gripper tasks Reach, Push and Slide (PG_ERR_STATE).
+ * mask [N] (DEVICE, NULL = all) selects the envs a primitive begins on.  pg_motion_step writes each env's action and target
+ * orientation (an env with no primitive left gets zero displacement, finger action 0 and its current orientation), then runs
+ * pg_step_oriented on `stream` without auto-reset, and writes remaining [N] (int32, may be NULL): the steps of the env's primitive
+ * still to take.  The primitives use the fork's unscaled actions: set pg_set_action_scale(env, 1.0, 1.0).  Plan state is not part
+ * of pg_save_state snapshots.  Errors: NULL plan or env, or a plan of another size or device, PG_ERR_ARG; a bare or joint-controlled
+ * handle PG_ERR_STATE; steps < 0 PG_ERR_ARG. */
+typedef struct pg_motion pg_motion;
+int pg_motion_create(int num_envs, int device, pg_motion** out);
+int pg_motion_destroy(pg_motion* plan);
+int pg_motion_move(pg_motion* plan, pg_env* env, const double* goal_pos, const double* goal_quat, const unsigned char* mask, void* stream);
+int pg_motion_gripper(pg_motion* plan, pg_env* env, double finger_action, int steps, const unsigned char* mask, void* stream);
+int pg_motion_step(pg_motion* plan, pg_env* env, float* obs, float* achieved_goal, float* desired_goal, float* reward,
+                   unsigned char* terminated, unsigned char* truncated, int* remaining, void* stream);
+
 /* The fork's camera path, PyBullet.render (panda_gym/pybullet.py:149-264) with the camera of get_cam2world_transforms (:70-107), for
  * every env of the handle: camera = {target x, y, z, distance, yaw, pitch, roll} (HOST, degrees; the reference's defaults are
  * {0,0,0, 1.4, 45, -30, 0}), fov 60, near 0.1, far 100.  Analytic ray casting of the primitives the kernels simulate (plane, table,

@@ -23,6 +23,7 @@ SYMBOLS = [
     "pg_inverse_kinematics", "pg_get_ee_pose", "pg_create_bare", "pg_set_motors", "pg_get_motors", "pg_sim_step", "pg_inverse_kinematics_link", "pg_get_link_state",
     "pg_save_state_async", "pg_restore_state_async", "pg_host_stage_allocations", "pg_reset_seeded", "pg_set_task_params", "pg_set_substeps",
     "pg_render", "pg_compute_reward_t", "pg_is_success_t", "pg_her_relabel_t", "pg_her_relabel_pitched", "pg_compute_reward_host_t", "pg_is_success_host_t", "pg_debug_schedule", "pg_debug_timing", "pg_diverged", "pg_contact_overflows", "pg_stats", "pg_kernel_launches", "pg_last_error",
+    "pg_motion_create", "pg_motion_destroy", "pg_motion_move", "pg_motion_gripper", "pg_motion_step",
 ]
 
 _lib = None
@@ -96,6 +97,11 @@ def load() -> ctypes.CDLL:
     lib.pg_diverged.argtypes = [vp, ctypes.POINTER(ctypes.c_longlong)]
     lib.pg_contact_overflows.argtypes = [vp, ctypes.POINTER(ctypes.c_longlong)]
     lib.pg_stats.argtypes = [vp, ctypes.POINTER(ctypes.c_double)]
+    lib.pg_motion_create.argtypes = [c_int, c_int, ctypes.POINTER(vp)]
+    lib.pg_motion_destroy.argtypes = [vp]
+    lib.pg_motion_move.argtypes = [vp, vp, vp, vp, vp, vp]
+    lib.pg_motion_gripper.argtypes = [vp, vp, cd, c_int, vp, vp]
+    lib.pg_motion_step.argtypes = [vp] * 10
     lib.pg_kernel_launches.restype = c_ll
     lib.pg_last_error.restype = ctypes.c_char_p
     _lib = lib

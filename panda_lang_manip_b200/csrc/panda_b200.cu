@@ -14,6 +14,7 @@
 #include "panda_model.h"
 #include "panda_scene.h"
 #include "panda_render.h"
+#include "panda_motion.cuh"
 
 namespace pg {
 long long g_launches = 0;
@@ -26,6 +27,9 @@ template <typename T, int TASK> cudaError_t configure_step(void);       // panda
 template <typename T> cudaError_t configure_bare(void);                 // panda_bare.cu
 template <typename T> void launch_render_setup(const EnvDev<T>& E, const RenderScene& R, RenderPrim* prims, cudaStream_t st);   // panda_render.cu
 void launch_render(const RenderPrim* prims, const RenderCamera& C, int n_envs, float* depth, unsigned char* rgba, unsigned char* seg, float* points, unsigned char* valid, cudaStream_t st);
+template <typename T> void launch_motion_move(const EnvDev<T>& E, const MotionPlan& P, const double* goal, const double* goal_quat, const unsigned char* mask, cudaStream_t st);   // panda_motion.cu
+void launch_motion_gripper(const MotionPlan& P, double finger, int steps, const unsigned char* mask, cudaStream_t st);
+template <typename T> void launch_motion_step(const EnvDev<T>& E, const MotionPlan& P, int act_dim, int* remaining, cudaStream_t st);
 #define PG_DECL(T, K)                                                                                        \
     extern template void launch_step<T, K>(const EnvDev<T>&, int, const StepIO&, cudaStream_t);              \
     extern template void launch_reset<T, K>(const EnvDev<T>&, const ResetIO&, cudaStream_t);                 \
@@ -748,6 +752,79 @@ int pg_diverged(pg_env* e, long long* count) {
 int pg_stats(pg_env* e, double out[4]) {
     if (!e || !out) return fail(PG_ERR_ARG, "pg_stats: NULL argument");
     return read_stats(e, 0, 4, out);
+}
+
+}  // extern "C"
+
+// Motion primitives: one allocation holds the plan rows (MotionPlan) and the step's scratch actions / orientations.
+struct pg_motion {
+    int n, device;
+    void* blob = nullptr;
+    MotionPlan P;
+};
+// the checks every motion entry point makes on its (plan, env) pair
+static int motion_env(pg_motion* m, pg_env* e, const char* who) {
+    if (!m || !e) return fail(PG_ERR_ARG, std::string(who) + ": NULL plan or env");
+    if (m->n != e->n || m->device != e->device) return fail(PG_ERR_ARG, std::string(who) + ": the plan was created for another batch size or device");
+    if (e->task == PG_TASK_BARE) return fail(PG_ERR_STATE, std::string(who) + ": a bare world has no ee action to drive");
+    if (e->ctrl != CTRL_EE) return fail(PG_ERR_STATE, std::string(who) + ": the motion primitives need an ee-controlled handle");
+    return PG_OK;
+}
+
+extern "C" {
+
+int pg_motion_create(int num_envs, int device, pg_motion** out) {
+    if (!out) return fail(PG_ERR_ARG, "pg_motion_create: out is NULL");
+    if (num_envs <= 0) return fail(PG_ERR_ARG, "pg_motion_create: num_envs must be > 0");
+    int rc = check_device(device, "pg_motion_create"); if (rc != PG_OK) return rc;
+    const size_t n = (size_t)num_envs;
+    const size_t f_bytes = MP_ROWS * n * sizeof(double), i_bytes = 3 * n * sizeof(int), act_bytes = 4 * n * sizeof(float), quat_bytes = 4 * n * sizeof(float);
+    pg_motion* m = new pg_motion();
+    m->n = num_envs; m->device = device;
+    cudaError_t ce = cudaMalloc(&m->blob, f_bytes + i_bytes + act_bytes + quat_bytes);
+    if (ce == cudaSuccess) ce = cudaMemset(m->blob, 0, f_bytes + i_bytes + act_bytes + quat_bytes);      // every env idle
+    if (ce != cudaSuccess) { cudaFree(m->blob); delete m; return cuda_fail(ce, "pg_motion_create"); }
+    char* b = (char*)m->blob;
+    m->P.n = num_envs;
+    m->P.f = (double*)b; b += f_bytes;
+    m->P.kind = (int*)b; m->P.step = m->P.kind + n; m->P.count = m->P.kind + 2 * n; b += i_bytes;
+    m->P.act = (float*)b; b += act_bytes;
+    m->P.quat = (float*)b;
+    *out = m;
+    return PG_OK;
+}
+int pg_motion_destroy(pg_motion* m) {
+    if (!m) return PG_OK;
+    cudaSetDevice(m->device);
+    cudaFree(m->blob);
+    delete m;
+    return PG_OK;
+}
+int pg_motion_move(pg_motion* m, pg_env* e, const double* goal_pos, const double* goal_quat, const unsigned char* mask, void* stream) {
+    int rc = motion_env(m, e, "pg_motion_move"); if (rc != PG_OK) return rc;
+    if (!goal_pos || !goal_quat) return fail(PG_ERR_ARG, "pg_motion_move: NULL goal_pos or goal_quat");
+    PG_CUDA(cudaSetDevice(e->device));
+    with_env(e, [&](auto& E) { launch_motion_move(E, m->P, goal_pos, goal_quat, mask, (cudaStream_t)stream); });
+    PG_CUDA(cudaGetLastError());
+    return PG_OK;
+}
+int pg_motion_gripper(pg_motion* m, pg_env* e, double finger_action, int steps, const unsigned char* mask, void* stream) {
+    if (steps < 0) return fail(PG_ERR_ARG, "pg_motion_gripper: steps must be >= 0");
+    int rc = motion_env(m, e, "pg_motion_gripper"); if (rc != PG_OK) return rc;
+    if (task_block_gripper(e->task)) return fail(PG_ERR_STATE, "pg_motion_gripper: this task blocks the gripper (Reach, Push, Slide have no finger action)");
+    PG_CUDA(cudaSetDevice(e->device));
+    launch_motion_gripper(m->P, finger_action, steps, mask, (cudaStream_t)stream);
+    PG_CUDA(cudaGetLastError());
+    return PG_OK;
+}
+int pg_motion_step(pg_motion* m, pg_env* e, float* obs, float* ag, float* dg, float* reward, unsigned char* terminated, unsigned char* truncated,
+                   int* remaining, void* stream) {
+    int rc = motion_env(m, e, "pg_motion_step"); if (rc != PG_OK) return rc;
+    PG_CUDA(cudaSetDevice(e->device));
+    return with_env(e, [&](auto& E) {
+        launch_motion_step(E, m->P, e->act_dim, remaining, (cudaStream_t)stream);
+        return step_impl(e, E, m->P.act, m->P.quat, obs, ag, dg, reward, terminated, truncated, 0, nullptr, nullptr, (cudaStream_t)stream, nullptr);
+    });
 }
 
 }  // extern "C"

@@ -381,6 +381,15 @@ template <typename T> PG_HD void rot_to_quat(const Frame<T>& F, T* q) {
     else if (R4 > R8) { T s = sqrt(T(1) + R4 - R0 - R8) * 2; q[3] = (R2 - R6) / s; q[0] = (R1 + R3) / s; q[1] = T(0.25) * s; q[2] = (R5 + R7) / s; }
     else { T s = sqrt(T(1) + R8 - R0 - R4) * 2; q[3] = (R3 - R1) / s; q[0] = (R2 + R6) / s; q[1] = (R5 + R7) / s; q[2] = T(0.25) * s; }
 }
+// End-effector (link 11) pose from joint vector q, as getLinkState(computeForwardKinematics=1) returns it: the link-11 origin sits on
+// the link-6 z axis, its axes are the link-6 axes rotated by -45 deg about z.  quat = (x, y, z, w).
+template <typename T> PG_HD void ee_pose(const Model<T>& M, const T* q, V3<T>& pos, T* quat) {
+    Frame<T> F[7]; fk_arm(M, q, F);
+    Frame<T> Ee; const T k = Consts<T>::k45;
+    Ee.p = F[6].p + F[6].Z * M.eez; Ee.X = (F[6].X - F[6].Y) * k; Ee.Y = (F[6].X + F[6].Y) * k; Ee.Z = F[6].Z;
+    pos = Ee.p;
+    rot_to_quat(Ee, quat);
+}
 template <typename T> PG_HD void ik_ee(const Model<T>& M, const T* q0, V3<T> target, const T* tq, T* qout) {
     T q[7];
 #pragma unroll

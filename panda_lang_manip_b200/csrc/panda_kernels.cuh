@@ -500,12 +500,9 @@ __global__ void __launch_bounds__(BLOCK) ee_pose_kernel(const __grid_constant__ 
     if (i >= E.n) return;
     T q[ND];
     for (int d = 0; d < ND; d++) q[d] = E.q[d * E.n + i];
-    Frame<T> F[7]; fk_arm(E.M, q, F);
-    Frame<T> Ee; const T k = Consts<T>::k45;
-    Ee.p = F[6].p + F[6].Z * E.M.eez; Ee.X = (F[6].X - F[6].Y) * k; Ee.Y = (F[6].X + F[6].Y) * k; Ee.Z = F[6].Z;
-    T qt[4]; rot_to_quat(Ee, qt);
+    V3<T> p; T qt[4]; ee_pose(E.M, q, p, qt);
     double* r = out + (size_t)i * 7;
-    r[0] = Ee.p.x; r[1] = Ee.p.y; r[2] = Ee.p.z; r[3] = qt[0]; r[4] = qt[1]; r[5] = qt[2]; r[6] = qt[3];
+    r[0] = p.x; r[1] = p.y; r[2] = p.z; r[3] = qt[0]; r[4] = qt[1]; r[5] = qt[2]; r[6] = qt[3];
 }
 
 // ---------------------------------------------------------------------------------------------- HER compute_reward / is_success
