@@ -55,15 +55,14 @@ int pg_dims(const pg_env* env, int* obs_dim, int* goal_dim, int* action_dim, int
 /* RobotTaskEnv.reset (core.py:240-250) for the envs whose mask byte is non-zero (NULL = all): neutral joints, zero
  * velocities, goal and object placement either sampled on the device (distributions of tasks/<task>.py _sample_goal /
  * _sample_object) or taken from goal_override [N,G] / object_override [N,3*n_objects] (float64; NULL = sample).
+ * seeds [N] uint64 (DEVICE) is RobotTaskEnv.reset(seed=k) batched (core.py:240-244: the task RNG is re-created from the seed):
+ * each reset env's draws are keyed by ITS seed alone, so equal seeds give equal goals / object placements in any env of any handle
+ * (reference test/seed_test.py); NULL keys them by the handle's seed, the global env index and the episode.  The draws come from
+ * the device's Philox stream, not numpy's PCG64 -- the single-env facade reproduces the reference's seeded values bit-for-bit on
+ * the host and injects them through the overrides.
  * Writes obs/ag/dg rows of the reset envs only (any of them may be NULL). */
-int pg_reset(pg_env* env, const unsigned char* mask, const double* goal_override, const double* object_override,
-             float* obs, float* achieved_goal, float* desired_goal, void* stream);
-/* RobotTaskEnv.reset(seed=k) batched (core.py:240-244: the task RNG is re-created from the seed): seeds [N] uint64 (DEVICE; NULL =
- * pg_reset) key each reset env's draws by ITS seed alone, so equal seeds give equal goals / object placements in any env of any
- * handle (reference test/seed_test.py).  The draws come from the device's Philox stream, not numpy's PCG64 -- the single-env facade
- * reproduces the reference's seeded values bit-for-bit on the host and injects them through the overrides. */
-int pg_reset_seeded(pg_env* env, const unsigned char* mask, const unsigned long long* seeds, const double* goal_override,
-                    const double* object_override, float* obs, float* achieved_goal, float* desired_goal, void* stream);
+int pg_reset(pg_env* env, const unsigned char* mask, const unsigned long long* seeds, const double* goal_override,
+             const double* object_override, float* obs, float* achieved_goal, float* desired_goal, void* stream);
 /* The task constructors' keyword arguments (tasks/reach.py:15-23 distance_threshold, goal_range; push.py:12-25; slide.py:12-27;
  * pick_and_place.py:13-29; stack.py:11-25; flip.py:13-24) as kernel parameters: the success / sparse-reward threshold used inside
  * pg_step, the goal noise box [low, high] (3 doubles each, HOST; what the reference builds from goal_range / goal_xy_range /
@@ -78,33 +77,30 @@ int pg_set_substeps(pg_env* env, int n_substeps);
  * (pybullet.py:52-55), _get_obs (core.py:229-238), is_success, compute_reward; truncated = TimeLimit.
  * auto_reset != 0: envs that terminated or truncated are reset in the same call (device-sampled goal/object) and their
  * obs/ag/dg rows hold the reset observation while reward/terminated/truncated describe the finished step.
+ * target_quat [N,4] (NULL = none) is the fork's orientation-target control (panda_gym/envs/robots/panda_ori.py:52-99:
+ * set_action(action, euler_xyz)): a per-env EE target quaternion (x,y,z,w; float32, normalised inside) fed to the IK instead of
+ * (1,0,0,0).  ee control only (PG_ERR_ARG otherwise).
+ * contacts / contact_count (NULL = no report) are pybullet getContactPoints after RobotTaskEnv.step, for every env: the contacts of
+ * the step's last sub-step (rows below; normalForce = applied impulse / timeStep) and their number per env.  contacts [N, C, 16]
+ * float32 with C = pg_max_contacts; rows at and beyond contact_count[i] are unspecified.  Row words:
+ *   0-2 contact point (world), as the contact model generates it;  3-5 normal on B, pointing from B to A (world);  6 normal force (N);
+ *   7 lateral friction force 1 (N), 8-10 its direction;  11 lateral friction force 2 (N), 12-14 its direction;  15 id_a + 32 * id_b
+ *   (an exact float).  Ids are pg_render's segmentation ids: 1 plane, 2 table, 3 / 4 objects, 14 hand (link 8), 15 / 16 fingers
+ *   (links 9 / 10).  There is no contactDistance.  With auto_reset the report describes the finished step, like reward.
  * Ordering: everything the call enqueues is ordered after the work already on `stream` and completes before work enqueued on
  * `stream` afterwards.  Batches of >= 4096 envs are advanced by several launches (a step cut into sub-step segments, each after a
  * re-sort of the thread -> env map) and, from 16384 envs, in env groups on streams the handle owns, forked from and joined back
  * to `stream` with events (legal under stream capture).  None of this changes a result. */
-int pg_step(pg_env* env, const float* actions, float* obs, float* achieved_goal, float* desired_goal, float* reward,
-            unsigned char* terminated, unsigned char* truncated, int auto_reset, void* stream);
-/* The fork's orientation-target control (panda_gym/envs/robots/panda_ori.py:52-99: set_action(action, euler_xyz)): as pg_step, with a
- * per-env EE target quaternion [N,4] (x,y,z,w; float32, normalised inside) fed to the IK instead of (1,0,0,0).  ee control only. */
-int pg_step_oriented(pg_env* env, const float* actions, const float* target_quat, float* obs, float* achieved_goal, float* desired_goal,
-                     float* reward, unsigned char* terminated, unsigned char* truncated, int auto_reset, void* stream);
-/* pybullet getContactPoints after RobotTaskEnv.step, for every env: as pg_step_oriented, plus the contacts of the step's last sub-step
- * (rows below; normalForce = applied impulse / timeStep) and their number per env.  contacts / contact_count may be NULL (DEVICE).
- * contacts [N, C, 16] float32 with C = pg_max_contacts; rows at and beyond contact_count[i] are unspecified.  Row words:
- *   0-2 contact point (world), as the contact model generates it;  3-5 normal on B, pointing from B to A (world);  6 normal force (N);
- *   7 lateral friction force 1 (N), 8-10 its direction;  11 lateral friction force 2 (N), 12-14 its direction;  15 id_a + 32 * id_b
- *   (an exact float).  Ids are pg_render's segmentation ids: 1 plane, 2 table, 3 / 4 objects, 14 hand (link 8), 15 / 16 fingers
- *   (links 9 / 10).  There is no contactDistance.  With auto_reset the report describes the finished step, like reward. */
-int pg_step_contacts(pg_env* env, const float* actions, const float* target_quat, float* obs, float* achieved_goal, float* desired_goal,
-                     float* reward, unsigned char* terminated, unsigned char* truncated, int auto_reset,
-                     float* contacts, unsigned char* contact_count, void* stream);
+int pg_step(pg_env* env, const float* actions, const float* target_quat, float* obs, float* achieved_goal, float* desired_goal,
+            float* reward, unsigned char* terminated, unsigned char* truncated, int auto_reset,
+            float* contacts, unsigned char* contact_count, void* stream);
 /* C of the rows above: contacts per env and sub-step of the handle's scene (10, or 22 for Stack; later candidates are dropped). */
 int pg_max_contacts(const pg_env* env, int* per_env);
 /* Action scaling of Panda.set_action: defaults 0.05 (ee / joint displacement, panda.py:81,103) and 0.2 (fingers, panda.py:65);
  * the fork's panda_cartesian.py:67,157 uses 1.0 / 1.0. */
 int pg_set_action_scale(pg_env* env, double ee_scale, double finger_scale);
-/* Same call with HOST buffers: actions are copied to the device, the step runs, all outputs are copied back and the
- * stream is synchronised before returning (the end-to-end path a CPU learner uses). */
+/* pg_step with HOST buffers and without orientation targets or contact report: actions are copied to the device, the step runs, all
+ * outputs are copied back and the stream is synchronised before returning (the end-to-end path a CPU learner uses). */
 int pg_step_host(pg_env* env, const float* actions, float* obs, float* achieved_goal, float* desired_goal, float* reward,
                  unsigned char* terminated, unsigned char* truncated, int auto_reset);
 
@@ -114,55 +110,39 @@ int pg_host_pin(void* ptr, size_t bytes);
 int pg_host_unpin(void* ptr);
 
 /* Task.compute_reward / Task.is_success (tasks/<task>.py, utils.py:4-30) on M rows of achieved/desired goals
- * (dtype PG_F32 or PG_F64 inputs; float32 rewards, uint8 success) -- the HER relabelling entry point. */
-int pg_compute_reward(int task, int reward_type, const void* achieved_goal, const void* desired_goal, float* reward,
-                      long long m, int dtype, void* stream);
-int pg_is_success(int task, const void* achieved_goal, const void* desired_goal, unsigned char* success, long long m,
-                  int dtype, void* stream);
-/* The same with the task's distance_threshold as an argument (the two calls above use the reference's defaults 0.05 / 0.1 / 0.2);
- * the threshold is compared in the dtype of the distance, as numpy does with a Python-float threshold. */
-int pg_compute_reward_t(int task, int reward_type, double threshold, const void* achieved_goal, const void* desired_goal,
-                        float* reward, long long m, int dtype, void* stream);
-int pg_is_success_t(int task, double threshold, const void* achieved_goal, const void* desired_goal, unsigned char* success,
-                    long long m, int dtype, void* stream);
+ * (dtype PG_F32 or PG_F64 inputs; float32 rewards, uint8 success) -- the HER relabelling entry point.  threshold is the task's
+ * distance_threshold (the reference's defaults: 0.05, 0.1 for Stack, 0.2 for Flip); it is compared in the dtype of the distance, as
+ * numpy does with a Python-float threshold. */
+int pg_compute_reward(int task, int reward_type, double threshold, const void* achieved_goal, const void* desired_goal,
+                      float* reward, long long m, int dtype, void* stream);
+int pg_is_success(int task, double threshold, const void* achieved_goal, const void* desired_goal, unsigned char* success,
+                  long long m, int dtype, void* stream);
 /* HER relabelling fused with compute_reward (replaces the gather + env.compute_reward round trip of stable-baselines3's
- * HerReplayBuffer that reference examples/train_push.py:1-12 sets up; rewards as tasks/<task>.py compute_reward).  next_achieved_goal and
- * desired_goal are the replay buffer's [R, G] goal arrays (device); for each of the M sampled transitions j: the new goal is
+ * HerReplayBuffer that reference examples/train_push.py:1-12 sets up; rewards as tasks/<task>.py compute_reward with threshold as
+ * above).  next_achieved_goal and desired_goal are the replay buffer's [R, G] goal arrays (device) with a row pitch of `pitch`
+ * elements (pitch >= G): a buffer that stores its goals padded to 32 bytes (pitch 8 for fp32 goals of 3, 4 or 6 components) makes
+ * every gathered row exactly one DRAM sector instead of one or two.  For each of the M sampled transitions j: the new goal is
  * next_achieved_goal[goal_src[j]] (desired_goal[src[j]] when goal_src[j] < 0) and the reward is compute_reward(next_achieved_goal[src[j]],
- * new goal).  Outputs: desired_goal_out [M, G], achieved_goal_out [M, G] (may be NULL), reward [M] float32. */
-int pg_her_relabel(int task, int reward_type, const void* next_achieved_goal, const void* desired_goal, const long long* src,
-                   const long long* goal_src, void* desired_goal_out, void* achieved_goal_out, float* reward, long long m, int dtype,
-                   void* stream);
-int pg_her_relabel_t(int task, int reward_type, double threshold, const void* next_achieved_goal, const void* desired_goal,
-                     const long long* src, const long long* goal_src, void* desired_goal_out, void* achieved_goal_out, float* reward,
-                     long long m, int dtype, void* stream);
-/* The same with a row pitch (elements) for the two replay-buffer goal arrays: a buffer that stores its goals padded to 32 bytes
- * (pitch 8 for fp32 goals of 3, 4 or 6 components) makes every gathered row exactly one DRAM sector instead of one or two.  Outputs
- * stay dense [M, G].  pitch >= G. */
-int pg_her_relabel_pitched(int task, int reward_type, double threshold, const void* next_achieved_goal, const void* desired_goal,
-                           long long pitch, const long long* src, const long long* goal_src, void* desired_goal_out,
-                           void* achieved_goal_out, float* reward, long long m, int dtype, void* stream);
+ * new goal).  Outputs (dense): desired_goal_out [M, G], achieved_goal_out [M, G] (may be NULL), reward [M] float32. */
+int pg_her_relabel(int task, int reward_type, double threshold, const void* next_achieved_goal, const void* desired_goal,
+                   long long pitch, const long long* src, const long long* goal_src, void* desired_goal_out,
+                   void* achieved_goal_out, float* reward, long long m, int dtype, void* stream);
 /* Task.compute_reward / is_success on HOST arrays (what RobotTaskEnv.compute_reward, core.py:226, is called with by a CPU learner). */
-int pg_compute_reward_host(int task, int reward_type, const void* achieved_goal, const void* desired_goal, float* reward,
-                           long long m, int dtype, int device);
-int pg_compute_reward_host_t(int task, int reward_type, double threshold, const void* achieved_goal, const void* desired_goal,
-                             float* reward, long long m, int dtype, int device);
-int pg_is_success_host_t(int task, double threshold, const void* achieved_goal, const void* desired_goal, unsigned char* success,
-                         long long m, int dtype, int device);
-int pg_is_success_host(int task, const void* achieved_goal, const void* desired_goal, unsigned char* success, long long m,
-                       int dtype, int device);
+int pg_compute_reward_host(int task, int reward_type, double threshold, const void* achieved_goal, const void* desired_goal,
+                           float* reward, long long m, int dtype, int device);
+int pg_is_success_host(int task, double threshold, const void* achieved_goal, const void* desired_goal, unsigned char* success,
+                       long long m, int dtype, int device);
 /* The two _host calls above stage through per-device buffers that only grow: number of (re)allocations so far (diagnostic). */
 long long pg_host_stage_allocations(void);
 
 /* RobotTaskEnv.save_state / restore_state / remove_state (core.py:252-278; pybullet.py:61-68,266-280): bit-exact device
- * snapshot of the whole batch (state, goals, episode counters). */
-int pg_save_state(pg_env* env, int* state_id);         /* blocking, on the legacy default stream */
-int pg_restore_state(pg_env* env, int state_id);
+ * snapshot of the whole batch (state, goals, episode counters).  Save and restore are one device-to-device copy enqueued on
+ * `stream`, with no synchronisation: with NULL (the legacy default stream), synchronise it if you need the copy complete.  A removed
+ * snapshot's buffer is reused by the next save, so a save / restore / remove loop allocates nothing after its first round and can be
+ * captured in a CUDA graph. */
+int pg_save_state(pg_env* env, int* state_id, void* stream);
+int pg_restore_state(pg_env* env, int state_id, void* stream);
 int pg_remove_state(pg_env* env, int state_id);
-/* Stream-ordered forms: one device-to-device copy enqueued on `stream`, no synchronisation; a removed snapshot's buffer is reused
- * by the next save, so a save / restore / remove loop allocates nothing after its first round and can be captured in a CUDA graph. */
-int pg_save_state_async(pg_env* env, int* state_id, void* stream);
-int pg_restore_state_async(pg_env* env, int state_id, void* stream);
 
 /* Raw state exchange for the facade getters/setters (pybullet.py:284-460) and the parity tests: float64 rows
  * [q(9) qd(9) | per object: pos(3) quat(4) lin(3) ang(3) | goal(G) | episode step], state_dim wide. */
@@ -193,7 +173,7 @@ int pg_get_ee_pose(pg_env* env, double* pose, void* stream);
  *     holding the current EE orientation.  Not for the blocked-gripper tasks Reach, Push and Slide (PG_ERR_STATE).
  * mask [N] (DEVICE, NULL = all) selects the envs a primitive begins on.  pg_motion_step writes each env's action and target
  * orientation (an env with no primitive left gets zero displacement, finger action 0 and its current orientation), then runs
- * pg_step_oriented on `stream` without auto-reset, and writes remaining [N] (int32, may be NULL): the steps of the env's primitive
+ * pg_step with the plan's orientations on `stream` without auto-reset, and writes remaining [N] (int32, may be NULL): the steps of the env's primitive
  * still to take.  The primitives use the fork's unscaled actions: set pg_set_action_scale(env, 1.0, 1.0).  Plan state is not part
  * of pg_save_state snapshots.  Errors: NULL plan or env, or a plan of another size or device, PG_ERR_ARG; a bare or joint-controlled
  * handle PG_ERR_STATE; steps < 0 PG_ERR_ARG. */

@@ -18,11 +18,11 @@ REWARD = {"sparse": 0, "dense": 1}
 PRECISION = {"f32": 0, "f64": 1}
 
 SYMBOLS = [
-    "pg_create", "pg_destroy", "pg_dims", "pg_reset", "pg_step", "pg_step_oriented", "pg_step_contacts", "pg_max_contacts", "pg_set_action_scale", "pg_step_host", "pg_host_pin", "pg_host_unpin", "pg_compute_reward", "pg_is_success",
+    "pg_create", "pg_destroy", "pg_dims", "pg_reset", "pg_step", "pg_max_contacts", "pg_set_action_scale", "pg_step_host", "pg_host_pin", "pg_host_unpin", "pg_compute_reward", "pg_is_success",
     "pg_compute_reward_host", "pg_is_success_host", "pg_her_relabel", "pg_save_state", "pg_restore_state", "pg_remove_state", "pg_get_state", "pg_set_state",
     "pg_inverse_kinematics", "pg_get_ee_pose", "pg_create_bare", "pg_set_motors", "pg_get_motors", "pg_sim_step", "pg_inverse_kinematics_link", "pg_get_link_state",
-    "pg_save_state_async", "pg_restore_state_async", "pg_host_stage_allocations", "pg_reset_seeded", "pg_set_task_params", "pg_set_substeps",
-    "pg_render", "pg_compute_reward_t", "pg_is_success_t", "pg_her_relabel_t", "pg_her_relabel_pitched", "pg_compute_reward_host_t", "pg_is_success_host_t", "pg_debug_schedule", "pg_debug_timing", "pg_diverged", "pg_contact_overflows", "pg_stats", "pg_kernel_launches", "pg_last_error",
+    "pg_host_stage_allocations", "pg_set_task_params", "pg_set_substeps",
+    "pg_render", "pg_debug_schedule", "pg_debug_timing", "pg_diverged", "pg_contact_overflows", "pg_stats", "pg_kernel_launches", "pg_last_error",
     "pg_motion_create", "pg_motion_destroy", "pg_motion_move", "pg_motion_gripper", "pg_motion_step",
 ]
 
@@ -46,27 +46,25 @@ def load() -> ctypes.CDLL:
     if not os.path.exists(LIB_PATH):
         raise PandaB200Error(f"{LIB_PATH} is missing: build the CUDA extension first (make -C {CSRC}); there is no CPU fallback")
     lib = ctypes.CDLL(LIB_PATH)
-    c_int, c_ll, c_ull, vp = ctypes.c_int, ctypes.c_longlong, ctypes.c_ulonglong, ctypes.c_void_p
+    c_int, c_ll, c_ull, vp, cd = ctypes.c_int, ctypes.c_longlong, ctypes.c_ulonglong, ctypes.c_void_p, ctypes.c_double
     pi = ctypes.POINTER(c_int)
     lib.pg_create.argtypes = [c_int, c_int, c_int, c_int, c_int, c_ull, c_ll, c_int, ctypes.POINTER(vp)]
     lib.pg_destroy.argtypes = [vp]
     lib.pg_dims.argtypes = [vp, pi, pi, pi, pi, pi]
-    lib.pg_reset.argtypes = [vp, vp, vp, vp, vp, vp, vp, vp]
-    lib.pg_step.argtypes = [vp, vp, vp, vp, vp, vp, vp, vp, c_int, vp]
-    lib.pg_step_oriented.argtypes = [vp, vp, vp, vp, vp, vp, vp, vp, vp, c_int, vp]
-    lib.pg_step_contacts.argtypes = [vp, vp, vp, vp, vp, vp, vp, vp, vp, c_int, vp, vp, vp]
+    lib.pg_reset.argtypes = [vp] * 9
+    lib.pg_step.argtypes = [vp, vp, vp, vp, vp, vp, vp, vp, vp, c_int, vp, vp, vp]
     lib.pg_max_contacts.argtypes = [vp, pi]
     lib.pg_set_action_scale.argtypes = [vp, ctypes.c_double, ctypes.c_double]
     lib.pg_step_host.argtypes = [vp, vp, vp, vp, vp, vp, vp, vp, c_int]
     lib.pg_host_pin.argtypes = [vp, ctypes.c_size_t]
     lib.pg_host_unpin.argtypes = [vp]
-    lib.pg_compute_reward.argtypes = [c_int, c_int, vp, vp, vp, c_ll, c_int, vp]
-    lib.pg_is_success.argtypes = [c_int, vp, vp, vp, c_ll, c_int, vp]
-    lib.pg_compute_reward_host.argtypes = [c_int, c_int, vp, vp, vp, c_ll, c_int, c_int]
-    lib.pg_is_success_host.argtypes = [c_int, vp, vp, vp, c_ll, c_int, c_int]
-    lib.pg_her_relabel.argtypes = [c_int, c_int, vp, vp, vp, vp, vp, vp, vp, c_ll, c_int, vp]
-    lib.pg_save_state.argtypes = [vp, pi]
-    lib.pg_restore_state.argtypes = [vp, c_int]
+    lib.pg_compute_reward.argtypes = [c_int, c_int, cd, vp, vp, vp, c_ll, c_int, vp]
+    lib.pg_is_success.argtypes = [c_int, cd, vp, vp, vp, c_ll, c_int, vp]
+    lib.pg_compute_reward_host.argtypes = [c_int, c_int, cd, vp, vp, vp, c_ll, c_int, c_int]
+    lib.pg_is_success_host.argtypes = [c_int, cd, vp, vp, vp, c_ll, c_int, c_int]
+    lib.pg_her_relabel.argtypes = [c_int, c_int, cd, vp, vp, c_ll, vp, vp, vp, vp, vp, c_ll, c_int, vp]
+    lib.pg_save_state.argtypes = [vp, pi, vp]
+    lib.pg_restore_state.argtypes = [vp, c_int, vp]
     lib.pg_remove_state.argtypes = [vp, c_int]
     lib.pg_get_state.argtypes = [vp, vp, vp]
     lib.pg_set_state.argtypes = [vp, vp, vp, vp]
@@ -78,20 +76,10 @@ def load() -> ctypes.CDLL:
     lib.pg_sim_step.argtypes = [vp, c_int, vp]
     lib.pg_inverse_kinematics_link.argtypes = [vp, c_int, vp, vp, vp, vp]
     lib.pg_get_link_state.argtypes = [vp, c_int, vp, vp]
-    lib.pg_save_state_async.argtypes = [vp, pi, vp]
-    lib.pg_restore_state_async.argtypes = [vp, c_int, vp]
     lib.pg_host_stage_allocations.restype = c_ll
-    cd = ctypes.c_double
-    lib.pg_reset_seeded.argtypes = [vp] * 9
     lib.pg_set_task_params.argtypes = [vp, cd, vp, vp, vp, vp]
     lib.pg_set_substeps.argtypes = [vp, c_int]
     lib.pg_render.argtypes = [vp, c_int, c_int, vp, c_int, vp, vp, vp, vp, vp, vp]
-    lib.pg_compute_reward_t.argtypes = [c_int, c_int, cd, vp, vp, vp, c_ll, c_int, vp]
-    lib.pg_is_success_t.argtypes = [c_int, cd, vp, vp, vp, c_ll, c_int, vp]
-    lib.pg_her_relabel_t.argtypes = [c_int, c_int, cd, vp, vp, vp, vp, vp, vp, vp, c_ll, c_int, vp]
-    lib.pg_her_relabel_pitched.argtypes = [c_int, c_int, cd, vp, vp, c_ll, vp, vp, vp, vp, vp, c_ll, c_int, vp]
-    lib.pg_compute_reward_host_t.argtypes = [c_int, c_int, cd, vp, vp, vp, c_ll, c_int, c_int]
-    lib.pg_is_success_host_t.argtypes = [c_int, cd, vp, vp, vp, c_ll, c_int, c_int]
     lib.pg_debug_schedule.argtypes = [vp, vp, vp]
     lib.pg_debug_timing.argtypes = [vp, vp]
     lib.pg_diverged.argtypes = [vp, ctypes.POINTER(ctypes.c_longlong)]

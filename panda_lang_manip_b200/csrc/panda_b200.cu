@@ -48,8 +48,6 @@ static int goal_layout(int task) { return task == TASK_STACK || task == TASK_FLI
 template <typename F> static auto with_dtype(int dtype, F&& f) { return dtype == PG_F32 ? f(float()) : f(double()); }
 static bool valid_task(int task) { return task >= 0 && task <= 5; }
 static bool valid_reward_type(int reward_type) { return reward_type >= 0 && reward_type <= 1; }
-// the reference's distance_threshold of a task; 0.0 for a bad task, which the _t form then rejects
-static double default_threshold(int task) { return valid_task(task) ? threshold_f64(task) : 0.0; }
 }  // namespace pg
 
 using namespace pg;
@@ -263,7 +261,7 @@ int pg_create(int task, int control_type, int reward_type, int num_envs, int dev
         for (int g = 0; g < e->groups; g++) { PG_CUDA(cudaStreamCreateWithFlags(&e->gstream[g], cudaStreamNonBlocking)); PG_CUDA(cudaEventCreateWithFlags(&e->ev_join[g], cudaEventDisableTiming)); }
     }
     *out = e;
-    rc = pg_reset(e, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr);
+    rc = pg_reset(e, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr);
     if (rc != PG_OK) { pg_destroy(e); *out = nullptr; return rc; }
     PG_CUDA(cudaDeviceSynchronize());
     return PG_OK;
@@ -347,11 +345,8 @@ int pg_dims(const pg_env* e, int* obs_dim, int* goal_dim, int* action_dim, int* 
     return PG_OK;
 }
 
-int pg_reset(pg_env* e, const unsigned char* mask, const double* goal_override, const double* object_override, float* obs, float* ag, float* dg, void* stream) {
-    return pg_reset_seeded(e, mask, nullptr, goal_override, object_override, obs, ag, dg, stream);
-}
-int pg_reset_seeded(pg_env* e, const unsigned char* mask, const unsigned long long* seeds, const double* goal_override, const double* object_override, float* obs, float* ag,
-                    float* dg, void* stream) {
+int pg_reset(pg_env* e, const unsigned char* mask, const unsigned long long* seeds, const double* goal_override, const double* object_override, float* obs, float* ag,
+             float* dg, void* stream) {
     if (!e) return fail(PG_ERR_ARG, "pg_reset: NULL handle");
     if (e->task == PG_TASK_BARE) return fail(PG_ERR_ARG, "pg_reset: a bare world has no task to reset; use pg_set_state");
     PG_CUDA(cudaSetDevice(e->device));
@@ -364,10 +359,6 @@ int pg_reset_seeded(pg_env* e, const unsigned char* mask, const unsigned long lo
     return PG_OK;
 }
 
-int pg_step(pg_env* e, const float* actions, float* obs, float* ag, float* dg, float* reward, unsigned char* terminated, unsigned char* truncated,
-            int auto_reset, void* stream) {
-    return pg_step_oriented(e, actions, nullptr, obs, ag, dg, reward, terminated, truncated, auto_reset, stream);
-}
 int pg_set_action_scale(pg_env* e, double ee_scale, double finger_scale) {
     if (!e || !(ee_scale > 0) || !(finger_scale > 0)) return fail(PG_ERR_ARG, "pg_set_action_scale: bad argument");
     e->Ef.M.ee_scale = (float)ee_scale; e->Ef.M.finger_scale = (float)finger_scale; e->Ed.M.ee_scale = ee_scale; e->Ed.M.finger_scale = finger_scale;
@@ -391,18 +382,14 @@ int pg_set_substeps(pg_env* e, int n_substeps) {
     e->Ef.P.nsub = e->Ed.P.nsub = n_substeps;
     return PG_OK;
 }
-int pg_step_contacts(pg_env* e, const float* actions, const float* target_quat, float* obs, float* ag, float* dg, float* reward, unsigned char* terminated,
-                     unsigned char* truncated, int auto_reset, float* contacts, unsigned char* contact_count, void* stream) {
+int pg_step(pg_env* e, const float* actions, const float* target_quat, float* obs, float* ag, float* dg, float* reward, unsigned char* terminated,
+            unsigned char* truncated, int auto_reset, float* contacts, unsigned char* contact_count, void* stream) {
     if (!e || !actions) return fail(PG_ERR_ARG, "pg_step: NULL handle or actions");
     if (e->task == PG_TASK_BARE) return fail(PG_ERR_ARG, "pg_step: a bare world is advanced with pg_sim_step");
-    if (target_quat && e->ctrl != CTRL_EE) return fail(PG_ERR_ARG, "pg_step_oriented: a target orientation needs ee control");
+    if (target_quat && e->ctrl != CTRL_EE) return fail(PG_ERR_ARG, "pg_step: a target orientation needs ee control");
     return with_env(e, [&](auto& E) {
         return step_impl(e, E, actions, target_quat, obs, ag, dg, reward, terminated, truncated, auto_reset, contacts, contact_count, (cudaStream_t)stream, nullptr);
     });
-}
-int pg_step_oriented(pg_env* e, const float* actions, const float* target_quat, float* obs, float* ag, float* dg, float* reward, unsigned char* terminated,
-                     unsigned char* truncated, int auto_reset, void* stream) {
-    return pg_step_contacts(e, actions, target_quat, obs, ag, dg, reward, terminated, truncated, auto_reset, nullptr, nullptr, stream);
 }
 int pg_max_contacts(const pg_env* e, int* per_env) {
     if (!e || !per_env) return fail(PG_ERR_ARG, "pg_max_contacts: NULL argument");
@@ -469,7 +456,7 @@ int pg_step_host(pg_env* e, const float* actions, float* obs, float* ag, float* 
     return PG_OK;
 }
 
-int pg_compute_reward_t(int task, int reward_type, double threshold, const void* ag, const void* dg, float* reward, long long m, int dtype, void* stream) {
+int pg_compute_reward(int task, int reward_type, double threshold, const void* ag, const void* dg, float* reward, long long m, int dtype, void* stream) {
     if (m == 0) return PG_OK;       // an empty batch is valid (its pointers may be NULL)
     if (!valid_task(task) || !valid_reward_type(reward_type) || !ag || !dg || !reward || m < 0 || !(threshold >= 0)) return fail(PG_ERR_ARG, "pg_compute_reward: bad argument");
     with_dtype(dtype, [&](auto x) {
@@ -479,7 +466,7 @@ int pg_compute_reward_t(int task, int reward_type, double threshold, const void*
     PG_CUDA(cudaGetLastError());
     return PG_OK;
 }
-int pg_is_success_t(int task, double threshold, const void* ag, const void* dg, unsigned char* success, long long m, int dtype, void* stream) {
+int pg_is_success(int task, double threshold, const void* ag, const void* dg, unsigned char* success, long long m, int dtype, void* stream) {
     if (m == 0) return PG_OK;
     if (!valid_task(task) || !ag || !dg || !success || m < 0 || !(threshold >= 0)) return fail(PG_ERR_ARG, "pg_is_success: bad argument");
     with_dtype(dtype, [&](auto x) {
@@ -489,32 +476,18 @@ int pg_is_success_t(int task, double threshold, const void* ag, const void* dg, 
     PG_CUDA(cudaGetLastError());
     return PG_OK;
 }
-int pg_compute_reward(int task, int reward_type, const void* ag, const void* dg, float* reward, long long m, int dtype, void* stream) {
-    return pg_compute_reward_t(task, reward_type, default_threshold(task), ag, dg, reward, m, dtype, stream);
-}
-int pg_is_success(int task, const void* ag, const void* dg, unsigned char* success, long long m, int dtype, void* stream) {
-    return pg_is_success_t(task, default_threshold(task), ag, dg, success, m, dtype, stream);
-}
-int pg_her_relabel_pitched(int task, int reward_type, double threshold, const void* next_ag, const void* dg, long long pitch, const long long* src, const long long* goal_src,
-                           void* dg_out, void* ag_out, float* reward, long long m, int dtype, void* stream) {
+int pg_her_relabel(int task, int reward_type, double threshold, const void* next_ag, const void* dg, long long pitch, const long long* src, const long long* goal_src,
+                   void* dg_out, void* ag_out, float* reward, long long m, int dtype, void* stream) {
     if (m == 0) return PG_OK;
     if (!valid_task(task) || !valid_reward_type(reward_type) || !next_ag || !dg || !src || !goal_src || !dg_out || !reward || m < 0 || !(threshold >= 0))
         return fail(PG_ERR_ARG, "pg_her_relabel: bad argument");
-    if (pitch < task_goal_dim(task)) return fail(PG_ERR_ARG, "pg_her_relabel_pitched: the row pitch is smaller than the goal dimension");
+    if (pitch < task_goal_dim(task)) return fail(PG_ERR_ARG, "pg_her_relabel: the row pitch is smaller than the goal dimension");
     with_dtype(dtype, [&](auto x) {
         using E = decltype(x);
         launch_her<E>(task, (const E*)next_ag, (const E*)dg, src, goal_src, (E*)dg_out, (E*)ag_out, reward, m, pitch, reward_type, threshold, (cudaStream_t)stream);
     });
     PG_CUDA(cudaGetLastError());
     return PG_OK;
-}
-int pg_her_relabel_t(int task, int reward_type, double threshold, const void* next_ag, const void* dg, const long long* src, const long long* goal_src, void* dg_out, void* ag_out,
-                     float* reward, long long m, int dtype, void* stream) {
-    return pg_her_relabel_pitched(task, reward_type, threshold, next_ag, dg, valid_task(task) ? task_goal_dim(task) : 0, src, goal_src, dg_out, ag_out, reward, m, dtype, stream);
-}
-int pg_her_relabel(int task, int reward_type, const void* next_ag, const void* dg, const long long* src, const long long* goal_src, void* dg_out, void* ag_out,
-                   float* reward, long long m, int dtype, void* stream) {
-    return pg_her_relabel_t(task, reward_type, default_threshold(task), next_ag, dg, src, goal_src, dg_out, ag_out, reward, m, dtype, stream);
 }
 // Host-array entry points (the path stable-baselines3's HerReplayBuffer takes through env_method("compute_reward"), reference
 // panda_gym/envs/core.py:226, examples/train_push.py:1-12).  Staging is cached per device and only ever grows: after the first call
@@ -549,7 +522,7 @@ static int reward_host(bool want_reward, int task, int reward_type, double thr, 
     int rc = stage_for(device, bytes, out_bytes, &h); if (rc != PG_OK) return rc;
     PG_CUDA(cudaMemcpyAsync(h->da, ag, bytes, cudaMemcpyHostToDevice, h->st));
     PG_CUDA(cudaMemcpyAsync(h->db, dg, bytes, cudaMemcpyHostToDevice, h->st));
-    rc = want_reward ? pg_compute_reward_t(task, reward_type, thr, h->da, h->db, (float*)h->dr, m, dtype, h->st) : pg_is_success_t(task, thr, h->da, h->db, (unsigned char*)h->dr, m, dtype, h->st);
+    rc = want_reward ? pg_compute_reward(task, reward_type, thr, h->da, h->db, (float*)h->dr, m, dtype, h->st) : pg_is_success(task, thr, h->da, h->db, (unsigned char*)h->dr, m, dtype, h->st);
     if (rc != PG_OK) return rc;
     const bool direct = host_pinned(result);
     PG_CUDA(cudaMemcpyAsync(direct ? result : h->hr, h->dr, out_bytes, cudaMemcpyDeviceToHost, h->st));
@@ -557,28 +530,22 @@ static int reward_host(bool want_reward, int task, int reward_type, double thr, 
     if (!direct) memcpy(result, h->hr, out_bytes);
     return PG_OK;
 }
-int pg_compute_reward_host_t(int task, int reward_type, double threshold, const void* ag, const void* dg, float* reward, long long m, int dtype, int device) {
+int pg_compute_reward_host(int task, int reward_type, double threshold, const void* ag, const void* dg, float* reward, long long m, int dtype, int device) {
     if (m == 0) return PG_OK;
     if (!valid_task(task) || !valid_reward_type(reward_type) || !ag || !dg || !reward || m < 0 || !(threshold >= 0)) return fail(PG_ERR_ARG, "pg_compute_reward_host: bad argument");
     return reward_host(true, task, reward_type, threshold, ag, dg, reward, m, dtype, device);
 }
-int pg_is_success_host_t(int task, double threshold, const void* ag, const void* dg, unsigned char* success, long long m, int dtype, int device) {
+int pg_is_success_host(int task, double threshold, const void* ag, const void* dg, unsigned char* success, long long m, int dtype, int device) {
     if (m == 0) return PG_OK;
     if (!valid_task(task) || !ag || !dg || !success || m < 0 || !(threshold >= 0)) return fail(PG_ERR_ARG, "pg_is_success_host: bad argument");
     return reward_host(false, task, 0, threshold, ag, dg, success, m, dtype, device);
-}
-int pg_compute_reward_host(int task, int reward_type, const void* ag, const void* dg, float* reward, long long m, int dtype, int device) {
-    return pg_compute_reward_host_t(task, reward_type, default_threshold(task), ag, dg, reward, m, dtype, device);
-}
-int pg_is_success_host(int task, const void* ag, const void* dg, unsigned char* success, long long m, int dtype, int device) {
-    return pg_is_success_host_t(task, default_threshold(task), ag, dg, success, m, dtype, device);
 }
 
 // Snapshots are stream-ordered: one device-to-device copy of the handle's single SoA allocation, enqueued on the caller's stream
 // (the env groups' streams are joined back to that stream by every pg_step, so ordering on it is sufficient).  No device-wide
 // synchronisation, no allocation when a removed snapshot's buffer can be reused -> a save / K x (restore, step) / remove loop can
 // be captured in a CUDA graph after its first, warm-up execution.
-int pg_save_state_async(pg_env* e, int* state_id, void* stream) {
+int pg_save_state(pg_env* e, int* state_id, void* stream) {
     if (!e || !state_id) return fail(PG_ERR_ARG, "pg_save_state: NULL argument");
     PG_CUDA(cudaSetDevice(e->device));
     void* p = nullptr;
@@ -589,23 +556,12 @@ int pg_save_state_async(pg_env* e, int* state_id, void* stream) {
     *state_id = e->next_snap++; e->snaps[*state_id] = p;
     return PG_OK;
 }
-int pg_restore_state_async(pg_env* e, int state_id, void* stream) {
+int pg_restore_state(pg_env* e, int state_id, void* stream) {
     if (!e) return fail(PG_ERR_ARG, "pg_restore_state: NULL handle");
     auto it = e->snaps.find(state_id);
     if (it == e->snaps.end()) return fail(PG_ERR_STATE, "pg_restore_state: unknown state id " + std::to_string(state_id));
     PG_CUDA(cudaSetDevice(e->device));
     PG_CUDA(cudaMemcpyAsync(e->blob, it->second, e->blob_bytes, cudaMemcpyDeviceToDevice, (cudaStream_t)stream));
-    return PG_OK;
-}
-// blocking forms on the legacy default stream (which orders against every blocking stream of the device)
-int pg_save_state(pg_env* e, int* state_id) {
-    int rc = pg_save_state_async(e, state_id, nullptr); if (rc != PG_OK) return rc;
-    PG_CUDA(cudaStreamSynchronize(nullptr));
-    return PG_OK;
-}
-int pg_restore_state(pg_env* e, int state_id) {
-    int rc = pg_restore_state_async(e, state_id, nullptr); if (rc != PG_OK) return rc;
-    PG_CUDA(cudaStreamSynchronize(nullptr));
     return PG_OK;
 }
 // The buffer goes back to the handle's pool: copies that still read or write it are ordered before any later reuse as long as the

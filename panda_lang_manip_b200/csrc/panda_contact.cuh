@@ -393,7 +393,7 @@ template <typename T, int NOBJ> PG_HD ContactCtx<T, NOBJ> contact_ctx(Contacts<T
 }
 
 // ---------------------------------------------------------------------------------------------- contact report
-// pybullet getContactPoints of the last sub-step, one row of REPORT_WORDS per contact (pg_step_contacts, include/panda_b200.h):
+// pybullet getContactPoints of the last sub-step, one row of REPORT_WORDS per contact (pg_step's contacts, include/panda_b200.h):
 // point (3), normal on B pointing from B to A (3), normal force, lateral friction force 1 and its direction (1 + 3), force 2 and its
 // direction (1 + 3), id_a + 32 id_b.  Forces are the solver's accumulated impulses / dt.  Body ids are the segmentation ids of
 // pg_render: 1 plane, 2 table, 3 / 4 objects, 14 hand, 15 / 16 fingers.  The record's distance word holds the normal row's rhs by now,

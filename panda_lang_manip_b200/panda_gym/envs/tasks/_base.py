@@ -55,8 +55,8 @@ class BuiltinTask(Task):
         a, d, lead, code = self._goals(achieved_goal, desired_goal)
         out = np.empty(lead, dtype=np.uint8)
         m = int(np.prod(lead)) if lead else 1
-        _lib.check(_lib.load().pg_is_success_host_t(_lib.TASKS[self.name], float(self.distance_threshold), a.ctypes.data, d.ctypes.data, out.ctypes.data, m, code,
-                                                    self.sim._require().device_index))
+        _lib.check(_lib.load().pg_is_success_host(_lib.TASKS[self.name], float(self.distance_threshold), a.ctypes.data, d.ctypes.data, out.ctypes.data, m, code,
+                                                  self.sim._require().device_index))
         return np.array(out.astype(np.bool_))
 
     def compute_reward(self, achieved_goal: np.ndarray, desired_goal: np.ndarray, info: Dict[str, Any] = {}) -> np.ndarray:
@@ -64,6 +64,6 @@ class BuiltinTask(Task):
         a, d, lead, code = self._goals(achieved_goal, desired_goal)
         out = np.empty(lead, dtype=np.float32)
         m = int(np.prod(lead)) if lead else 1
-        _lib.check(_lib.load().pg_compute_reward_host_t(_lib.TASKS[self.name], _lib.REWARD[self.reward_type], float(self.distance_threshold), a.ctypes.data, d.ctypes.data,
-                                                        out.ctypes.data, m, code, self.sim._require().device_index))
+        _lib.check(_lib.load().pg_compute_reward_host(_lib.TASKS[self.name], _lib.REWARD[self.reward_type], float(self.distance_threshold), a.ctypes.data, d.ctypes.data,
+                                                      out.ctypes.data, m, code, self.sim._require().device_index))
         return out

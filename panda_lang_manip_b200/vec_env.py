@@ -42,11 +42,11 @@ class _Handle:
         """Stream-ordered snapshot (one device-to-device copy on the current stream, no synchronisation)."""
         import ctypes
         sid = ctypes.c_int()
-        _lib.check(self.lib.pg_save_state_async(self._h, ctypes.byref(sid), self._stream()))
+        _lib.check(self.lib.pg_save_state(self._h, ctypes.byref(sid), self._stream()))
         return sid.value
 
     def restore_state(self, state_id: int) -> None:
-        _lib.check(self.lib.pg_restore_state_async(self._h, int(state_id), self._stream()))
+        _lib.check(self.lib.pg_restore_state(self._h, int(state_id), self._stream()))
 
     def remove_state(self, state_id: int) -> None:
         _lib.check(self.lib.pg_remove_state(self._h, int(state_id)))
@@ -178,7 +178,7 @@ class PandaVecEnv(_Handle):
         sd = None
         if seeds is not None:       # uint64 bit patterns travel as int64
             sd = torch.as_tensor(np.asarray(seeds.cpu() if torch.is_tensor(seeds) else seeds).astype(np.uint64).view(np.int64), device=self.device).reshape(self.num_envs).contiguous()
-        _lib.check(self.lib.pg_reset_seeded(self._h, _ptr(m), _ptr(sd), _ptr(g), _ptr(o), _ptr(self.obs), _ptr(self.achieved_goal), _ptr(self.desired_goal), self._stream()))
+        _lib.check(self.lib.pg_reset(self._h, _ptr(m), _ptr(sd), _ptr(g), _ptr(o), _ptr(self.obs), _ptr(self.achieved_goal), _ptr(self.desired_goal), self._stream()))
         if sd is not None:
             torch.cuda.current_stream(self.device).synchronize()
         return self._obs_dict()
@@ -209,9 +209,9 @@ class PandaVecEnv(_Handle):
         if a.shape != (self.num_envs, self.action_dim):
             raise ValueError(f"actions must be [{self.num_envs}, {self.action_dim}], got {tuple(a.shape)}")
         tq = None if target_orientation is None else target_orientation.to(device=self.device, dtype=torch.float32).reshape(self.num_envs, 4).contiguous()
-        _lib.check(self.lib.pg_step_contacts(self._h, _ptr(a), _ptr(tq), _ptr(self.obs), _ptr(self.achieved_goal), _ptr(self.desired_goal), _ptr(self.reward),
-                                             _ptr(self.terminated), _ptr(self.truncated), int(self.auto_reset), _ptr(self._contacts), _ptr(self._contact_count),
-                                             self._stream()))
+        _lib.check(self.lib.pg_step(self._h, _ptr(a), _ptr(tq), _ptr(self.obs), _ptr(self.achieved_goal), _ptr(self.desired_goal), _ptr(self.reward),
+                                    _ptr(self.terminated), _ptr(self.truncated), int(self.auto_reset), _ptr(self._contacts), _ptr(self._contact_count),
+                                    self._stream()))
         return self._obs_dict(), self.reward, self.terminated, self.truncated, {"is_success": self.terminated}
 
     def contacts(self) -> Dict[str, torch.Tensor]:
@@ -342,7 +342,7 @@ def compute_reward(task: str, reward_type: str, achieved_goal: torch.Tensor, des
     out = torch.empty(lead, dtype=torch.float32, device=a.device)
     thr = DEFAULT_THRESHOLD[task] if threshold is None else float(threshold)
     with torch.cuda.device(a.device):
-        _lib.check(_lib.load().pg_compute_reward_t(_lib.TASKS[task], _lib.REWARD[reward_type], thr, _ptr(a), _ptr(d), _ptr(out), m, code, torch.cuda.current_stream(a.device).cuda_stream))
+        _lib.check(_lib.load().pg_compute_reward(_lib.TASKS[task], _lib.REWARD[reward_type], thr, _ptr(a), _ptr(d), _ptr(out), m, code, torch.cuda.current_stream(a.device).cuda_stream))
     return out
 
 
@@ -351,7 +351,7 @@ def is_success(task: str, achieved_goal: torch.Tensor, desired_goal: torch.Tenso
     out = torch.empty(lead, dtype=torch.uint8, device=a.device)
     thr = DEFAULT_THRESHOLD[task] if threshold is None else float(threshold)
     with torch.cuda.device(a.device):
-        _lib.check(_lib.load().pg_is_success_t(_lib.TASKS[task], thr, _ptr(a), _ptr(d), _ptr(out), m, code, torch.cuda.current_stream(a.device).cuda_stream))
+        _lib.check(_lib.load().pg_is_success(_lib.TASKS[task], thr, _ptr(a), _ptr(d), _ptr(out), m, code, torch.cuda.current_stream(a.device).cuda_stream))
     return out.bool()
 
 
@@ -371,7 +371,7 @@ def her_relabel(task: str, reward_type: str, next_achieved_goal: torch.Tensor, d
 
     def rows(t):
         """[R, G] view and its row pitch in elements: a 2-D tensor whose rows are unit-stride slices of a wider (padded) buffer is used
-        in place (pg_her_relabel_pitched); anything else is flattened to dense rows."""
+        in place (the pitch argument of pg_her_relabel); anything else is flattened to dense rows."""
         t = t.to(device=next_achieved_goal.device, dtype=dt)
         if t.dim() == 2 and t.shape[1] == g and t.stride(1) == 1 and t.stride(0) >= g:
             return t, t.stride(0)
@@ -392,9 +392,9 @@ def her_relabel(task: str, reward_type: str, next_achieved_goal: torch.Tensor, d
     ag_out = torch.empty((m, g), dtype=dt, device=a.device) if return_achieved else None
     rew = torch.empty((m,), dtype=torch.float32, device=a.device)
     with torch.cuda.device(a.device):
-        _lib.check(_lib.load().pg_her_relabel_pitched(_lib.TASKS[task], _lib.REWARD[reward_type], DEFAULT_THRESHOLD[task] if threshold is None else float(threshold),
-                                                      _ptr(a), _ptr(d), pa, _ptr(s_), _ptr(gs), _ptr(new_dg), _ptr(ag_out), _ptr(rew),
-                                                      m, 1 if dt == torch.float64 else 0, torch.cuda.current_stream(a.device).cuda_stream))
+        _lib.check(_lib.load().pg_her_relabel(_lib.TASKS[task], _lib.REWARD[reward_type], DEFAULT_THRESHOLD[task] if threshold is None else float(threshold),
+                                              _ptr(a), _ptr(d), pa, _ptr(s_), _ptr(gs), _ptr(new_dg), _ptr(ag_out), _ptr(rew),
+                                              m, 1 if dt == torch.float64 else 0, torch.cuda.current_stream(a.device).cuda_stream))
     return (new_dg, rew, ag_out) if return_achieved else (new_dg, rew)
 
 

@@ -1,8 +1,8 @@
 """Cost of the batched motion primitives (CartesianMotion / pg_motion_step) on one GPU.
 
-1. Device time per env step, pg_motion_step against pg_step_oriented with the same actions: PickAndPlace at 32,768 envs (a release:
+1. Device time per env step, pg_motion_step against pg_step with the same actions and orientations: PickAndPlace at 32,768 envs (a release:
    finger action 1, zero displacement, the current EE orientation) and Reach ee at 65,536 envs (idle: zero displacement, the current
-   EE orientation).  Both legs start from the same snapshot; the pg_step_oriented leg reads each step's orientation with pg_get_ee_pose
+   EE orientation).  Both legs start from the same snapshot; the pg_step leg reads each step's orientation with pg_get_ee_pose
    outside its timed window, so both legs step the same trajectory.  Blocks of the two legs alternate.  CUDA events around every step;
    the state fits in L2 and is not flushed (the step kernel is compute-bound).  A move's motion step is timed as well.
 2. The per-step kernel's own device time (motion_step_kernel), from torch.profiler in a run of its own.

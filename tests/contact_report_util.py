@@ -1,4 +1,4 @@
-"""The contact report (pybullet getContactPoints after a step, pg_step_contacts): row layout, the oracle's rows, and physical invariants
+"""The contact report (pybullet getContactPoints after a step, pg_step's contacts): row layout, the oracle's rows, and physical invariants
 that any backend's report must satisfy on the scenes of tests/contact_kats.py."""
 import ctypes
 

@@ -38,20 +38,15 @@ def _ll():
 # entry point -> (arguments after the NULL handle, error text)
 NULL_HANDLE = {
     "pg_dims": (lambda: [_int() for _ in range(5)], "pg_dims: NULL handle"),
-    "pg_reset": (lambda: [P] * 6 + [None], "pg_reset: NULL handle"),
-    "pg_reset_seeded": (lambda: [P] * 7 + [None], "pg_reset: NULL handle"),
+    "pg_reset": (lambda: [P] * 7 + [None], "pg_reset: NULL handle"),
     "pg_set_task_params": (lambda: [0.05] + [P] * 4, "pg_set_task_params: needs a task handle"),
     "pg_set_substeps": (lambda: [20], "pg_set_substeps: needs a task handle (bare worlds pass the count to pg_sim_step)"),
-    "pg_step": (lambda: [P] * 7 + [1, None], "pg_step: NULL handle or actions"),
-    "pg_step_oriented": (lambda: [P] * 8 + [1, None], "pg_step: NULL handle or actions"),
-    "pg_step_contacts": (lambda: [P] * 8 + [1, P, P, None], "pg_step: NULL handle or actions"),
+    "pg_step": (lambda: [P] * 8 + [1, P, P, None], "pg_step: NULL handle or actions"),
     "pg_max_contacts": (lambda: [_int()], "pg_max_contacts: NULL argument"),
     "pg_set_action_scale": (lambda: [0.05, 0.2], "pg_set_action_scale: bad argument"),
     "pg_step_host": (lambda: [P] * 7 + [1], "pg_step_host: NULL handle or actions"),
-    "pg_save_state": (lambda: [_int()], "pg_save_state: NULL argument"),
-    "pg_save_state_async": (lambda: [_int(), None], "pg_save_state: NULL argument"),
-    "pg_restore_state": (lambda: [0], "pg_restore_state: NULL handle"),
-    "pg_restore_state_async": (lambda: [0, None], "pg_restore_state: NULL handle"),
+    "pg_save_state": (lambda: [_int(), None], "pg_save_state: NULL argument"),
+    "pg_restore_state": (lambda: [0, None], "pg_restore_state: NULL handle"),
     "pg_remove_state": (lambda: [0], "pg_remove_state: NULL handle"),
     "pg_get_state": (lambda: [P, None], "pg_get_state: NULL argument"),
     "pg_set_state": (lambda: [P, P, None], "pg_set_state: NULL argument"),
@@ -135,19 +130,13 @@ def test_create_bare_bad_body_row(lib, col, value):
     _rejected(lib, _create_bare(lib, [BODY, bad]), BODY_BAD)
 
 
-# goal-array entry points: name -> (takes reward_type, takes threshold, takes pitch, error text)
+# goal-array entry points (all take a threshold, pg_her_relabel also a row pitch): name -> (takes reward_type, error text)
 REWARD = {
-    "pg_compute_reward": (True, False, False, "pg_compute_reward: bad argument"),
-    "pg_compute_reward_t": (True, True, False, "pg_compute_reward: bad argument"),
-    "pg_is_success": (False, False, False, "pg_is_success: bad argument"),
-    "pg_is_success_t": (False, True, False, "pg_is_success: bad argument"),
-    "pg_compute_reward_host": (True, False, False, "pg_compute_reward_host: bad argument"),
-    "pg_compute_reward_host_t": (True, True, False, "pg_compute_reward_host: bad argument"),
-    "pg_is_success_host": (False, False, False, "pg_is_success_host: bad argument"),
-    "pg_is_success_host_t": (False, True, False, "pg_is_success_host: bad argument"),
-    "pg_her_relabel": (True, False, False, "pg_her_relabel: bad argument"),
-    "pg_her_relabel_t": (True, True, False, "pg_her_relabel: bad argument"),
-    "pg_her_relabel_pitched": (True, True, True, "pg_her_relabel: bad argument"),
+    "pg_compute_reward": (True, "pg_compute_reward: bad argument"),
+    "pg_is_success": (False, "pg_is_success: bad argument"),
+    "pg_compute_reward_host": (True, "pg_compute_reward_host: bad argument"),
+    "pg_is_success_host": (False, "pg_is_success_host: bad argument"),
+    "pg_her_relabel": (True, "pg_her_relabel: bad argument"),
 }
 
 
@@ -157,11 +146,11 @@ def _arrays(name):
 
 
 def _goal_call(lib, name, task=0, reward_type=0, threshold=0.05, arrays=None, m=4, pitch=3):
-    takes_rt, takes_thr, takes_pitch, _ = REWARD[name]
+    takes_rt, _ = REWARD[name]
     a = [P] * _arrays(name) if arrays is None else arrays
-    args = [task] + ([reward_type] if takes_rt else []) + ([threshold] if takes_thr else [])
+    args = [task] + ([reward_type] if takes_rt else []) + [threshold]
     if name.startswith("pg_her"):
-        args += a[:2] + ([pitch] if takes_pitch else []) + a[2:5] + [None, a[5]]      # achieved_goal_out may be NULL
+        args += a[:2] + [pitch] + a[2:5] + [None, a[5]]      # achieved_goal_out may be NULL
     else:
         args += a
     return getattr(lib, name)(*args, m, 0, 0 if "_host" in name else None)
@@ -169,7 +158,7 @@ def _goal_call(lib, name, task=0, reward_type=0, threshold=0.05, arrays=None, m=
 
 @pytest.mark.parametrize("name", sorted(REWARD))
 def test_goal_entry_points(lib, name):
-    takes_rt, takes_thr, takes_pitch, text = REWARD[name]
+    takes_rt, text = REWARD[name]
     for task in (-1, 6):
         _rejected(lib, _goal_call(lib, name, task=task), text)
     if takes_rt:
@@ -179,12 +168,11 @@ def test_goal_entry_points(lib, name):
         a = [P] * _arrays(name)
         a[k] = None
         _rejected(lib, _goal_call(lib, name, arrays=a), text)
-    if takes_thr:
-        for thr in (-0.05, float("nan")):
-            _rejected(lib, _goal_call(lib, name, threshold=thr), text)
+    for thr in (-0.05, float("nan")):
+        _rejected(lib, _goal_call(lib, name, threshold=thr), text)
     _rejected(lib, _goal_call(lib, name, m=-1), text)
-    if takes_pitch:
+    if name == "pg_her_relabel":
         for task, pitch in ((0, 2), (4, 5), (5, 3)):
             _rejected(lib, _goal_call(lib, name, task=task, pitch=pitch),
-                      "pg_her_relabel_pitched: the row pitch is smaller than the goal dimension")
+                      "pg_her_relabel: the row pitch is smaller than the goal dimension")
     assert _goal_call(lib, name, arrays=[None] * _arrays(name), m=0) == PG_OK

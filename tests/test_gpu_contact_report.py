@@ -1,4 +1,4 @@
-"""The contact report (PandaVecEnv(contact_report=True).contacts(), pg_step_contacts) on the GPU: the physical invariants of
+"""The contact report (PandaVecEnv(contact_report=True).contacts(), pg_step's contacts) on the GPU: the physical invariants of
 tests/contact_report_util.py, per-step parity with the oracle's report, no effect on any other output, invisibility of the scheduling,
 and the auto-reset rule (the report describes the finished step)."""
 import numpy as np

@@ -286,6 +286,16 @@ def test_oriented_ee_control_parity():
     assert worst_q < 1e-4 and worst_ee < 1e-4, (worst_q, worst_ee)
 
 
+def test_target_orientation_needs_ee_control():
+    import panda_lang_manip_b200 as p
+    env = p.PandaVecEnv("reach", 4, control_type="joints", auto_reset=False)
+    q = torch.tensor([[1.0, 0.0, 0.0, 0.0]] * 4, device="cuda")
+    with pytest.raises(p.PandaB200Error) as err:
+        env.step(torch.zeros((4, 7), device="cuda"), target_orientation=q)
+    assert str(err.value).endswith("pg_step: a target orientation needs ee control")
+    env.close()
+
+
 def test_edge_cases_ragged_unaligned_empty():
     """Ragged env counts (not a multiple of the 128-thread block, sorted and identity thread->env maps), unaligned goal views
     (scalar path of the reward kernel), empty batches, host-buffer stepping, every task's kernels."""

@@ -161,7 +161,7 @@ def test_motion_create_and_destroy_arguments(lib):
     assert lib.pg_motion_destroy(None) == PG_OK
 
 
-@pytest.mark.parametrize("plan,env", [(None, None), (None, P), (P, None)])
+@pytest.mark.parametrize("plan,env", [(None, None), (None, P), (P, None)], ids=["None-None", "None-ptr", "ptr-None"])   # P is an address: not an id
 def test_motion_null_plan_or_env(lib, plan, env):
     _rejected(lib, lib.pg_motion_move(plan, env, P, P, None, None), "pg_motion_move: NULL plan or env")
     _rejected(lib, lib.pg_motion_gripper(plan, env, -1.0, 30, None, None), "pg_motion_gripper: NULL plan or env")
