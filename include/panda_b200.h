@@ -28,7 +28,8 @@ typedef struct pg_env pg_env;
 
 /* Replaces PandaXxxEnv.__init__ (panda_gym/envs/panda_tasks.py:14-113: PyBullet + Panda at (-0.6,0,0) + task scene) for
  * num_envs environments.  precision: PG_F32 (product path) or PG_F64 (parity debugging).  seed + env_id_offset key the
- * device RNG by GLOBAL environment index, so a sharded run reproduces the unsharded one.  All envs start reset. */
+ * device RNG by GLOBAL environment index, so a sharded run reproduces the unsharded one.  All envs start reset.  *out is written
+ * only on success; after an error it is left as it was and nothing the call allocated is kept. */
 int pg_create(int task, int control_type, int reward_type, int num_envs, int device, unsigned long long seed,
               long long env_id_offset, int precision, pg_env** out);
 /* The reference's sim facade used WITHOUT a task (panda_gym/pybullet.py:16-68: PyBullet() + loadURDF :510-529 + create_box / create_cylinder
@@ -38,7 +39,8 @@ int pg_create(int task, int control_type, int reward_type, int num_envs, int dev
  * an optional table top at z = 0 over table_rect = {x0, x1, y0, y1} (HOST, NULL: none) and an optional ground plane at *ground_z
  * (HOST, NULL: none).  Joints start at 0 with the velocity motors loadURDF leaves (target 0, max impulse 1 per sub-step).
  * Such a handle is advanced with pg_sim_step and driven with pg_set_motors; pg_get_state / pg_set_state / pg_get_link_state /
- * pg_inverse_kinematics_link / snapshots work as on task handles (state rows without a goal). */
+ * pg_inverse_kinematics_link / snapshots work as on task handles (state rows without a goal).  *out is written only on success, as
+ * with pg_create. */
 int pg_create_bare(int num_envs, int device, int precision, const double* robot_base, int n_bodies, const double* bodies,
                    const double* table_rect, const double* ground_z, pg_env** out);
 /* PyBullet.control_joints -> setJointMotorControlArray (pybullet.py:462-477), per world: DEVICE rows [N, 9, 5] =

@@ -6,8 +6,11 @@
 #include <string.h>
 #include <algorithm>
 #include <map>
+#include <memory>
 #include <string>
 #include <type_traits>
+#include <utility>
+#include <variant>
 #include <vector>
 #include "panda_b200.h"
 #include "panda_kernels.cuh"
@@ -48,31 +51,78 @@ static int goal_layout(int task) { return task == TASK_STACK || task == TASK_FLI
 template <typename F> static auto with_dtype(int dtype, F&& f) { return dtype == PG_F32 ? f(float()) : f(double()); }
 static bool valid_task(int task) { return task >= 0 && task <= 5; }
 static bool valid_reward_type(int reward_type) { return reward_type >= 0 && reward_type <= 1; }
+
+// One CUDA resource: freed when its owner goes out of scope (a NULL one is not).  Move-only; the raw value is `p`.
+template <typename P, cudaError_t (*Free)(P)> struct Own {
+    P p{};
+    Own() = default;
+    Own(Own&& o) noexcept : p(o.p) { o.p = P{}; }
+    Own& operator=(Own&& o) noexcept { std::swap(p, o.p); return *this; }
+    ~Own() { if (p) Free(p); }
+};
+using DevBuf = Own<void*, cudaFree>;
+using PinnedBuf = Own<void*, cudaFreeHost>;
+using Stream = Own<cudaStream_t, cudaStreamDestroy>;
+using Event = Own<cudaEvent_t, cudaEventDestroy>;
+
+// page-locked (cudaHostAlloc / cudaHostRegister / pg_host_pin) host memory can be the source / target of an async copy directly
+static bool host_pinned(const void* p) {
+    cudaPointerAttributes a;
+    if (cudaPointerGetAttributes(&a, p) != cudaSuccess) { cudaGetLastError(); return false; }
+    return a.type == cudaMemoryTypeHost;
+}
+// The host ends of an async copy to or from a caller's host buffer: a page-locked buffer is copied directly, any other one goes
+// through pinned staging memory -- copied there before the upload (host_source), or out of it after the stream is synchronised
+// (host_target, then copy_back).  A NULL output is not copied.
+static const void* host_source(const void* user, void* stage, size_t bytes) { return host_pinned(user) ? user : memcpy(stage, user, bytes); }
+static void* host_target(void* user, void* stage) { return user && !host_pinned(user) ? stage : user; }
+static void copy_back(void* user, const void* target, size_t bytes) { if (target != user) memcpy(user, target, bytes); }
+
+// Staging of the host-buffer entry points: a private stream, one device input and one device output buffer, and a pinned mirror of
+// each.  It only grows: a direction that is too small is re-allocated 25 % larger than asked for, and its capacity is recorded only
+// once both of its buffers exist, so the next reserve after a failed one allocates again instead of using a half-built stage.
+struct Staging {
+    unsigned flags = cudaStreamNonBlocking;     // of the stream
+    Stream st; DevBuf d_in, d_out; PinnedBuf h_in, h_out; size_t cap_in = 0, cap_out = 0;
+    long long allocs = 0;                       // (re)allocations so far, one per direction
+    int reserve(size_t in_bytes, size_t out_bytes) {
+        if (!st.p) PG_CUDA(cudaStreamCreateWithFlags(&st.p, flags));
+        const int rc = in_bytes > cap_in ? grow(d_in, h_in, cap_in, in_bytes) : PG_OK;
+        return rc == PG_OK && out_bytes > cap_out ? grow(d_out, h_out, cap_out, out_bytes) : rc;
+    }
+    int grow(DevBuf& d, PinnedBuf& h, size_t& cap, size_t bytes) {
+        PG_CUDA(cudaStreamSynchronize(st.p));
+        cap = 0; d = DevBuf(); h = PinnedBuf();
+        const size_t c = bytes + bytes / 4;
+        PG_CUDA(cudaMalloc(&d.p, c)); PG_CUDA(cudaMallocHost(&h.p, c));
+        cap = c; allocs++;
+        return PG_OK;
+    }
+};
 }  // namespace pg
 
 using namespace pg;
 
 struct pg_env {
-    int task, ctrl, reward, n, device, precision;
+    int task, ctrl, reward, n, device;
     int obs_dim, goal_dim, act_dim, max_steps, state_dim, nobj;
-    void* blob = nullptr; size_t blob_bytes = 0;      // one allocation: q, qd, obj, goal, steps, episode, ret, stats
-    EnvDev<float> Ef; EnvDev<double> Ed;
-    std::map<int, void*> snaps; int next_snap = 0;
-    RenderPrim* prims = nullptr; RenderScene rscene;  // analytic renderer: per-env primitive lists (allocated at the first pg_render)
-    std::vector<void*> snap_pool;                    // buffers of removed snapshots, reused by the next save (no allocation in a save / remove loop)
+    DevBuf blob; size_t blob_bytes = 0;               // one allocation: q, qd, obj, goal, steps, episode, ret, stats
+    std::variant<EnvDev<float>, EnvDev<double>> env;  // the state in blob: EnvDev<float> for PG_F32 handles, EnvDev<double> for PG_F64
+    std::map<int, DevBuf> snaps; int next_snap = 0;
+    DevBuf prims; RenderScene rscene;                 // analytic renderer: per-env primitive lists (allocated at the first pg_render)
+    std::vector<DevBuf> snap_pool;                    // buffers of removed snapshots, reused by the next save (no allocation in a save / remove loop)
     // env groups: sorted batches are cut into groups of consecutive envs, each advanced on its own stream, so that the tail of
     // one group's launch (a few contact-heavy blocks) overlaps with the other groups' launches instead of idling the GPU
-    long long* dbg = nullptr;
-    int groups = 1; cudaStream_t gstream[8] = {}; cudaEvent_t ev_fork = nullptr, ev_join[8] = {};
+    DevBuf dbg;
+    int groups = 1; Stream gstream[8]; Event ev_fork, ev_join[8];
     int segments = 4;                                 // launches per step for sorted batches (see pg_create)
-    // host-buffer path: pinned staging + device I/O buffers + private stream
-    cudaStream_t hstream = nullptr;
-    float *h_act = nullptr, *h_out = nullptr; float* d_act = nullptr; float* d_out = nullptr; size_t out_floats = 0; size_t out_bytes = 0;
+    // pg_step_host's staging, on a blocking stream: like work on a caller's stream, it is ordered after what the legacy default stream holds
+    Staging host{cudaStreamDefault};
+    ~pg_env() { cudaSetDevice(device); }               // the members are freed after this body runs, on the handle's device
 };
 
-// f(E) with the handle's bound state: Ef for PG_F32 handles, Ed for PG_F64 ones.  Only that copy points at device memory (the
-// other one's pointers are NULL), so every read of a handle's device state goes through here.
-template <typename F> static auto with_env(pg_env* e, F&& f) { return e->precision == PG_F32 ? f(e->Ef) : f(e->Ed); }
+// f(E) with the handle's state
+template <typename F> static auto with_env(pg_env* e, F&& f) { return std::visit(f, e->env); }
 // One thread per env on `stream`: f(E, grid, st) launches a BLOCK-wide kernel over the bound state E.
 template <typename F> static int launch_per_env(pg_env* e, void* stream, F&& f) {
     PG_CUDA(cudaSetDevice(e->device));
@@ -167,12 +217,12 @@ template <typename T> static int step_impl(pg_env* e, EnvDev<T> E, const float* 
     // group g owns the envs (and thread slots) [g * gsize, min(n, (g + 1) * gsize)), gsize a multiple of the sort chunk
     const int gsize = ((e->n + groups - 1) / groups + PERM_CHUNK - 1) / PERM_CHUNK * PERM_CHUNK;
     const size_t A = e->act_dim, O = e->obs_dim, G = e->goal_dim;
-    if (groups > 1) PG_CUDA(cudaEventRecord(e->ev_fork, stream));
+    if (groups > 1) PG_CUDA(cudaEventRecord(e->ev_fork.p, stream));
     for (int g = 0; g < groups; g++) {
         const int t0 = g * gsize, cnt = std::min(e->n, t0 + gsize) - t0;
         if (cnt <= 0) break;
-        cudaStream_t st = groups > 1 ? e->gstream[g] : stream;
-        if (groups > 1) PG_CUDA(cudaStreamWaitEvent(st, e->ev_fork, 0));
+        cudaStream_t st = groups > 1 ? e->gstream[g].p : stream;
+        if (groups > 1) PG_CUDA(cudaStreamWaitEvent(st, e->ev_fork.p, 0));
         if (hio) PG_CUDA(cudaMemcpyAsync(const_cast<float*>(actions) + t0 * A, hio->act + t0 * A, (size_t)cnt * A * sizeof(float), cudaMemcpyHostToDevice, st));
         E.t0 = t0; E.tcount = cnt;
         const int nchunks = (cnt + PERM_CHUNK - 1) / PERM_CHUNK;
@@ -197,7 +247,7 @@ template <typename T> static int step_impl(pg_env* e, EnvDev<T> E, const float* 
             if (hio->term) PG_CUDA(cudaMemcpyAsync(hio->term + t0, terminated + t0, (size_t)cnt, cudaMemcpyDeviceToHost, st));
             if (hio->trunc) PG_CUDA(cudaMemcpyAsync(hio->trunc + t0, truncated + t0, (size_t)cnt, cudaMemcpyDeviceToHost, st));
         }
-        if (groups > 1) { PG_CUDA(cudaEventRecord(e->ev_join[g], st)); PG_CUDA(cudaStreamWaitEvent(stream, e->ev_join[g], 0)); }
+        if (groups > 1) { PG_CUDA(cudaEventRecord(e->ev_join[g].p, st)); PG_CUDA(cudaStreamWaitEvent(stream, e->ev_join[g].p, 0)); }
     }
     PG_CUDA(cudaGetLastError());
     return PG_OK;
@@ -216,15 +266,16 @@ static int check_device(int device, const char* who) {
     PG_CUDA(cudaSetDevice(device));
     return PG_OK;
 }
-// state allocation + model; the caller fills the scene
-static int alloc_state(pg_env* e, unsigned long long seed, long long env_id_offset, const double base[3]) {
+// the bound state for `precision`, its allocation and the model; the caller fills the scene and the task parameters
+static int alloc_state(pg_env* e, int precision, unsigned long long seed, long long env_id_offset, const double base[3]) {
+    with_dtype(precision, [&](auto x) { e->env.emplace<EnvDev<decltype(x)>>(); });
     return with_env(e, [&](auto& E) -> int {
         using T = std::remove_pointer_t<decltype(E.q)>;
         bind(E, e, nullptr, seed, env_id_offset);
-        cudaError_t err = cudaMalloc(&e->blob, e->blob_bytes);
+        cudaError_t err = cudaMalloc(&e->blob.p, e->blob_bytes);
         if (err != cudaSuccess) return cuda_fail(err, "cudaMalloc(state)");
-        PG_CUDA(cudaMemset(e->blob, 0, e->blob_bytes));
-        bind(E, e, (char*)e->blob, seed, env_id_offset); E.M = make_model<T>(base);
+        PG_CUDA(cudaMemset(e->blob.p, 0, e->blob_bytes));
+        bind(E, e, (char*)e->blob.p, seed, env_id_offset); E.M = make_model<T>(base);
         // the > 48 kB dynamic shared memory opt-in is per function and per device: done for this handle's device, errors reported
         cudaError_t ce = cudaSuccess;
         if (e->task == PG_TASK_BARE) ce = configure_bare<T>();
@@ -240,30 +291,29 @@ int pg_create(int task, int control_type, int reward_type, int num_envs, int dev
     if (!valid_task(task) || control_type < 0 || control_type > 1 || !valid_reward_type(reward_type) || num_envs <= 0 || precision < 0 || precision > 1)
         return fail(PG_ERR_ARG, "pg_create: bad task / control_type / reward_type / num_envs / precision");
     int rc = check_device(device, "pg_create"); if (rc != PG_OK) return rc;
-    pg_env* e = new pg_env();
-    e->task = task; e->ctrl = control_type; e->reward = reward_type; e->n = num_envs; e->device = device; e->precision = precision;
+    auto e = std::make_unique<pg_env>();
+    e->task = task; e->ctrl = control_type; e->reward = reward_type; e->n = num_envs; e->device = device;
     e->nobj = task_nobj(task); e->obs_dim = task_obs_dim(task); e->goal_dim = task_goal_dim(task); e->act_dim = task_act_dim(task, control_type);
     e->max_steps = task_max_steps(task); e->state_dim = 18 + 13 * e->nobj + e->goal_dim + 1;
     const double base[3] = {-0.6, 0.0, 0.0};   // panda_tasks.py:26,43,60,77,94,111
-    rc = alloc_state(e, seed, env_id_offset, base);
-    if (rc != PG_OK) { pg_destroy(e); return rc; }
-    e->Ef.S = make_scene<float>(task); e->Ed.S = make_scene<double>(task);
-    e->Ef.P = e->Ed.P = make_task_params(task);
+    rc = alloc_state(e.get(), precision, seed, env_id_offset, base); if (rc != PG_OK) return rc;
     const bool light = e->nobj == 0 && control_type == CTRL_JOINTS;
     e->segments = light ? 4 : 20;
-    { const char* v = getenv("PG_DEBUG_TIMING"); if (v && v[0] == '1') { PG_CUDA(cudaMalloc(&e->dbg, (size_t)e->n * 2 * sizeof(long long))); PG_CUDA(cudaMemset(e->dbg, 0, (size_t)e->n * 2 * sizeof(long long))); } }
-    e->Ef.dbg = e->dbg; e->Ed.dbg = e->dbg;
+    { const char* v = getenv("PG_DEBUG_TIMING"); if (v && v[0] == '1') { PG_CUDA(cudaMalloc(&e->dbg.p, (size_t)e->n * 2 * sizeof(long long))); PG_CUDA(cudaMemset(e->dbg.p, 0, (size_t)e->n * 2 * sizeof(long long))); } }
+    with_env(e.get(), [&](auto& E) {
+        using T = std::remove_pointer_t<decltype(E.q)>;
+        E.S = make_scene<T>(task); E.P = make_task_params(task); E.dbg = (long long*)e->dbg.p;
+    });
     // measured defaults (profiles/r1_notes.md): contact scenes and ee control re-sort before every sub-step and run 4 env groups (2 for ee-controlled Reach);
     // joint-controlled Reach (few contacts) keeps 4 launches per step on one stream
     e->groups = (num_envs >= 16384 && !light) ? (e->nobj == 0 ? 2 : 4) : 1;
     if (e->groups > 1) {
-        PG_CUDA(cudaEventCreateWithFlags(&e->ev_fork, cudaEventDisableTiming));
-        for (int g = 0; g < e->groups; g++) { PG_CUDA(cudaStreamCreateWithFlags(&e->gstream[g], cudaStreamNonBlocking)); PG_CUDA(cudaEventCreateWithFlags(&e->ev_join[g], cudaEventDisableTiming)); }
+        PG_CUDA(cudaEventCreateWithFlags(&e->ev_fork.p, cudaEventDisableTiming));
+        for (int g = 0; g < e->groups; g++) { PG_CUDA(cudaStreamCreateWithFlags(&e->gstream[g].p, cudaStreamNonBlocking)); PG_CUDA(cudaEventCreateWithFlags(&e->ev_join[g].p, cudaEventDisableTiming)); }
     }
-    *out = e;
-    rc = pg_reset(e, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr);
-    if (rc != PG_OK) { pg_destroy(e); *out = nullptr; return rc; }
+    rc = pg_reset(e.get(), nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr); if (rc != PG_OK) return rc;
     PG_CUDA(cudaDeviceSynchronize());
+    *out = e.release();
     return PG_OK;
 }
 
@@ -277,66 +327,50 @@ int pg_create_bare(int num_envs, int device, int precision, const double* robot_
         if ((b[0] != SH_BOX && b[0] != SH_CYL) || !(b[1] > 0) || !(b[2] > 0) || !(b[3] > 0) || !(b[4] > 0) || !(b[5] >= 0))
             return fail(PG_ERR_ARG, "pg_create_bare: body rows are [shape(0 box,1 z-cylinder) hx hy hz mass(>0) mu pos3 quat4]");
     }
+    double pose[MAXOBJ][7];                     // the bodies' creation poses, quaternions normalised
+    for (int o = 0; o < n_bodies; o++) {
+        const double* b = bodies + 13 * o;
+        const double nq = sqrt(b[9] * b[9] + b[10] * b[10] + b[11] * b[11] + b[12] * b[12]);
+        if (!(nq > 0)) return fail(PG_ERR_ARG, "pg_create_bare: zero quaternion");
+        for (int k = 0; k < 7; k++) pose[o][k] = k < 3 ? b[6 + k] : b[6 + k] / nq;
+    }
     int rc = check_device(device, "pg_create_bare"); if (rc != PG_OK) return rc;
-    pg_env* e = new pg_env();
-    e->task = PG_TASK_BARE; e->ctrl = CTRL_JOINTS; e->reward = 0; e->n = num_envs; e->device = device; e->precision = precision;
+    auto e = std::make_unique<pg_env>();
+    e->task = PG_TASK_BARE; e->ctrl = CTRL_JOINTS; e->reward = 0; e->n = num_envs; e->device = device;
     e->nobj = n_bodies; e->obs_dim = 0; e->goal_dim = 0; e->act_dim = 0; e->max_steps = 0; e->state_dim = 18 + 13 * n_bodies + 1;
     // a world without a robot still carries one (the kernels are built around it): it is parked 1 km up, out of reach of everything
     const double parked[3] = {0.0, 0.0, 1000.0};
-    rc = alloc_state(e, 0, 0, robot_base ? robot_base : parked);
-    if (rc != PG_OK) { pg_destroy(e); return rc; }
+    rc = alloc_state(e.get(), precision, 0, 0, robot_base ? robot_base : parked); if (rc != PG_OK) return rc;
     Scene<double> S = make_scene<double>(TASK_REACH);
     S.nobj = n_bodies;
     for (int o = 0; o < n_bodies; o++) { const double* b = bodies + 13 * o; scene_set_obj(S, o, (int)b[0], b[1], b[2], b[3], b[4], b[5]); }
     if (table_rect) { S.table_x0 = table_rect[0]; S.table_x1 = table_rect[1]; S.table_y0 = table_rect[2]; S.table_y1 = table_rect[3]; }
     else { S.table_x0 = 1.0; S.table_x1 = -1.0; S.table_y0 = 1.0; S.table_y1 = -1.0; }     // empty rectangle: no table
     S.ground_z = ground_z ? *ground_z : -1e30;                                               // no plane: nothing to land on
-    e->Ed.S = S; e->Ef.S = scene_cast<float>(S);
-    e->Ef.P = e->Ed.P = make_task_params(TASK_REACH);
+    with_env(e.get(), [&](auto& E) {
+        using T = std::remove_pointer_t<decltype(E.q)>;
+        E.S = scene_cast<T>(S); E.P = make_task_params(TASK_REACH);
+    });
     // initial state: joints at 0 (loadURDF), bodies at their creation poses, velocity motors (target 0, max impulse 1 per sub-step)
     std::vector<double> st((size_t)num_envs * e->state_dim, 0.0), mot((size_t)num_envs * 45, 0.0);
     for (int i = 0; i < num_envs; i++) {
         double* r = st.data() + (size_t)i * e->state_dim;
-        for (int o = 0; o < n_bodies; o++) {
-            const double* b = bodies + 13 * o; double* p = r + 18 + 13 * o;
-            double nq = sqrt(b[9] * b[9] + b[10] * b[10] + b[11] * b[11] + b[12] * b[12]);
-            if (!(nq > 0)) { pg_destroy(e); return fail(PG_ERR_ARG, "pg_create_bare: zero quaternion"); }
-            p[0] = b[6]; p[1] = b[7]; p[2] = b[8]; p[3] = b[9] / nq; p[4] = b[10] / nq; p[5] = b[11] / nq; p[6] = b[12] / nq;
-        }
+        for (int o = 0; o < n_bodies; o++) std::copy(pose[o], pose[o] + 7, r + 18 + 13 * o);
         for (int d = 0; d < 9; d++) { double* m = mot.data() + ((size_t)i * 9 + d) * 5; m[0] = 0.0; m[1] = 1.0; m[2] = 0.0; m[3] = 0.0; m[4] = 1.0 * 500.0; }
     }
-    double *d_st = nullptr, *d_mot = nullptr;
-    cudaError_t ce = cudaMalloc(&d_st, st.size() * sizeof(double)); if (ce == cudaSuccess) ce = cudaMalloc(&d_mot, mot.size() * sizeof(double));
-    if (ce == cudaSuccess) ce = cudaMemcpy(d_st, st.data(), st.size() * sizeof(double), cudaMemcpyHostToDevice);
-    if (ce == cudaSuccess) ce = cudaMemcpy(d_mot, mot.data(), mot.size() * sizeof(double), cudaMemcpyHostToDevice);
-    rc = ce == cudaSuccess ? PG_OK : cuda_fail(ce, "pg_create_bare: initial state upload");
-    if (rc == PG_OK) rc = pg_set_state(e, d_st, nullptr, nullptr);
-    if (rc == PG_OK) rc = pg_set_motors(e, d_mot, nullptr, nullptr);
-    if (rc == PG_OK) { ce = cudaDeviceSynchronize(); if (ce != cudaSuccess) rc = cuda_fail(ce, "pg_create_bare"); }
-    cudaFree(d_st); cudaFree(d_mot);
-    if (rc != PG_OK) { pg_destroy(e); return rc; }
-    *out = e;
+    DevBuf d_st, d_mot;
+    cudaError_t ce = cudaMalloc(&d_st.p, st.size() * sizeof(double)); if (ce == cudaSuccess) ce = cudaMalloc(&d_mot.p, mot.size() * sizeof(double));
+    if (ce == cudaSuccess) ce = cudaMemcpy(d_st.p, st.data(), st.size() * sizeof(double), cudaMemcpyHostToDevice);
+    if (ce == cudaSuccess) ce = cudaMemcpy(d_mot.p, mot.data(), mot.size() * sizeof(double), cudaMemcpyHostToDevice);
+    if (ce != cudaSuccess) return cuda_fail(ce, "pg_create_bare: initial state upload");
+    rc = pg_set_state(e.get(), (const double*)d_st.p, nullptr, nullptr); if (rc != PG_OK) return rc;
+    rc = pg_set_motors(e.get(), (const double*)d_mot.p, nullptr, nullptr); if (rc != PG_OK) return rc;
+    ce = cudaDeviceSynchronize(); if (ce != cudaSuccess) return cuda_fail(ce, "pg_create_bare");
+    *out = e.release();
     return PG_OK;
 }
 
-int pg_destroy(pg_env* e) {
-    if (!e) return PG_OK;
-    cudaSetDevice(e->device);
-    for (auto& kv : e->snaps) cudaFree(kv.second);
-    for (void* p : e->snap_pool) cudaFree(p);
-    if (e->h_act) cudaFreeHost(e->h_act);
-    if (e->h_out) cudaFreeHost(e->h_out);
-    if (e->d_act) cudaFree(e->d_act);
-    if (e->d_out) cudaFree(e->d_out);
-    if (e->hstream) cudaStreamDestroy(e->hstream);
-    for (int g = 0; g < 8; g++) { if (e->gstream[g]) cudaStreamDestroy(e->gstream[g]); if (e->ev_join[g]) cudaEventDestroy(e->ev_join[g]); }
-    if (e->ev_fork) cudaEventDestroy(e->ev_fork);
-    if (e->dbg) cudaFree(e->dbg);
-    if (e->prims) cudaFree(e->prims);
-    cudaFree(e->blob);
-    delete e;
-    return PG_OK;
-}
+int pg_destroy(pg_env* e) { delete e; return PG_OK; }
 
 int pg_dims(const pg_env* e, int* obs_dim, int* goal_dim, int* action_dim, int* max_episode_steps, int* state_dim) {
     if (!e) return fail(PG_ERR_ARG, "pg_dims: NULL handle");
@@ -361,7 +395,7 @@ int pg_reset(pg_env* e, const unsigned char* mask, const unsigned long long* see
 
 int pg_set_action_scale(pg_env* e, double ee_scale, double finger_scale) {
     if (!e || !(ee_scale > 0) || !(finger_scale > 0)) return fail(PG_ERR_ARG, "pg_set_action_scale: bad argument");
-    e->Ef.M.ee_scale = (float)ee_scale; e->Ef.M.finger_scale = (float)finger_scale; e->Ed.M.ee_scale = ee_scale; e->Ed.M.finger_scale = finger_scale;
+    with_env(e, [&](auto& E) { E.M.ee_scale = ee_scale; E.M.finger_scale = finger_scale; });
     return PG_OK;
 }
 int pg_set_task_params(pg_env* e, double distance_threshold, const double* goal_range_low, const double* goal_range_high, const double* obj_range_low, const double* obj_range_high) {
@@ -373,13 +407,13 @@ int pg_set_task_params(pg_env* e, double distance_threshold, const double* goal_
     for (int k = 0; k < 2; k++) { if (obj_range_low) P.obj_lo[k] = obj_range_low[k]; if (obj_range_high) P.obj_hi[k] = obj_range_high[k]; }
     for (int k = 0; k < 3; k++) if (!(P.goal_lo[k] <= P.goal_hi[k])) return fail(PG_ERR_ARG, "pg_set_task_params: goal range low > high");
     for (int k = 0; k < 2; k++) if (!(P.obj_lo[k] <= P.obj_hi[k])) return fail(PG_ERR_ARG, "pg_set_task_params: object range low > high");
-    e->Ef.P = e->Ed.P = P;
+    with_env(e, [&](auto& E) { E.P = P; });
     return PG_OK;
 }
 int pg_set_substeps(pg_env* e, int n_substeps) {
     if (!e || e->task == PG_TASK_BARE) return fail(PG_ERR_ARG, "pg_set_substeps: needs a task handle (bare worlds pass the count to pg_sim_step)");
     if (n_substeps < 1 || n_substeps > 1000) return fail(PG_ERR_ARG, "pg_set_substeps: 1 <= n_substeps <= 1000");
-    e->Ef.P.nsub = e->Ed.P.nsub = n_substeps;
+    with_env(e, [&](auto& E) { E.P.nsub = n_substeps; });
     return PG_OK;
 }
 int pg_step(pg_env* e, const float* actions, const float* target_quat, float* obs, float* ag, float* dg, float* reward, unsigned char* terminated,
@@ -398,26 +432,6 @@ int pg_max_contacts(const pg_env* e, int* per_env) {
     return PG_OK;
 }
 
-static int ensure_host_path(pg_env* e) {
-    if (e->hstream) return PG_OK;
-    const size_t n = (size_t)e->n;
-    // one pinned + one device output slab: obs | ag | dg | reward | terminated | truncated (flags padded to floats)
-    e->out_floats = n * (size_t)(e->obs_dim + 2 * e->goal_dim + 1) + (2 * n + 3) / 4 + 4;
-    e->out_bytes = e->out_floats * sizeof(float);
-    PG_CUDA(cudaStreamCreate(&e->hstream));
-    PG_CUDA(cudaMallocHost(&e->h_act, n * e->act_dim * sizeof(float)));
-    PG_CUDA(cudaMallocHost(&e->h_out, e->out_bytes));
-    PG_CUDA(cudaMalloc(&e->d_act, n * e->act_dim * sizeof(float)));
-    PG_CUDA(cudaMalloc(&e->d_out, e->out_bytes));
-    return PG_OK;
-}
-
-// page-locked (cudaHostAlloc / cudaHostRegister / pg_host_pin) host memory can be the source / target of an async copy directly
-static bool host_pinned(const void* p) {
-    cudaPointerAttributes a;
-    if (cudaPointerGetAttributes(&a, p) != cudaSuccess) { cudaGetLastError(); return false; }
-    return a.type == cudaMemoryTypeHost;
-}
 int pg_host_pin(void* ptr, size_t bytes) {
     if (!ptr || bytes == 0) return fail(PG_ERR_ARG, "pg_host_pin: bad argument");
     PG_CUDA(cudaHostRegister(ptr, bytes, cudaHostRegisterDefault));
@@ -433,26 +447,26 @@ int pg_step_host(pg_env* e, const float* actions, float* obs, float* ag, float* 
     if (!e || !actions) return fail(PG_ERR_ARG, "pg_step_host: NULL handle or actions");
     if (e->task == PG_TASK_BARE) return fail(PG_ERR_ARG, "pg_step_host: a bare world is advanced with pg_sim_step");
     PG_CUDA(cudaSetDevice(e->device));
-    int rc = ensure_host_path(e); if (rc != PG_OK) return rc;
-    const size_t n = (size_t)e->n, O = e->obs_dim, G = e->goal_dim;
-    // pageable buffers go through the handle's pinned staging slabs (one extra host copy each way); pinned ones are copied directly
-    const float* src = actions;
-    if (!host_pinned(actions)) { memcpy(e->h_act, actions, n * e->act_dim * sizeof(float)); src = e->h_act; }
-    float* d_obs = e->d_out; float* d_ag = d_obs + n * O; float* d_dg = d_ag + n * G; float* d_rew = d_dg + n * G;
-    unsigned char* d_term = (unsigned char*)(d_rew + n); unsigned char* d_trunc = d_term + n;
-    struct Out { void* user; const void* dev; void* host; size_t bytes; bool direct; };
-    Out outs[6] = {{obs, d_obs, nullptr, n * O * sizeof(float), false}, {ag, d_ag, nullptr, n * G * sizeof(float), false}, {dg, d_dg, nullptr, n * G * sizeof(float), false},
-                   {reward, d_rew, nullptr, n * sizeof(float), false}, {terminated, d_term, nullptr, n, false}, {truncated, d_trunc, nullptr, n, false}};
-    for (Out& o : outs) {
-        if (!o.user) continue;
-        o.direct = host_pinned(o.user);
-        o.host = o.direct ? o.user : (void*)((char*)e->h_out + ((const char*)o.dev - (const char*)e->d_out));
-    }
-    HostIO hio{src, (float*)outs[0].host, (float*)outs[1].host, (float*)outs[2].host, (float*)outs[3].host, (unsigned char*)outs[4].host, (unsigned char*)outs[5].host};
-    rc = with_env(e, [&](auto& E) { return step_impl(e, E, e->d_act, nullptr, d_obs, d_ag, d_dg, d_rew, d_term, d_trunc, auto_reset, nullptr, nullptr, e->hstream, &hio); });
+    const size_t n = (size_t)e->n, O = e->obs_dim, G = e->goal_dim, act_bytes = n * e->act_dim * sizeof(float);
+    // the outputs share one device slab and its pinned mirror: obs | ag | dg | reward | terminated | truncated
+    void* user[6] = {obs, ag, dg, reward, terminated, truncated};
+    const size_t bytes[6] = {n * O * sizeof(float), n * G * sizeof(float), n * G * sizeof(float), n * sizeof(float), n, n};
+    size_t off[7] = {0};
+    for (int k = 0; k < 6; k++) off[k + 1] = off[k] + bytes[k];
+    Staging& s = e->host;
+    int rc = s.reserve(act_bytes, off[6]); if (rc != PG_OK) return rc;
+    char* dev = (char*)s.d_out.p;
+    void* host[6];
+    for (int k = 0; k < 6; k++) host[k] = host_target(user[k], (char*)s.h_out.p + off[k]);
+    HostIO hio{(const float*)host_source(actions, s.h_in.p, act_bytes), (float*)host[0], (float*)host[1], (float*)host[2], (float*)host[3],
+               (unsigned char*)host[4], (unsigned char*)host[5]};
+    rc = with_env(e, [&](auto& E) {
+        return step_impl(e, E, (float*)s.d_in.p, nullptr, (float*)(dev + off[0]), (float*)(dev + off[1]), (float*)(dev + off[2]), (float*)(dev + off[3]),
+                         (unsigned char*)(dev + off[4]), (unsigned char*)(dev + off[5]), auto_reset, nullptr, nullptr, s.st.p, &hio);
+    });
     if (rc != PG_OK) return rc;
-    PG_CUDA(cudaStreamSynchronize(e->hstream));
-    for (const Out& o : outs) if (o.user && !o.direct) memcpy(o.user, o.host, o.bytes);
+    PG_CUDA(cudaStreamSynchronize(s.st.p));
+    for (int k = 0; k < 6; k++) copy_back(user[k], host[k], bytes[k]);
     return PG_OK;
 }
 
@@ -490,44 +504,32 @@ int pg_her_relabel(int task, int reward_type, double threshold, const void* next
     return PG_OK;
 }
 // Host-array entry points (the path stable-baselines3's HerReplayBuffer takes through env_method("compute_reward"), reference
-// panda_gym/envs/core.py:226, examples/train_push.py:1-12).  Staging is cached per device and only ever grows: after the first call
-// of a given size there is no allocation, one private stream carries H2D -> kernel -> D2H, one stream synchronisation at the end.
-struct HostStage { cudaStream_t st = nullptr; void *da = nullptr, *db = nullptr, *dr = nullptr, *hr = nullptr; size_t cap_in = 0, cap_out = 0; };
-static HostStage g_stage[64];
-static long long g_stage_allocs = 0;
-static int stage_for(int device, size_t in_bytes, size_t out_bytes, HostStage** out) {
+// panda_gym/envs/core.py:226, examples/train_push.py:1-12).  They stage through one Staging per device: after the first call of a
+// given size there is no allocation, its stream carries H2D -> kernel -> D2H, one stream synchronisation at the end.  The stages
+// are never destroyed: at process exit the CUDA runtime may be gone before static destructors run.
+static Staging* const device_stages = new Staging[64];
+long long pg_host_stage_allocations(void) {
+    long long allocs = 0;
+    for (int d = 0; d < 64; d++) allocs += device_stages[d].allocs;
+    return allocs;
+}
+static int reward_host(bool want_reward, int task, int reward_type, double thr, const void* ag, const void* dg, void* result, long long m, int dtype, int device) {
     if (device < 0 || device >= 64) return fail(PG_ERR_ARG, "host path: bad device index");
     int rc = check_device(device, "host path"); if (rc != PG_OK) return rc;
-    HostStage& h = g_stage[device];
-    if (!h.st) PG_CUDA(cudaStreamCreateWithFlags(&h.st, cudaStreamNonBlocking));
-    if (in_bytes > h.cap_in) {
-        PG_CUDA(cudaStreamSynchronize(h.st));
-        if (h.da) cudaFree(h.da); if (h.db) cudaFree(h.db); h.da = h.db = nullptr; h.cap_in = 0;
-        const size_t cap = in_bytes + in_bytes / 4;
-        PG_CUDA(cudaMalloc(&h.da, cap)); PG_CUDA(cudaMalloc(&h.db, cap)); h.cap_in = cap; g_stage_allocs++;
-    }
-    if (out_bytes > h.cap_out) {
-        PG_CUDA(cudaStreamSynchronize(h.st));
-        if (h.dr) cudaFree(h.dr); if (h.hr) cudaFreeHost(h.hr); h.dr = h.hr = nullptr; h.cap_out = 0;
-        const size_t cap = out_bytes + out_bytes / 4;
-        PG_CUDA(cudaMalloc(&h.dr, cap)); PG_CUDA(cudaMallocHost(&h.hr, cap)); h.cap_out = cap; g_stage_allocs++;
-    }
-    *out = &h;
-    return PG_OK;
-}
-long long pg_host_stage_allocations(void) { return g_stage_allocs; }
-static int reward_host(bool want_reward, int task, int reward_type, double thr, const void* ag, const void* dg, void* result, long long m, int dtype, int device) {
     const size_t es = with_dtype(dtype, [](auto x) { return sizeof(x); }), bytes = (size_t)m * task_goal_dim(task) * es, out_bytes = (size_t)m * (want_reward ? 4 : 1);
-    HostStage* h = nullptr;
-    int rc = stage_for(device, bytes, out_bytes, &h); if (rc != PG_OK) return rc;
-    PG_CUDA(cudaMemcpyAsync(h->da, ag, bytes, cudaMemcpyHostToDevice, h->st));
-    PG_CUDA(cudaMemcpyAsync(h->db, dg, bytes, cudaMemcpyHostToDevice, h->st));
-    rc = want_reward ? pg_compute_reward(task, reward_type, thr, h->da, h->db, (float*)h->dr, m, dtype, h->st) : pg_is_success(task, thr, h->da, h->db, (unsigned char*)h->dr, m, dtype, h->st);
+    const size_t dg_off = (bytes + 255) & ~(size_t)255;      // dg 256-byte aligned like ag: reward_kernel's 16-byte loads need both
+    Staging& s = device_stages[device];
+    rc = s.reserve(dg_off + bytes, out_bytes); if (rc != PG_OK) return rc;
+    char *d_in = (char*)s.d_in.p, *h_in = (char*)s.h_in.p;
+    PG_CUDA(cudaMemcpyAsync(d_in, host_source(ag, h_in, bytes), bytes, cudaMemcpyHostToDevice, s.st.p));
+    PG_CUDA(cudaMemcpyAsync(d_in + dg_off, host_source(dg, h_in + dg_off, bytes), bytes, cudaMemcpyHostToDevice, s.st.p));
+    rc = want_reward ? pg_compute_reward(task, reward_type, thr, d_in, d_in + dg_off, (float*)s.d_out.p, m, dtype, s.st.p)
+                     : pg_is_success(task, thr, d_in, d_in + dg_off, (unsigned char*)s.d_out.p, m, dtype, s.st.p);
     if (rc != PG_OK) return rc;
-    const bool direct = host_pinned(result);
-    PG_CUDA(cudaMemcpyAsync(direct ? result : h->hr, h->dr, out_bytes, cudaMemcpyDeviceToHost, h->st));
-    PG_CUDA(cudaStreamSynchronize(h->st));
-    if (!direct) memcpy(result, h->hr, out_bytes);
+    void* host = host_target(result, s.h_out.p);
+    PG_CUDA(cudaMemcpyAsync(host, s.d_out.p, out_bytes, cudaMemcpyDeviceToHost, s.st.p));
+    PG_CUDA(cudaStreamSynchronize(s.st.p));
+    copy_back(result, host, out_bytes);
     return PG_OK;
 }
 int pg_compute_reward_host(int task, int reward_type, double threshold, const void* ag, const void* dg, float* reward, long long m, int dtype, int device) {
@@ -548,12 +550,12 @@ int pg_is_success_host(int task, double threshold, const void* ag, const void* d
 int pg_save_state(pg_env* e, int* state_id, void* stream) {
     if (!e || !state_id) return fail(PG_ERR_ARG, "pg_save_state: NULL argument");
     PG_CUDA(cudaSetDevice(e->device));
-    void* p = nullptr;
-    if (!e->snap_pool.empty()) { p = e->snap_pool.back(); e->snap_pool.pop_back(); }
-    else PG_CUDA(cudaMalloc(&p, e->blob_bytes));
-    cudaError_t ce = cudaMemcpyAsync(p, e->blob, e->blob_bytes, cudaMemcpyDeviceToDevice, (cudaStream_t)stream);
-    if (ce != cudaSuccess) { e->snap_pool.push_back(p); return cuda_fail(ce, "cudaMemcpyAsync(snapshot)"); }
-    *state_id = e->next_snap++; e->snaps[*state_id] = p;
+    DevBuf p;
+    if (!e->snap_pool.empty()) { p = std::move(e->snap_pool.back()); e->snap_pool.pop_back(); }
+    else PG_CUDA(cudaMalloc(&p.p, e->blob_bytes));
+    cudaError_t ce = cudaMemcpyAsync(p.p, e->blob.p, e->blob_bytes, cudaMemcpyDeviceToDevice, (cudaStream_t)stream);
+    if (ce != cudaSuccess) { e->snap_pool.push_back(std::move(p)); return cuda_fail(ce, "cudaMemcpyAsync(snapshot)"); }
+    *state_id = e->next_snap++; e->snaps[*state_id] = std::move(p);
     return PG_OK;
 }
 int pg_restore_state(pg_env* e, int state_id, void* stream) {
@@ -561,7 +563,7 @@ int pg_restore_state(pg_env* e, int state_id, void* stream) {
     auto it = e->snaps.find(state_id);
     if (it == e->snaps.end()) return fail(PG_ERR_STATE, "pg_restore_state: unknown state id " + std::to_string(state_id));
     PG_CUDA(cudaSetDevice(e->device));
-    PG_CUDA(cudaMemcpyAsync(e->blob, it->second, e->blob_bytes, cudaMemcpyDeviceToDevice, (cudaStream_t)stream));
+    PG_CUDA(cudaMemcpyAsync(e->blob.p, it->second.p, e->blob_bytes, cudaMemcpyDeviceToDevice, (cudaStream_t)stream));
     return PG_OK;
 }
 // The buffer goes back to the handle's pool: copies that still read or write it are ordered before any later reuse as long as the
@@ -570,7 +572,7 @@ int pg_remove_state(pg_env* e, int state_id) {
     if (!e) return fail(PG_ERR_ARG, "pg_remove_state: NULL handle");
     auto it = e->snaps.find(state_id);
     if (it == e->snaps.end()) return fail(PG_ERR_STATE, "pg_remove_state: unknown state id " + std::to_string(state_id));
-    e->snap_pool.push_back(it->second); e->snaps.erase(it);
+    e->snap_pool.push_back(std::move(it->second)); e->snaps.erase(it);
     return PG_OK;
 }
 
@@ -638,7 +640,7 @@ int pg_render(pg_env* e, int width, int height, const double* camera, int crop, 
     if (!e || !camera || width <= 0 || height <= 0 || width > 4096 || height > 4096) return fail(PG_ERR_ARG, "pg_render: bad argument");
     if (valid && !points) return fail(PG_ERR_ARG, "pg_render: valid is the point cloud's mask, it needs points");
     PG_CUDA(cudaSetDevice(e->device));
-    if (!e->prims) { PG_CUDA(cudaMalloc(&e->prims, (size_t)e->n * RENDER_MAX_PRIMS * sizeof(RenderPrim))); fill_render_scene(e); }
+    if (!e->prims.p) { PG_CUDA(cudaMalloc(&e->prims.p, (size_t)e->n * RENDER_MAX_PRIMS * sizeof(RenderPrim))); fill_render_scene(e); }
     // b3ComputeViewMatrixFromYawPitchRoll (up axis 2) + computeProjectionMatrixFOV(fov 60, near 0.1, far 100): pybullet.py:90-102
     const double rad = 0.01745329251994329547, yaw = camera[4] * rad, pitch = camera[5] * rad, roll = camera[6] * rad, dist = camera[3];
     const double cy = cos(yaw), sy = sin(yaw), cr = cos(roll), sr = sin(roll), cp = cos(pitch), sp = sin(pitch);
@@ -665,8 +667,8 @@ int pg_render(pg_env* e, int width, int height, const double* camera, int crop, 
                                                       {26, 230, 26, 255}, {235, 235, 235, 255}};     // plane 0.15, table 0.95, objects (tasks/ *.py rgba_color), robot
     memcpy(C.color, col, sizeof col);
     C.background[0] = 223; C.background[1] = 54; C.background[2] = 45; C.background[3] = 255;          // pybullet.py:28 default background_color
-    with_env(e, [&](auto& E) { launch_render_setup(E, e->rscene, e->prims, (cudaStream_t)stream); });
-    launch_render(e->prims, C, e->n, depth, rgba, segmentation, points, valid, (cudaStream_t)stream);
+    with_env(e, [&](auto& E) { launch_render_setup(E, e->rscene, (RenderPrim*)e->prims.p, (cudaStream_t)stream); });
+    launch_render((const RenderPrim*)e->prims.p, C, e->n, depth, rgba, segmentation, points, valid, (cudaStream_t)stream);
     PG_CUDA(cudaGetLastError());
     return PG_OK;
 }
@@ -685,10 +687,10 @@ int pg_debug_schedule(pg_env* e, unsigned short* key_host, int* perm_host) {
 }
 int pg_debug_timing(pg_env* e, long long* out) {
     if (!e || !out) return fail(PG_ERR_ARG, "pg_debug_timing: NULL argument");
-    if (!e->dbg) return fail(PG_ERR_ARG, "pg_debug_timing: create the handle with PG_DEBUG_TIMING=1 in the environment");
+    if (!e->dbg.p) return fail(PG_ERR_ARG, "pg_debug_timing: create the handle with PG_DEBUG_TIMING=1 in the environment");
     PG_CUDA(cudaSetDevice(e->device));
     PG_CUDA(cudaDeviceSynchronize());
-    PG_CUDA(cudaMemcpy(out, e->dbg, (size_t)e->n * 2 * sizeof(long long), cudaMemcpyDeviceToHost));
+    PG_CUDA(cudaMemcpy(out, e->dbg.p, (size_t)e->n * 2 * sizeof(long long), cudaMemcpyDeviceToHost));
     return PG_OK;
 }
 int pg_contact_overflows(pg_env* e, long long* count) {
@@ -715,8 +717,9 @@ int pg_stats(pg_env* e, double out[4]) {
 // Motion primitives: one allocation holds the plan rows (MotionPlan) and the step's scratch actions / orientations.
 struct pg_motion {
     int n, device;
-    void* blob = nullptr;
+    DevBuf blob;
     MotionPlan P;
+    ~pg_motion() { cudaSetDevice(device); }          // blob is freed after this body runs, on the plan's device
 };
 // the checks every motion entry point makes on its (plan, env) pair
 static int motion_env(pg_motion* m, pg_env* e, const char* who) {
@@ -735,27 +738,21 @@ int pg_motion_create(int num_envs, int device, pg_motion** out) {
     int rc = check_device(device, "pg_motion_create"); if (rc != PG_OK) return rc;
     const size_t n = (size_t)num_envs;
     const size_t f_bytes = MP_ROWS * n * sizeof(double), i_bytes = 3 * n * sizeof(int), act_bytes = 4 * n * sizeof(float), quat_bytes = 4 * n * sizeof(float);
-    pg_motion* m = new pg_motion();
+    auto m = std::make_unique<pg_motion>();
     m->n = num_envs; m->device = device;
-    cudaError_t ce = cudaMalloc(&m->blob, f_bytes + i_bytes + act_bytes + quat_bytes);
-    if (ce == cudaSuccess) ce = cudaMemset(m->blob, 0, f_bytes + i_bytes + act_bytes + quat_bytes);      // every env idle
-    if (ce != cudaSuccess) { cudaFree(m->blob); delete m; return cuda_fail(ce, "pg_motion_create"); }
-    char* b = (char*)m->blob;
+    cudaError_t ce = cudaMalloc(&m->blob.p, f_bytes + i_bytes + act_bytes + quat_bytes);
+    if (ce == cudaSuccess) ce = cudaMemset(m->blob.p, 0, f_bytes + i_bytes + act_bytes + quat_bytes);      // every env idle
+    if (ce != cudaSuccess) return cuda_fail(ce, "pg_motion_create");
+    char* b = (char*)m->blob.p;
     m->P.n = num_envs;
     m->P.f = (double*)b; b += f_bytes;
     m->P.kind = (int*)b; m->P.step = m->P.kind + n; m->P.count = m->P.kind + 2 * n; b += i_bytes;
     m->P.act = (float*)b; b += act_bytes;
     m->P.quat = (float*)b;
-    *out = m;
+    *out = m.release();
     return PG_OK;
 }
-int pg_motion_destroy(pg_motion* m) {
-    if (!m) return PG_OK;
-    cudaSetDevice(m->device);
-    cudaFree(m->blob);
-    delete m;
-    return PG_OK;
-}
+int pg_motion_destroy(pg_motion* m) { delete m; return PG_OK; }
 int pg_motion_move(pg_motion* m, pg_env* e, const double* goal_pos, const double* goal_quat, const unsigned char* mask, void* stream) {
     int rc = motion_env(m, e, "pg_motion_move"); if (rc != PG_OK) return rc;
     if (!goal_pos || !goal_quat) return fail(PG_ERR_ARG, "pg_motion_move: NULL goal_pos or goal_quat");

@@ -130,6 +130,10 @@ def test_create_bare_bad_body_row(lib, col, value):
     _rejected(lib, _create_bare(lib, [BODY, bad]), BODY_BAD)
 
 
+def test_create_bare_zero_quaternion(lib):
+    _rejected(lib, _create_bare(lib, [BODY, BODY[:9] + [0.0] * 4]), "pg_create_bare: zero quaternion")
+
+
 # goal-array entry points (all take a threshold, pg_her_relabel also a row pitch): name -> (takes reward_type, error text)
 REWARD = {
     "pg_compute_reward": (True, "pg_compute_reward: bad argument"),

@@ -164,6 +164,33 @@ def test_sb3_vec_env_interface():
     venv.close()
 
 
+def test_host_reward_staging_grows_only():
+    """pg_compute_reward_host / pg_is_success_host stage through per-device buffers that only grow: once a size has been served,
+    calls of that size allocate nothing (pg_host_stage_allocations is unchanged) and a larger call grows them.  Page-locked and
+    pageable host arrays give the same results."""
+    from panda_lang_manip_b200 import _lib
+    lib = _lib.load()
+    rng = np.random.default_rng(4)
+
+    def call(m, pinned):
+        ag, dg = rng.uniform(-0.2, 0.2, (2, m, 3))
+        rew, ok = np.empty(m, np.float32), np.empty(m, np.uint8)
+        if pinned:
+            ag, dg, rew, ok = (torch.from_numpy(x).pin_memory().numpy() for x in (ag, dg, rew, ok))
+        _lib.check(lib.pg_compute_reward_host(0, 1, 0.05, ag.ctypes.data, dg.ctypes.data, rew.ctypes.data, m, 1, 0))
+        _lib.check(lib.pg_is_success_host(0, 0.05, ag.ctypes.data, dg.ctypes.data, ok.ctypes.data, m, 1, 0))
+        want_r, want_s = reward_np("reach", "dense", ag, dg)
+        assert rew.tobytes() == want_r.tobytes() and np.array_equal(ok, want_s)
+
+    call(10_000, False)
+    before = lib.pg_host_stage_allocations()
+    for pinned in (False, True, False, True):
+        call(10_000, pinned)
+    assert lib.pg_host_stage_allocations() == before
+    call(1 << 21, False)                # larger than any other host reward call of the suite
+    assert lib.pg_host_stage_allocations() > before
+
+
 @pytest.mark.gpu
 def test_index_sorted_her_batch_is_the_same_set_of_transitions():
     """her_sample_indices(sort=True): ascending src, goals inside the transition's own episode, and the relabelled batch is what the unsorted
